@@ -5,6 +5,7 @@ data-parallel over the GPUs of the run (rank r sweeps its contiguous 1024/N shar
 
     python bench.py [--gpus N --steps K --warmup W]            # this repository's CUDA path (one rank per GPU)
     python bench.py --impl reference [...]                     # the reference's CPU path (oracle port) on host cores
+    python bench.py [...] --dump-outputs DIR                   # also save the last timed step's results as DIR/*.npy
 
 A step = one Stage-1 calibration sweep over the whole 1024-image calibration set: embeddings, 12 encoder blocks with the
 fused fc1+GELU+score GEMM, score finisher, and for N>1 the all-reduce of the score vector. `scaling` is "strong": the
@@ -59,7 +60,15 @@ def parse():
     ap.add_argument("--no-extra", action="store_true", help="skip torch_cuda_baseline, weak scaling and the other BASELINE configs")
     ap.add_argument("--model", default="base", choices=["small", "base", "large"], help="other BASELINE configs as the main line (not the bench line)")
     ap.add_argument("--sparsity", type=float, default=0.375)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save what the last one returned, float32: DIR/s1_score_sums.npy (resident sweep: "
+                         "per-neuron sums over all images, blocks concatenated) and DIR/ffn_importance.npy (API call: [blocks, F])")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the B200 arm (the reference arm sizes its sample by the host's speed)")
+    return args
 
 
 def flops_per_image(D=768, F=3072, B=12, T=T_TOKENS, C=1000):
@@ -246,7 +255,8 @@ class Ctx:
         return float(t.item())
 
     def timed(self, fn, steps, warmup):
-        """W untimed calls, then K calls between barrier + synchronize, CUDA events on the launching stream, max over ranks."""
+        """W untimed calls, then K calls between barrier + synchronize, CUDA events on the launching stream, max over ranks.
+        Returns (ms, launches, what the last timed call returned)."""
         for i in range(warmup):
             fn(i)
         self.barrier()
@@ -255,11 +265,11 @@ class Ctx:
         l0 = self.lib.tssp_launch_count()
         e0.record()
         for i in range(steps):
-            fn(warmup + i)
+            last = fn(warmup + i)
         e1.record()
         torch.cuda.synchronize()
         self.barrier()
-        return self.max_over_ranks(e0.elapsed_time(e1)), int(self.lib.tssp_launch_count() - l0)
+        return self.max_over_ranks(e0.elapsed_time(e1)), int(self.lib.tssp_launch_count() - l0), last
 
 
 def shard(n: int, rank: int, world: int) -> slice:
@@ -267,7 +277,8 @@ def shard(n: int, rank: int, world: int) -> slice:
     return D.shard_slice(n, rank, world)
 
 
-def measure_sweep(cx: Ctx, model_name: str, model, px_dev, px_host, bs: int, steps: int, warmup: int, profile: bool, weak: bool):
+def measure_sweep(cx: Ctx, model_name: str, model, px_dev, px_host, bs: int, steps: int, warmup: int, profile: bool, weak: bool,
+                  outputs: bool = False):
     """Stage-1 sweep of the whole calibration set, sharded over the ranks (strong scaling): device-timed value, the
     end-to-end API arm, optionally the weak-scaling line and the per-kernel-class profile."""
     api, L, lib, world, rank, dev = cx.api, cx.L, cx.lib, cx.world, cx.rank, cx.dev
@@ -305,17 +316,21 @@ def measure_sweep(cx: Ctx, model_name: str, model, px_dev, px_host, bs: int, ste
         return api._compute_ffn_activation_importance(model, host_batches, device=dev, group=cx.group)
 
     out = {"images": n_total, "batch": bs_local, "images_per_rank": n_local}
-    ms, launches = cx.timed(step_resident, steps, warmup)
+    ms, launches, sums = cx.timed(step_resident, steps, warmup)
     out.update(ms_total=ms, launches=launches, value=n_total * steps / (ms * 1e-3), ms_per_step=ms / steps)
     # the host-batch path settles over its first ~7 calls (tools/e2e_scaling_probe.py: 13.9 -> 11.5 ms per call at 4 ranks
     # right after the resident loop), so it gets its own warm-up of at least 8 calls
     e2e_warmup = max(warmup, 8)
-    ms_e, _ = cx.timed(step_e2e, steps, e2e_warmup)
+    ms_e, _, importance = cx.timed(step_e2e, steps, e2e_warmup)
+    if outputs:
+        # what each timed path hands its caller in the last step: the engine's score sums over all images (device, flat)
+        # and the API's per-block importance (host, sums / images)
+        out["outputs"] = {"s1_score_sums": sums.cpu().numpy(), "ffn_importance": torch.stack(importance).numpy()}
     out["e2e"] = {"value": n_total * steps / (ms_e * 1e-3), "unit": "images/s", "ms_per_step": ms_e / steps, "warmup": e2e_warmup,
                   "h2d_bytes_per_step": int(n_total * 3 * 224 * 224 * 4), "d2h_bytes_per_step": int(sum_f * 4 * world),
                   "api": "twossp_b200.api._compute_ffn_activation_importance(model, pinned host batches of the rank's shard, device='cuda', group=...)"}
     if weak and world > 1:
-        ms_w, _ = cx.timed(step_weak, max(2, steps // 2), 2)
+        ms_w, _, _ = cx.timed(step_weak, max(2, steps // 2), 2)
         out["weak"] = {"value": n_total * world * max(2, steps // 2) / (ms_w * 1e-3), "unit": "images/s", "ms_per_step": ms_w / max(2, steps // 2),
                        "images_per_gpu_per_step": n_total, "note": "every rank sweeps the whole set (last round's headline): work grows with N"}
     D_, F_, B_ = SHAPE[model_name]
@@ -588,8 +603,14 @@ def run_b200(args):
     px_host.copy_(px_dev)
 
     sampler = ClockSampler(cx.local) if rank == 0 and not args.no_clocks else None
-    main = measure_sweep(cx, args.model, model, px_dev, px_host, bs, args.steps, args.warmup, profile=True, weak=not args.no_extra)
+    main = measure_sweep(cx, args.model, model, px_dev, px_host, bs, args.steps, args.warmup, profile=True, weak=not args.no_extra,
+                         outputs=rank == 0 and bool(args.dump_outputs))
     clocks = sampler.stop() if sampler is not None else None
+    if rank == 0 and args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in main.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
 
     peaks = measured_peaks()
     # everything below is secondary to the line's headline numbers: a failure there is reported inside the line, not instead of it

@@ -19,6 +19,7 @@ from __future__ import annotations
 
 import contextlib
 import copy
+import hashlib
 import importlib.util
 import io
 import json
@@ -86,6 +87,24 @@ def pack_bits(mask_lists):
     return np.packbits(np.asarray(mask_lists, dtype=np.uint8), axis=-1)
 
 
+WEIGHT_SAMPLE = 512
+
+
+def weight_fixture(state):
+    """The seeded init in a file well under 1 MB: per tensor its shape, the SHA-256 of its bytes and a fixed sample of
+    its entries (all of them for tensors of at most WEIGHT_SAMPLE entries) at the stored flat positions."""
+    out = {}
+    rng = np.random.default_rng(0)
+    for k, v in state.items():
+        v = np.ascontiguousarray(v, dtype=np.float32)
+        idx = np.arange(v.size) if v.size <= WEIGHT_SAMPLE else np.sort(rng.choice(v.size, WEIGHT_SAMPLE, replace=False))
+        out[k] = v.reshape(-1)[idx]
+        out[f"{k}:index"] = idx.astype(np.int64)
+        out[f"{k}:shape"] = np.asarray(v.shape, dtype=np.int64)
+        out[f"{k}:sha256"] = np.array(hashlib.sha256(v.tobytes()).hexdigest())
+    return out
+
+
 def golden_for(vp, mc, name: str, n_img: int, batch: int, t_prune: int, store_weights: bool, s2: bool):
     model = synth.make_vit(name, seed=0)
     image = synth.SHAPES[name][0]
@@ -98,6 +117,7 @@ def golden_for(vp, mc, name: str, n_img: int, batch: int, t_prune: int, store_we
             "pixels_sha": synth.sha256_tensors([pixels]), "torch": torch.__version__}
     import transformers
     meta["transformers"] = transformers.__version__
+    meta["cpu_threads"] = torch.get_num_threads()   # oneDNN's bf16 GEMMs split work by thread count: the as-is bits follow
 
     with autocast_disabled():
         s_fp32 = quiet(vp._compute_ffn_activation_importance, model, batches, device="cpu", batch_limit=None)
@@ -144,7 +164,7 @@ def golden_for(vp, mc, name: str, n_img: int, batch: int, t_prune: int, store_we
                       "num_to_prune": max(1, nb // 3)}
     if store_weights:
         sd = model.state_dict()
-        np.savez_compressed(GOLDEN / f"{name}_weights.npz", **{k: v.numpy() for k, v in sd.items()})
+        np.savez_compressed(GOLDEN / f"{name}_weights.npz", **weight_fixture({k: v.numpy() for k, v in sd.items()}))
     np.savez_compressed(GOLDEN / f"{name}_ref.npz", **out)
     return meta
 

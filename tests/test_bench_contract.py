@@ -52,3 +52,31 @@ def test_b200_arm_refuses_to_run_without_a_gpu():
     r = _run(["--steps", "1", "--warmup", "0"], timeout=300)
     assert r.returncode != 0 and "no CUDA device" in (r.stderr + r.stdout)
     assert not any(ln.startswith("{") for ln in r.stdout.splitlines())  # no number without a GPU
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step_and_repeat_exactly(tmp_path):
+    """--dump-outputs saves what the timed step returned; another run on the same inputs, with another step count, saves
+    the same bits; --steps sets the number of timed steps (the launches counted in the timed region scale with it)."""
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    import numpy as np
+    n_img = 96
+    common = ["--model", "small", "--images", str(n_img), "--batch", "32", "--warmup", "1",
+              "--no-prune", "--no-extra", "--no-cpu-baseline", "--no-clocks"]
+    lines, dumps = {}, {}
+    for steps in (1, 3):
+        d = tmp_path / f"steps{steps}"
+        r = _run([*common, "--steps", str(steps), "--dump-outputs", str(d)], timeout=900)
+        assert r.returncode == 0, r.stderr[-3000:]
+        lines[steps] = json.loads(next(ln for ln in r.stdout.splitlines() if ln.startswith("{")))
+        dumps[steps] = {name: np.load(d / f"{name}.npy") for name in ("s1_score_sums", "ffn_importance")}
+    assert lines[1]["steps"] == 1 and lines[3]["steps"] == 3
+    assert lines[3]["gpu_launches"] == 3 * lines[1]["gpu_launches"] > 0
+    sums, imp = dumps[1]["s1_score_sums"], dumps[1]["ffn_importance"]
+    assert sums.dtype == np.float32 and imp.dtype == np.float32
+    assert sums.shape == (12 * 1536,) and imp.shape == (12, 1536)      # ViT-S/16: 12 blocks of 1536 neurons
+    assert np.isfinite(sums).all() and (sums > 0).all()
+    assert np.allclose(imp.reshape(-1), sums / n_img, rtol=1e-5)
+    for name in dumps[1]:
+        assert np.array_equal(dumps[1][name], dumps[3][name]), name

@@ -1,7 +1,9 @@
 """The oracle (oracle/twossp_oracle.py) against the golden vectors recorded from the UNMODIFIED reference by
 oracle/make_golden.py. CPU only. Integer/index results must be identical; float results are produced by the same
 torch ops in the same order, so they are compared bit-for-bit too."""
+import contextlib
 import copy
+import hashlib
 
 import numpy as np
 import pytest
@@ -28,25 +30,44 @@ def _unpack(bits, width):
     return np.unpackbits(bits, axis=-1)[..., :width]
 
 
+@contextlib.contextmanager
+def _cpu_threads(n):
+    saved = torch.get_num_threads()
+    torch.set_num_threads(n)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(saved)
+
+
 @pytest.mark.parametrize("name", ["tiny", "base"])
 def test_s1_scores_match_reference(name, golden_dir, golden_meta):
     model, pixels, m = _setup(name, golden_meta)
     g = _load(golden_dir, name)
     batches = synth.make_batches(pixels, None, m["batch"])
-    fp32 = torch.stack(O.s1_scores(model, batches, "cpu", None, autocast=False)).numpy()
+    # CPU autocast runs oneDNN's bf16 GEMMs, which split their work by the intra-op thread count: the recorded bits are
+    # those of the recording's thread count, whatever the cores of the machine running the test
+    with _cpu_threads(m["cpu_threads"]):
+        fp32 = torch.stack(O.s1_scores(model, batches, "cpu", None, autocast=False)).numpy()
+        asis = O.s1_scores(model, batches, "cpu", None, autocast=True)
     assert np.array_equal(fp32, g["scores_fp32"])
-    asis = O.s1_scores(model, batches, "cpu", None, autocast=True)
     assert str(asis[0].dtype) == str(g["scores_asis_dtype"])
     assert np.array_equal(torch.stack([s.float() for s in asis]).numpy(), g["scores_asis"])
 
 
 def test_tiny_weights_fixture_matches_seeded_init(golden_dir, golden_meta):
+    # the fixture holds, per tensor, its shape, the SHA-256 of all its bytes and a sample of its entries
+    # (oracle/make_golden.py: weight_fixture)
     model, _, _ = _setup("tiny", golden_meta)
     w = np.load(f"{golden_dir}/tiny_weights.npz")
     sd = model.state_dict()
-    assert set(w.files) == set(sd.keys())
-    for k in w.files:
-        assert np.array_equal(w[k], sd[k].numpy()), k
+    keys = {f for f in w.files if ":" not in f}
+    assert keys == set(sd.keys())
+    for k in keys:
+        v = np.ascontiguousarray(sd[k].numpy(), dtype=np.float32)
+        assert list(v.shape) == w[f"{k}:shape"].tolist(), k
+        assert np.array_equal(v.reshape(-1)[w[f"{k}:index"]], w[k]), k
+        assert hashlib.sha256(v.tobytes()).hexdigest() == str(w[f"{k}:sha256"]), k
 
 
 @pytest.mark.parametrize("name", ["tiny", "base"])

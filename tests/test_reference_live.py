@@ -1,7 +1,9 @@
-"""Live differential tests against the UNMODIFIED reference, for the parts of the path that are pure host logic
-(planner, parameter accounting, selection + masks given scores). They run only where the reference is mounted
-(/root/reference in the build container; never on the GPU box, where the golden fixtures stand in) and widen the
-pinned golden rows to a few hundred random configurations."""
+"""Differential tests against the UNMODIFIED reference, for the parts of the path that are pure host logic
+(planner, parameter accounting, selection + masks given scores). They widen the pinned golden rows of tests/golden/ to a
+few hundred random configurations. The reference is not part of this repository: the comparisons with it run when
+TSSP_REFERENCE names a checkout of it (zvezdvv/2ssp-X-vit) and skip otherwise. The planner and the parameter accounting
+are also compared, on the same random configurations and on every run, with the oracle (oracle/twossp_oracle.py), which
+the golden rows pin to the reference."""
 import contextlib
 import io
 import os
@@ -13,8 +15,9 @@ import pytest
 import torch
 
 ROOT = Path(__file__).resolve().parent.parent
-REF = Path(os.environ.get("TSSP_REFERENCE", "/root/reference"))
-pytestmark = pytest.mark.skipif(not (REF / "src" / "vit_pruning.py").exists(), reason="reference sources not mounted here")
+REF = Path(os.environ["TSSP_REFERENCE"]) if os.environ.get("TSSP_REFERENCE") else None
+needs_reference = pytest.mark.skipif(REF is None or not (REF / "src" / "vit_pruning.py").exists(),
+                                     reason="TSSP_REFERENCE does not name a checkout of the reference")
 
 
 @pytest.fixture(scope="module")
@@ -40,33 +43,70 @@ def _quiet(fn, *a, **k):
         return fn(*a, **k)
 
 
-def test_planner_and_accounting_match_the_reference_on_random_shapes(ref_vp):
-    from twossp_b200 import api
+def _planner_cases():
+    """12 random tiny ViTs (heads, widths, depths, odd FFN widths), 25 random (target, min_remaining, forced_blocks) each:
+    yields (model, None) once per model, then (model, (target, min_remaining, forced_blocks)) per plan."""
     rng = random.Random(20261018)
-    n_cases = 0
     for m in range(12):
         heads = rng.choice([1, 2, 4])
         hidden = heads * rng.choice([8, 16, 32])
         layers = rng.randint(2, 9)
         ffn = rng.choice([hidden, 2 * hidden, 4 * hidden, 4 * hidden + 8, 3 * hidden - 8])
         model = _tiny_vit(hidden, layers, heads, ffn, seed=m)
-        assert api.count_total_params(model) == ref_vp.count_total_params(model)
-        assert api.count_block_params(model) == ref_vp.count_block_params(model)
-        assert api._count_attention_params_per_block(model) == ref_vp._count_attention_params_per_block(model)
-        assert api._count_ffn_params_per_block(model) == ref_vp._count_ffn_params_per_block(model)
+        yield model, None
         for _ in range(25):
             target = rng.choice([0.02, 0.1, 0.25, 0.375, 0.5, 0.6, 0.75, rng.uniform(0.01, 0.9)])
             mr = rng.choice([1, 8, ffn // 4, ffn // 2, ffn, 2 * ffn])
             forced = rng.choice([None, None, None, 0, 1, layers - 1])
-            ours = _quiet(api.plan_2ssp_allocation, model, target, min_remaining=mr, forced_blocks=forced)
-            theirs = _quiet(ref_vp.plan_2ssp_allocation, model, target, min_remaining=mr, forced_blocks=forced)
-            key = lambda p: (p.target_sparsity, p.num_blocks_total, p.blocks_to_prune, p.per_block_neurons_to_prune, p.stage2_fraction,
-                             p.estimated_total_removed_params, p.est_error_params)
-            assert key(ours) == key(theirs), (hidden, layers, heads, ffn, target, mr, forced, key(ours), key(theirs))
-            n_cases += 1
+            yield model, (target, mr, forced)
+
+
+def _plan_key(p):
+    return (p.target_sparsity, p.num_blocks_total, p.blocks_to_prune, p.per_block_neurons_to_prune, p.stage2_fraction,
+            p.estimated_total_removed_params, p.est_error_params)
+
+
+def test_planner_and_accounting_match_the_oracle_on_random_shapes():
+    from oracle import twossp_oracle as O
+    from twossp_b200 import api
+    n_cases = 0
+    for model, case in _planner_cases():
+        if case is None:
+            blocks = O.blocks_of(model)[1]
+            pairs = O.mlp_pairs(model)
+            assert api.count_total_params(model) == O._numel(model)
+            assert api.count_block_params(model) == [O._numel(b) for b in blocks]
+            assert api._count_attention_params_per_block(model) == [O._numel(b.attention) for b in blocks]
+            assert api._count_ffn_params_per_block(model) == [O._numel(a) + O._numel(c) for a, c in pairs]
+            continue
+        target, mr, forced = case
+        ours = _quiet(api.plan_2ssp_allocation, model, target, min_remaining=mr, forced_blocks=forced)
+        oracle = O.plan(model, target, min_remaining=mr, forced_blocks=forced)
+        assert _plan_key(ours) == _plan_key(oracle), (case, _plan_key(ours), _plan_key(oracle))
+        n_cases += 1
     assert n_cases == 300
 
 
+@needs_reference
+def test_planner_and_accounting_match_the_reference_on_random_shapes(ref_vp):
+    from twossp_b200 import api
+    n_cases = 0
+    for model, case in _planner_cases():
+        if case is None:
+            assert api.count_total_params(model) == ref_vp.count_total_params(model)
+            assert api.count_block_params(model) == ref_vp.count_block_params(model)
+            assert api._count_attention_params_per_block(model) == ref_vp._count_attention_params_per_block(model)
+            assert api._count_ffn_params_per_block(model) == ref_vp._count_ffn_params_per_block(model)
+            continue
+        target, mr, forced = case
+        ours = _quiet(api.plan_2ssp_allocation, model, target, min_remaining=mr, forced_blocks=forced)
+        theirs = _quiet(ref_vp.plan_2ssp_allocation, model, target, min_remaining=mr, forced_blocks=forced)
+        assert _plan_key(ours) == _plan_key(theirs), (case, _plan_key(ours), _plan_key(theirs))
+        n_cases += 1
+    assert n_cases == 300
+
+
+@needs_reference
 def test_selection_and_masks_given_scores_match_the_reference_on_cpu_tensors(ref_vp):
     # the selection arithmetic of prune_vit_mlp_width (n_prune truncation, min_remaining clamp, argsort / sort, mask layout,
     # skipped blocks) restated by the oracle, against the reference itself, on random widths and score vectors with ties
@@ -100,7 +140,9 @@ def _load_script(name, file):
     return mod
 
 
-@pytest.mark.skipif(not (REF / "manual-experiments" / "consensus_mask.py").exists(), reason="reference scripts not mounted here")
+@needs_reference
+@pytest.mark.skipif(REF is None or not (REF / "manual-experiments" / "consensus_mask.py").exists(),
+                    reason="TSSP_REFERENCE does not name a checkout of the reference with its manual-experiments scripts")
 def test_mask_builder_oracle_matches_the_reference_scripts_on_random_inputs():
     # consensus (growing-t intersection), summation masks and min-max normalisation: the oracle restatement against the
     # unmodified scripts on 40 random configurations (files, ragged widths, heavy ties, every rounding mode, tiny fractions)
@@ -174,6 +216,7 @@ def hf_tuple_shim():
     mv.ViTLayer.forward = saved
 
 
+@needs_reference
 @pytest.mark.parametrize("autocast", [True, False])
 def test_stage1_and_stage2_oracle_match_the_reference_live(ref_vp, ref_iface, hf_tuple_shim, autocast):
     # random tiny ViTs and inputs beyond the committed fixtures: Stage-1 scores bit for bit (as-is = CPU autocast bf16, and
@@ -218,6 +261,7 @@ def test_stage1_and_stage2_oracle_match_the_reference_live(ref_vp, ref_iface, hf
         assert ours_sel["original_metrics"] == ref_sel["original_metrics"] and ours_sel["final_metrics"] == ref_sel["final_metrics"]
 
 
+@needs_reference
 def test_api_surface_mirrors_the_reference(ref_vp):
     """Every function of the path that the reference exports has a counterpart with the same parameter names in the same
     order (extra keyword-only / trailing parameters allowed), and the plugin class has the same constructor and methods.

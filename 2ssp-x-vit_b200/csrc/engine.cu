@@ -20,6 +20,7 @@
 #include "gemm_tcgen05.cuh"
 #include "kernels.cuh"
 #include "attention_tcgen05.cuh"
+#include "attention_long_tcgen05.cuh"
 #include "mask_builders.cuh"
 #include "gather.cuh"
 
@@ -467,8 +468,31 @@ static int get_tmap_qkv(const CUtensorMap** out, const void* qkv, int n, int T, 
     return 0;
 }
 
-// softmax(Q K^T / sqrt(64)) V per (image, head): attention_tcgen05.cuh
+// softmax(Q K^T / sqrt(64)) V per (image, head): attention_tcgen05.cuh up to 208 padded keys, attention_long_tcgen05.cuh
+// (keys in tiles of 128) beyond
 static long long* g_attn_trace = nullptr;  // device buffer set by tssp_debug_attention_trace (diagnostics only)
+
+static int op_attention_long(const void* qkv, void* ctx, int n, int T, int heads, int D, cudaStream_t s, const float* qk_norms,
+                             int ld_norms, bool first_tile_only) {
+    const CUtensorMap *tqkv, *tctx;
+    TSSP_TRY(get_tmap_qkv(&tqkv, qkv, n, T, 3 * D, 128));
+    TSSP_TRY(get_tmap_qkv(&tctx, ctx, n, T, D, 32));
+    TSSP_TRY(ensure_smem(attention_long_tcgen05_kernel, ATL_SMEM_BYTES));
+    AttnLongParams p;
+    p.n_img = n; p.T = T; p.heads = heads; p.D = D;
+    p.MT = first_tile_only ? 1 : ceil_div(T, 128);
+    p.n_groups = ceil_div(p.MT, ATL_MAX_G);
+    p.NKT = ceil_div(T, ATL_KT);
+    p.scale_log2e = 1.4426950408889634f / sqrtf(static_cast<float>(ATT_HD));
+    p.norms = qk_norms; p.ld_norms = ld_norms;
+    p.qkv = static_cast<const __nv_bfloat16*>(qkv);
+    p.reverse = chain_dir();
+    const long long units = static_cast<long long>(n) * heads * p.n_groups;
+    const int grid = units < num_sms() ? static_cast<int>(units) : num_sms();
+    TSSP_CUDA(launch_pdl(attention_long_tcgen05_kernel, dim3(grid), dim3(ATL_THREADS), ATL_SMEM_BYTES, s, *tqkv, *tctx, p));
+    TSSP_LAUNCH_CHECK("attention_long_tcgen05_kernel");
+    return 0;
+}
 
 // first_tile_only: only the first 128 query rows of every (image, head) are computed (the rest of ctx is left alone) --
 // for the last block of a classifier forward, where the CLS row (row 0) is all that is read afterwards
@@ -476,7 +500,8 @@ static int op_attention(const void* qkv, void* ctx, int n, int T, int heads, int
                         const float* qk_norms = nullptr, int ld_norms = 0, bool first_tile_only = false) {
     if (D != heads * ATT_HD) return fail("attention: head_dim must be 64 (D=%d heads=%d)", D, heads);
     const int Tp = round_up(T, 16);
-    if (T < 16 || Tp > ATC_KV_ROWS) return fail("attention: T=%d outside the supported [16, %d] tokens", T, ATC_KV_ROWS);
+    if (T < 16 || T > ATL_MAX_T) return fail("attention: T=%d outside the supported [16, %d] tokens", T, ATL_MAX_T);
+    if (Tp > ATC_KV_ROWS) return op_attention_long(qkv, ctx, n, T, heads, D, s, qk_norms, ld_norms, first_tile_only);
     const float scale_log2e = 1.4426950408889634f / sqrtf(static_cast<float>(ATT_HD));
     const CUtensorMap *tq, *tkv;
     const CUtensorMap* tctx;
@@ -660,7 +685,7 @@ static int validate(const tssp_config_t& c) {
     if (c.heads * 64 != c.hidden) return fail("config: head_dim must be 64 (hidden=%d heads=%d)", c.hidden, c.heads);
     if (c.patch_size % 8 || c.image_size % c.patch_size) return fail("config: image %d / patch %d unsupported", c.image_size, c.patch_size);
     const int G = c.image_size / c.patch_size, T = G * G + 1;
-    if (T < 32 || T > 208) return fail("config: tokens per image T=%d must be in [32,208]", T);
+    if (T < 32 || T > ATL_MAX_T) return fail("config: tokens per image T=%d must be in [32,%d]", T, ATL_MAX_T);
     if ((c.channels * c.patch_size * c.patch_size) % 8) return fail("config: patch vector length not a multiple of 8");
     if (c.max_images < 1) return fail("config: max_images=%d", c.max_images);
     for (int b = 0; b < c.n_blocks; ++b)

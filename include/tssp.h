@@ -36,7 +36,9 @@ extern "C" {
 typedef struct tssp_engine* tssp_handle_t;
 
 /* Model anatomy, as discovered by the reference's _get_encoder/_gather_mlp_pairs walkers
- * (src/vit_pruning.py:28-75) on an HF ViTForImageClassification or a timm VisionTransformer. */
+ * (src/vit_pruning.py:28-75) on an HF ViTForImageClassification or a timm VisionTransformer.
+ * Tokens per image T = (image_size / patch_size)^2 + 1 must lie in [32, 1025]: ViT-x/16 up to 512x512 (T = 1025),
+ * ViT-x/8 up to 256x256; tssp_create rejects other shapes before it touches a device. */
 typedef struct tssp_config {
     int32_t n_blocks;                      /* B: encoder blocks */
     int32_t hidden;                        /* D: multiple of 128, <= 1024 */
@@ -153,6 +155,8 @@ int tssp_op_score_finish(const float* partials, int ldp, float* norms, int ldn, 
                          float* scores, void* stream);
 int tssp_op_layernorm(const float* x, int64_t in_stride, const float* gamma, const float* beta, void* out_bf16,
                       int rows, int D, float eps, void* stream);
+/* ctx[n*T, D] = softmax(Q K^T / 8) V per (image, head) from the fused qkv[n*T, 3D]; head_dim 64, 16 <= T <= 1025
+ * (up to 208 padded keys one kernel holds a whole key row, beyond that a second one streams keys in tiles of 128). */
 int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream);
 int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream);
 int tssp_op_cast_bf16(const float* in, int rows, int cols, int ld_in, void* out_bf16, int rows_pad, int cols_pad,

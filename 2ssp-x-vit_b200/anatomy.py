@@ -2,8 +2,10 @@
 
 Mirrors the reference's attribute walking (src/vit_pruning.py:28-75 `_get_encoder`, `_gather_mlp_pairs`,
 `_get_hidden_and_inter_sizes`): HF `ViTModel` / `ViTForImageClassification`
-(`.vit.encoder.layer[i].{attention,intermediate,output}`) and timm-shaped `VisionTransformer`
-(`.blocks[i].{norm1,attn,norm2,mlp.fc1,mlp.fc2}`).
+(`.vit.encoder.layer[i].{attention,intermediate,output}`), HF `DeiTModel` / `DeiTForImageClassification` /
+`DeiTForImageClassificationWithTeacher` (`.deit`, the same layer layout; the reference reaches it through
+`model.base_model`) and timm-shaped `VisionTransformer` (`.blocks[i].{norm1,attn,norm2,mlp.fc1,mlp.fc2}`), distilled
+ones (`dist_token`, `head_dist`) included.
 """
 from __future__ import annotations
 
@@ -100,6 +102,8 @@ class Anatomy:
     ffn_dims: List[int]
     attn_present: List[bool]
     score_point: int                      # 0 post-GELU (HF hook point), 1 pre-GELU (timm hook point)
+    prefix_tokens: int = 1                # tokens ahead of the patches: 1 (CLS) or 2 (CLS, distillation token: DeiT)
+    dist_head: bool = False               # logits = (head(row 0) + dist_head(row 1)) / 2 (globals_ "head_dist_w/_b")
     globals_: Dict[str, Optional[torch.Tensor]] = field(default_factory=dict)
     blocks: List[Dict[str, Optional[torch.Tensor]]] = field(default_factory=list)
 
@@ -122,16 +126,49 @@ def _head(module) -> Tuple[int, int, Optional[torch.Tensor], Optional[torch.Tens
     raise AttributeError(f"Unsupported classification head: {type(module).__name__}")
 
 
+def _dist_head(main: Tuple, module) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """(weight, bias) of a distillation head averaged with the main head `main` (a `_head` tuple), or (None, None)."""
+    if module is None or isinstance(module, nn.Identity):
+        if main[0] > 0:
+            raise AttributeError("a classification head without its distillation head is not supported")
+        return None, None
+    if main[1] > 0:
+        raise AttributeError("a distillation head combined with a Sequential classification head is not supported")
+    if not isinstance(module, nn.Linear):
+        raise AttributeError(f"Unsupported distillation head: {type(module).__name__}")
+    if module.out_features != main[0]:
+        raise AttributeError(f"distillation head has {module.out_features} outputs, the classification head {main[0]}")
+    return _p(module.weight), _p(module.bias)
+
+
+def _hf_root(vit_model):
+    for name in ("vit", "deit"):
+        if hasattr(vit_model, name):
+            return getattr(vit_model, name)
+    return vit_model
+
+
 def describe(vit_model) -> Anatomy:
     kind, blocks = get_blocks(vit_model)
     pairs = gather_mlp_pairs(vit_model)
     hidden = pairs[0][0].weight.size(1)
+    prefix = 1
+    hdw = hdb = None
+    dist = False
     if kind == "hf":
-        vit = vit_model.vit if hasattr(vit_model, "vit") else vit_model
+        vit = _hf_root(vit_model)
         emb = vit.embeddings
         conv = emb.patch_embeddings.projection
         final_ln = vit.layernorm
-        n_classes, head_hidden, h0, hw, hb = _head(getattr(vit_model, "classifier", None))
+        if getattr(emb, "distillation_token", None) is not None:  # DeiTEmbeddings: [CLS, distillation, patches]
+            prefix = 2
+        if hasattr(vit_model, "cls_classifier"):                  # DeiTForImageClassificationWithTeacher: averaged heads
+            head = _head(vit_model.cls_classifier)
+            hdw, hdb = _dist_head(head, getattr(vit_model, "distillation_classifier", None))
+            dist = hdw is not None
+        else:
+            head = _head(getattr(vit_model, "classifier", None))
+        n_classes, head_hidden, h0, hw, hb = head
         cfg = vit_model.config
         heads = int(cfg.num_attention_heads)
         act = getattr(cfg, "hidden_act", "gelu")
@@ -140,6 +177,7 @@ def describe(vit_model) -> Anatomy:
         g = {
             "patch_w": _p(conv.weight), "patch_b": _p(conv.bias), "cls": _p(emb.cls_token), "pos": _p(emb.position_embeddings),
             "final_ln_w": _p(final_ln.weight), "final_ln_b": _p(final_ln.bias), "head0_w": h0, "head_w": hw, "head_b": hb,
+            "dist": _p(getattr(emb, "distillation_token", None)), "head_dist_w": hdw, "head_dist_b": hdb,
         }
         blks = []
         for b in blocks:
@@ -164,12 +202,18 @@ def describe(vit_model) -> Anatomy:
         root = vit_model
         conv = root.patch_embed.proj
         final_ln = root.norm
-        n_classes, head_hidden, h0, hw, hb = _head(getattr(root, "head", None))
+        head = _head(getattr(root, "head", None))
+        if getattr(root, "dist_token", None) is not None:  # timm VisionTransformerDistilled: eval output averages both heads
+            prefix = 2
+            hdw, hdb = _dist_head(head, getattr(root, "head_dist", None))
+            dist = hdw is not None
+        n_classes, head_hidden, h0, hw, hb = head
         first_attn = next((b.attn for b in blocks if has_attention(kind, b)), None)
         heads = int(first_attn.num_heads) if first_attn is not None else hidden // 64
         g = {
             "patch_w": _p(conv.weight), "patch_b": _p(conv.bias), "cls": _p(root.cls_token), "pos": _p(root.pos_embed),
             "final_ln_w": _p(final_ln.weight), "final_ln_b": _p(final_ln.bias), "head0_w": h0, "head_w": hw, "head_b": hb,
+            "dist": _p(getattr(root, "dist_token", None)), "head_dist_w": hdw, "head_dist_b": hdb,
         }
         blks = []
         for b in blocks:
@@ -195,12 +239,14 @@ def describe(vit_model) -> Anatomy:
     pw = g["patch_w"]
     channels, patch = int(pw.shape[1]), int(pw.shape[2])
     n_tokens = int(g["pos"].reshape(-1, hidden).shape[0])
-    grid = int(round((n_tokens - 1) ** 0.5))
-    if grid * grid + 1 != n_tokens:
-        raise AttributeError(f"position table with {n_tokens} rows is not a square grid plus CLS")
+    grid = int(round(max(0, n_tokens - prefix) ** 0.5))
+    if grid * grid + prefix != n_tokens:
+        what = "CLS" if prefix == 1 else "CLS and distillation token"
+        raise AttributeError(f"position table with {n_tokens} rows fits neither layout: not a square grid plus {what} "
+                             f"({prefix} prefix token{'s' if prefix > 1 else ''})")
     return Anatomy(
         kind=kind, n_blocks=len(blocks), hidden=int(hidden), heads=heads, image_size=grid * patch, patch_size=patch,
         channels=channels, n_classes=int(n_classes), head_hidden=int(head_hidden), ln_eps=eps,
         ffn_dims=[int(p[0].weight.size(0)) for p in pairs], attn_present=[has_attention(kind, b) for b in blocks],
-        score_point=score_point, globals_=g, blocks=blks,
+        score_point=score_point, prefix_tokens=prefix, dist_head=dist, globals_=g, blocks=blks,
     )

@@ -382,31 +382,36 @@ static inline int grid_for(long long work, int threads) {
     return static_cast<int>(g);
 }
 
-static int op_cast(const float* in, int rows, int cols, int ld_in, void* out, int rows_pad, int cols_pad, int ld_out, cudaStream_t s) {
+static int op_cast(const float* in, int rows, int cols, int ld_in, void* out, int rows_pad, int cols_pad, int ld_out, cudaStream_t s,
+                   float scale = 1.0f) {
     const long long total = static_cast<long long>(rows_pad) * cols_pad;
     if (total == 0) return 0;
-    cast_pad_bf16_kernel<<<grid_for(total, 256), 256, 0, s>>>(in, rows, cols, ld_in, static_cast<__nv_bfloat16*>(out), rows_pad, cols_pad, ld_out);
+    cast_pad_bf16_kernel<<<grid_for(total, 256), 256, 0, s>>>(in, rows, cols, ld_in, static_cast<__nv_bfloat16*>(out), rows_pad, cols_pad, ld_out,
+                                                              scale);
     TSSP_LAUNCH_CHECK("cast_pad_bf16_kernel");
     return 0;
 }
 
-static int op_im2col(const float* pixels, void* out, int n, int C, int H, int W, int P, cudaStream_t s) {
+// prefix: zero rows ahead of every image's patches (1: CLS; 2: CLS and the DeiT distillation token)
+static int op_im2col(const float* pixels, void* out, int n, int C, int H, int W, int P, cudaStream_t s, int prefix = 1) {
     if (H % P || W % P || (P & 7) || H != W) return fail("im2col: H=%d W=%d P=%d unsupported (square images, P multiple of 8)", H, W, P);
-    const int T = (H / P) * (W / P) + 1;
+    if (prefix < 1 || prefix > 2) return fail("im2col: prefix=%d must be 1 or 2", prefix);
+    const int T = (H / P) * (W / P) + prefix;
     const long long total = static_cast<long long>(n) * T * (C * P * P / 8);
-    im2col_patches_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T);
+    im2col_patches_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T, prefix);
     TSSP_LAUNCH_CHECK("im2col_patches_kernel");
     return 0;
 }
 
 static int op_layernorm(const float* x, long long in_stride, const float* g, const float* b, void* out, int rows, int D, float eps, cudaStream_t s,
                         bool stream_in = false) {
-    if ((D & 127) || D > 1024) return fail("layernorm: D=%d must be a multiple of 128 and <= 1024", D);
+    if (((D & 127) && D != 192) || D > 1024) return fail("layernorm: D=%d must be 192 or a multiple of 128 <= 1024", D);
     if (in_stride & 3) return fail("layernorm: row pitch %lld must be a multiple of 4 elements", in_stride);
     if (rows <= 0) return 0;
     // persistent: resident CTAs per SM. Narrow rows need more warps for the same bytes in flight; at D = 1024 the kernel
     // holds 150 registers (row, prefetched row, gamma, beta), so 12 warps fit as three CTAs of 128 threads but only 8
-    // as one CTA of 256 (re-reading gamma / beta instead of holding them was measured slower: 0.60 against 0.75 of peak)
+    // as one CTA of 256 (re-reading gamma / beta instead of holding them was measured slower: 0.60 against 0.75 of peak).
+    // D = 192 (64-element slabs, six values a lane) takes the D <= 512 setting.
     const int threads = D > 768 ? 128 : 256;
     const int per_sm = D <= 512 ? 4 : (D > 768 ? 3 : 2);
     const int ctas = ceil_div(rows, threads / 32);
@@ -417,6 +422,7 @@ static int op_layernorm(const float* x, long long in_stride, const float* g, con
 #define TSSP_LN_CASE(d, NS, VPL) \
     case d: TSSP_CUDA(launch_pdl(layernorm_bf16_slab_kernel<NS, VPL>, dim3(grid), dim3(threads), 0, s, x, in_stride, g, b, o, rows, eps, rev, hint)); break;
     switch (D) {
+        case 192: TSSP_CUDA(launch_pdl(layernorm_bf16_slab64_kernel<3>, dim3(grid), dim3(threads), 0, s, x, in_stride, g, b, o, rows, eps, rev, hint)); break;
         TSSP_LN_CASE(128, 1, 1)
         TSSP_LN_CASE(256, 1, 2)
         TSSP_LN_CASE(384, 3, 1)
@@ -574,6 +580,8 @@ struct tssp_engine {
     tssp_config_t cfg;
     int device;
     int T, M_cap, Kp, G;
+    int prefix;     // tokens ahead of the patches: 1 (CLS) or 2 (CLS, DeiT distillation token)
+    bool dist_head; // a distillation head is loaded: logits = (cls_head(row 0) + dist_head(row 1)) / 2
     int sumF;  // sum of current F over blocks (score vector length)
     int ldn;   // pitch of the per-image norm buffer = sum of F_cap
     bool weights_loaded;
@@ -582,8 +590,8 @@ struct tssp_engine {
     std::vector<size_t> alloc_bytes;
     std::vector<tssp::BlockWeights> blk;
     // global weights
-    __nv_bfloat16 *patch_w, *head0_w, *head_w;
-    float *posmod, *final_ln_w, *final_ln_b, *head_b;
+    __nv_bfloat16 *patch_w, *head0_w, *head_w, *head_dist_w;  // with a distillation head both heads are packed at 0.5 scale
+    float *posmod, *final_ln_w, *final_ln_b, *head_b, *head_dist_b;
     int Cp, Hhp;  // padded classes / head hidden
     // workspace
     float* pixels[2];          // double-buffered staging of host pixel batches
@@ -596,7 +604,8 @@ struct tssp_engine {
     bool s1_fresh;         // no batch since tssp_s1_reset: nothing is running that a host copy could hide behind
     int next_slot, staged_slot;
     int host_slot;         // slot of the host batch staged by the running entry point (-1: none); see finish_host_batch
-    __nv_bfloat16 *patchA, *xn, *qkv, *ctx, *h, *cls_norm, *head_hidden;
+    __nv_bfloat16 *patchA, *xn, *qkv, *ctx, *h, *head_hidden;
+    __nv_bfloat16* cls_norm;   // final LayerNorm of the prefix rows: [prefix][max_images][D] (CLS rows, then distillation rows)
     float *x, *partials, *norms, *scores, *logits;
     float* qk_norms;  // [M_cap][2*heads]: |q|^2 and |k|^2 per (token, head), written by the QKV GEMM epilogue
     size_t partials_stride;  // floats between two blocks' partial buffers
@@ -679,12 +688,14 @@ static int dev_alloc(tssp_engine* e, Tp** out, size_t count) {
     return 0;
 }
 
-static int validate(const tssp_config_t& c) {
+static int validate(const tssp_config_t& c, int prefix) {
+    if (prefix < 1 || prefix > 2) return fail("config: prefix_tokens=%d must be 1 (CLS) or 2 (CLS and distillation token)", prefix);
     if (c.n_blocks < 1 || c.n_blocks > TSSP_MAX_BLOCKS) return fail("config: n_blocks=%d out of range", c.n_blocks);
-    if (c.hidden % 128 || c.hidden > 1024 || c.hidden < 128) return fail("config: hidden=%d must be a multiple of 128 in [128,1024]", c.hidden);
+    if ((c.hidden % 128 && c.hidden != 192) || c.hidden > 1024 || c.hidden < 128)
+        return fail("config: hidden=%d must be 192 or a multiple of 128 in [128,1024]", c.hidden);
     if (c.heads * 64 != c.hidden) return fail("config: head_dim must be 64 (hidden=%d heads=%d)", c.hidden, c.heads);
     if (c.patch_size % 8 || c.image_size % c.patch_size) return fail("config: image %d / patch %d unsupported", c.image_size, c.patch_size);
-    const int G = c.image_size / c.patch_size, T = G * G + 1;
+    const int G = c.image_size / c.patch_size, T = G * G + prefix;
     if (T < 32 || T > ATL_MAX_T) return fail("config: tokens per image T=%d must be in [32,%d]", T, ATL_MAX_T);
     if ((c.channels * c.patch_size * c.patch_size) % 8) return fail("config: patch vector length not a multiple of 8");
     if (c.max_images < 1) return fail("config: max_images=%d", c.max_images);
@@ -693,8 +704,8 @@ static int validate(const tssp_config_t& c) {
     return 0;
 }
 
-static int engine_create(const tssp_config_t* cfg, int device, tssp_engine** out) {
-    TSSP_TRY(validate(*cfg));
+static int engine_create(const tssp_config_t* cfg, int prefix, int device, tssp_engine** out) {
+    TSSP_TRY(validate(*cfg, prefix));
     int n_dev = 0;
     TSSP_CUDA(cudaGetDeviceCount(&n_dev));
     if (device < 0 || device >= n_dev) return fail("device %d out of range (%d visible)", device, n_dev);
@@ -709,7 +720,9 @@ static int engine_create(const tssp_config_t* cfg, int device, tssp_engine** out
     e->weights_loaded = false;
     const int D = cfg->hidden, B = cfg->n_blocks;
     e->G = cfg->image_size / cfg->patch_size;
-    e->T = e->G * e->G + 1;
+    e->prefix = prefix;
+    e->dist_head = false;
+    e->T = e->G * e->G + prefix;
     e->M_cap = cfg->max_images * e->T;
     e->Kp = cfg->channels * cfg->patch_size * cfg->patch_size;
     e->Cp = round_up(cfg->n_classes > 0 ? cfg->n_classes : 8, 8);
@@ -724,6 +737,12 @@ static int engine_create(const tssp_config_t* cfg, int device, tssp_engine** out
     A(&e->head0_w, static_cast<size_t>(e->Hhp) * D);
     A(&e->head_w, static_cast<size_t>(e->Cp) * (e->Hhp > 0 ? e->Hhp : D));
     A(&e->head_b, e->Cp);
+    e->head_dist_w = nullptr;
+    e->head_dist_b = nullptr;
+    if (prefix == 2 && cfg->n_classes > 0) {
+        A(&e->head_dist_w, static_cast<size_t>(e->Cp) * D);
+        A(&e->head_dist_b, e->Cp);
+    }
     e->blk.resize(B);
     int Fp_max = 0, off = 0;
     for (int b = 0; b < B; ++b) {
@@ -760,7 +779,7 @@ static int engine_create(const tssp_config_t* cfg, int device, tssp_engine** out
     A(&e->partials, e->partials_stride * B);
     A(&e->norms, static_cast<size_t>(cfg->max_images) * e->ldn);
     A(&e->scores, e->ldn);
-    A(&e->cls_norm, static_cast<size_t>(cfg->max_images) * D);
+    A(&e->cls_norm, static_cast<size_t>(prefix) * cfg->max_images * D);
     A(&e->head_hidden, static_cast<size_t>(cfg->max_images) * (e->Hhp > 0 ? e->Hhp : 8));
     A(&e->logits, static_cast<size_t>(cfg->max_images) * e->Cp);
     A(&e->preds, cfg->max_images);
@@ -795,24 +814,25 @@ static int engine_create(const tssp_config_t* cfg, int device, tssp_engine** out
     return 0;
 }
 
-// posmod[0] = cls + pos[0]; posmod[t>0] = pos[t] + conv_bias  (so the patch GEMM needs no bias and the CLS row,
-// whose im2col row is zero, receives exactly cls + pos[0]: HF ViTEmbeddings.forward)
-__global__ void build_posmod_kernel(const float* __restrict__ pos, const float* __restrict__ cls,
-                                    const float* __restrict__ conv_b, float* __restrict__ out, int T, int D) {
+// posmod[0] = cls + pos[0]; with two prefix tokens posmod[1] = dist + pos[1]; posmod[t >= prefix] = pos[t] + conv_bias
+// (so the patch GEMM needs no bias and the prefix rows, whose im2col rows are zero, receive exactly token + pos:
+// HF ViTEmbeddings.forward / DeiTEmbeddings.forward)
+__global__ void build_posmod_kernel(const float* __restrict__ pos, const float* __restrict__ cls, const float* __restrict__ dist,
+                                    const float* __restrict__ conv_b, float* __restrict__ out, int T, int D, int prefix) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= T * D) return;
     const int t = i / D, d = i % D;
-    out[i] = pos[i] + (t == 0 ? cls[d] : (conv_b != nullptr ? conv_b[d] : 0.0f));
+    out[i] = pos[i] + (t < prefix ? (t == 0 ? cls[d] : dist[d]) : (conv_b != nullptr ? conv_b[d] : 0.0f));
 }
 
-__global__ void copy_pad_f32_kernel(const float* __restrict__ in, int n, float* __restrict__ out, int n_pad) {
+__global__ void copy_pad_f32_kernel(const float* __restrict__ in, int n, float* __restrict__ out, int n_pad, float scale) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n_pad) out[i] = (in != nullptr && i < n) ? in[i] : 0.0f;
+    if (i < n_pad) out[i] = (in != nullptr && i < n) ? in[i] * scale : 0.0f;
 }
 
 // out[0, n_pad) = in[0, n), zero padded
-static int copy_vec(const float* in, int n, float* out, int n_pad, cudaStream_t s) {
-    copy_pad_f32_kernel<<<ceil_div(n_pad, 256), 256, 0, s>>>(in, n, out, n_pad);
+static int copy_vec(const float* in, int n, float* out, int n_pad, cudaStream_t s, float scale = 1.0f) {
+    copy_pad_f32_kernel<<<ceil_div(n_pad, 256), 256, 0, s>>>(in, n, out, n_pad, scale);
     TSSP_LAUNCH_CHECK("copy_pad_f32_kernel");
     return 0;
 }
@@ -832,16 +852,33 @@ static int pack_ffn(tssp_engine* e, int b, int F, const float* fc1_w, const floa
 static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cudaStream_t s) {
     const tssp_config_t& c = e->cfg;
     const int D = c.hidden, B = c.n_blocks;
-    if (n_entries != TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT) return fail("load_weights: expected %d pointers, got %d", TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT, n_entries);
+    const int n_expected = TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT + (e->prefix == 2 ? TSSP_WX_COUNT : 0);
+    if (n_entries != n_expected)
+        return fail("load_weights: expected %d pointers for %d prefix token(s), got %d", n_expected, e->prefix, n_entries);
     auto need = [&](int idx, const char* name) -> int { return t[idx] == nullptr ? fail("load_weights: %s is NULL", name) : 0; };
     TSSP_TRY(need(TSSP_W_PATCH_W, "patch_w")); TSSP_TRY(need(TSSP_W_CLS, "cls_token")); TSSP_TRY(need(TSSP_W_POS, "pos_embed"));
     TSSP_TRY(need(TSSP_W_FINAL_LN_W, "final_ln_w")); TSSP_TRY(need(TSSP_W_FINAL_LN_B, "final_ln_b"));
+    const float* const* x = t + TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT;  // extension entries (two prefix tokens only)
+    const bool dist_head = e->prefix == 2 && x[TSSP_WX_HEAD_DIST_W] != nullptr;
+    if (e->prefix == 2) {
+        if (x[TSSP_WX_DIST_TOKEN] == nullptr) return fail("load_weights: distillation token is NULL");
+        if (dist_head && c.n_classes <= 0) return fail("load_weights: a distillation head needs n_classes > 0");
+        if (dist_head && c.head_hidden > 0) return fail("load_weights: a distillation head cannot be combined with a Sequential head");
+    }
     TSSP_TRY(op_cast(t[TSSP_W_PATCH_W], D, e->Kp, e->Kp, e->patch_w, D, e->Kp, e->Kp, s));
-    build_posmod_kernel<<<ceil_div(e->T * D, 256), 256, 0, s>>>(t[TSSP_W_POS], t[TSSP_W_CLS], t[TSSP_W_PATCH_B], e->posmod, e->T, D);
+    build_posmod_kernel<<<ceil_div(e->T * D, 256), 256, 0, s>>>(t[TSSP_W_POS], t[TSSP_W_CLS], e->prefix == 2 ? x[TSSP_WX_DIST_TOKEN] : nullptr,
+                                                               t[TSSP_W_PATCH_B], e->posmod, e->T, D, e->prefix);
     TSSP_LAUNCH_CHECK("build_posmod_kernel");
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_W], D, e->final_ln_w, D, s));
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_B], D, e->final_ln_b, D, s));
-    if (c.n_classes > 0) {
+    if (c.n_classes > 0 && dist_head) {
+        // (cls_head(x0) + dist_head(x1)) / 2 as two GEMMs into the same logits (run_head): both heads at half scale
+        TSSP_TRY(need(TSSP_W_HEAD_W, "head_w"));
+        TSSP_TRY(op_cast(t[TSSP_W_HEAD_W], c.n_classes, D, D, e->head_w, e->Cp, D, D, s, 0.5f));
+        TSSP_TRY(copy_vec(t[TSSP_W_HEAD_B], c.n_classes, e->head_b, e->Cp, s, 0.5f));
+        TSSP_TRY(op_cast(x[TSSP_WX_HEAD_DIST_W], c.n_classes, D, D, e->head_dist_w, e->Cp, D, D, s, 0.5f));
+        TSSP_TRY(copy_vec(x[TSSP_WX_HEAD_DIST_B], c.n_classes, e->head_dist_b, e->Cp, s, 0.5f));
+    } else if (c.n_classes > 0) {
         TSSP_TRY(need(TSSP_W_HEAD_W, "head_w"));
         if (c.head_hidden > 0) {
             TSSP_TRY(need(TSSP_W_HEAD0_W, "head0_w"));
@@ -876,6 +913,7 @@ static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cud
         TSSP_TRY(pack_ffn(e, b, bw.F, w[TSSP_BW_FC1_W], w[TSSP_BW_FC1_B], w[TSSP_BW_FC2_W], s));
         TSSP_TRY(copy_vec(w[TSSP_BW_FC2_B], D, bw.fc2_b, D, s));
     }
+    e->dist_head = dist_head;
     e->weights_loaded = true;
     return 0;
 }
@@ -1027,7 +1065,7 @@ static unsigned long long block_mask(const int32_t* flags, int B) {
 // caller's / the staged pixels, kept outside the captured chains so that those do not depend on where a batch lives
 static int run_im2col(tssp_engine* e, const float* dev_pixels, int n, cudaStream_t s) {
     const tssp_config_t& c = e->cfg;
-    TSSP_PROF(KC_MISC, s, op_im2col(dev_pixels, e->patchA, n, c.channels, c.image_size, c.image_size, c.patch_size, s));
+    TSSP_PROF(KC_MISC, s, op_im2col(dev_pixels, e->patchA, n, c.channels, c.image_size, c.image_size, c.patch_size, s, e->prefix));
     if (e->staged_slot >= 0) {  // the host-staged pixel buffer may be refilled once im2col has read it
         TSSP_CUDA(cudaEventRecord(e->ev_consumed[e->staged_slot], s));
         e->staged_slot = -1;
@@ -1058,6 +1096,8 @@ enum Fc1Mode { FC1_PLAIN = 0, FC1_SCORE = 1 };
 // output projection, the LayerNorm before the FFN, fc1 and fc2 run on the n CLS rows in place (tensor maps over x / ctx with
 // a row pitch of T rows) instead of on n * T rows; the other rows of x are left as they are, nobody reads them. One block
 // forward of the 13 per Stage-2 candidate sweep and of every evaluation loses two thirds of its work.
+// With a distillation head the classifier also reads row 1 (DeiT's distillation token): the row-wise part then runs a second
+// time on the n rows 1, at base offset D with the same pitch. (Attention's first query tile already covers both rows.)
 static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_mode, bool run_fc2, cudaStream_t s, bool cls_only = false) {
     const tssp_config_t& c = e->cfg;
     const int M = n * e->T, D = c.hidden;
@@ -1065,13 +1105,25 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     cls_only = cls_only && fc1_mode == FC1_PLAIN && run_fc2;
     const int rows = cls_only ? n : M;              // rows the row-wise part of the block works on
     const int pitch = cls_only ? e->T * D : D;      // their distance in x / ctx
-    if (e->attn_present[b] && !skip_attn) {
+    const bool attn = e->attn_present[b] && !skip_attn;
+    if (attn) {
         TSSP_PROF(KC_LN, s, op_layernorm(e->x, D, w.ln1_w, w.ln1_b, e->xn, M, D, c.ln_eps, s));
         TSSP_PROF(KC_QKV, s, gemm(EPI_BF16_ROWNORM, e->xn, D, w.qkv_w, D, e->qkv, 3 * D, M, 3 * D, D, w.qkv_b, nullptr, 0, e->T, 0, s,
                                   e->qk_norms, 2 * c.heads, 2 * c.heads));
         TSSP_PROF(KC_ATTN, s, op_attention(e->qkv, e->ctx, n, e->T, c.heads, D, s, e->qk_norms, 2 * c.heads, /*first_tile_only=*/cls_only));
-        TSSP_PROF(KC_PROJ, s, gemm(EPI_F32, e->ctx, pitch, w.proj_w, D, e->x, pitch, rows, D, D, w.proj_b, nullptr, 0, e->T, 1, s));
     }
+    if (cls_only && e->dist_head) {
+        for (int r = 0; r < 2; ++r) {
+            float* xr = e->x + static_cast<size_t>(r) * D;
+            if (attn) TSSP_PROF(KC_PROJ, s, gemm(EPI_F32, e->ctx + static_cast<size_t>(r) * D, pitch, w.proj_w, D, xr, pitch, n, D, D, w.proj_b,
+                                                 nullptr, 0, e->T, 1, s));
+            TSSP_PROF(KC_LN, s, op_layernorm(xr, pitch, w.ln2_w, w.ln2_b, e->xn, n, D, c.ln_eps, s));
+            TSSP_PROF(KC_FC1, s, gemm(EPI_BF16_GELU, e->xn, D, w.fc1_w, D, e->h, w.Fp, n, w.Fp, D, w.fc1_b, nullptr, 0, e->T, 0, s));
+            TSSP_PROF(KC_FC2, s, gemm(EPI_F32, e->h, w.Fp, w.fc2_w, w.Fp, xr, pitch, n, D, w.Fp, w.fc2_b, nullptr, 0, e->T, 1, s));
+        }
+        return 0;
+    }
+    if (attn) TSSP_PROF(KC_PROJ, s, gemm(EPI_F32, e->ctx, pitch, w.proj_w, D, e->x, pitch, rows, D, D, w.proj_b, nullptr, 0, e->T, 1, s));
     TSSP_PROF(KC_LN, s, op_layernorm(e->x, pitch, w.ln2_w, w.ln2_b, e->xn, rows, D, c.ln_eps, s, /*stream_in=*/!cls_only));
     if (fc1_mode == FC1_SCORE) {
         const int mode = c.score_point == 1 ? EPI_BF16_GELU_SCORE_PRE : EPI_BF16_GELU_SCORE;
@@ -1086,12 +1138,22 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     return 0;
 }
 
-// final LayerNorm on the CLS rows + classification head -> e->logits [n, Cp]
+// final LayerNorm on the CLS rows + classification head -> e->logits [n, Cp]. With a distillation head (DeiT
+// ForImageClassificationWithTeacher, timm's distilled models in eval) the rows 1 are normalised too, and
+// logits = (cls_head(row 0) + dist_head(row 1)) / 2: the CLS GEMM stores half its result, the distillation GEMM adds half of
+// its own (both heads are packed at 0.5 scale, exact in bf16 and fp32), one fp32 rounding of the sum as in the module.
 static int run_head(tssp_engine* e, int n, cudaStream_t s) {
     const tssp_config_t& c = e->cfg;
     const int D = c.hidden;
     if (c.n_classes <= 0) return fail("model has no classification head: logits unavailable");
     TSSP_PROF(KC_LN, s, op_layernorm(e->x, static_cast<long long>(e->T) * D, e->final_ln_w, e->final_ln_b, e->cls_norm, n, D, c.ln_eps, s));
+    if (e->dist_head) {
+        __nv_bfloat16* dist_norm = e->cls_norm + static_cast<size_t>(n) * D;
+        TSSP_PROF(KC_LN, s, op_layernorm(e->x + D, static_cast<long long>(e->T) * D, e->final_ln_w, e->final_ln_b, dist_norm, n, D, c.ln_eps, s));
+        TSSP_PROF(KC_HEAD, s, gemm(EPI_F32, e->cls_norm, D, e->head_w, D, e->logits, e->Cp, n, e->Cp, D, e->head_b, nullptr, 0, e->T, 0, s));
+        TSSP_PROF(KC_HEAD, s, gemm(EPI_F32, dist_norm, D, e->head_dist_w, D, e->logits, e->Cp, n, e->Cp, D, e->head_dist_b, nullptr, 0, e->T, 1, s));
+        return 0;
+    }
     if (c.head_hidden > 0) {
         TSSP_PROF(KC_HEAD, s, gemm(EPI_BF16_GELU, e->cls_norm, D, e->head0_w, D, e->head_hidden, e->Hhp, n, e->Hhp, D, nullptr, nullptr, 0, e->T, 0, s));
         TSSP_PROF(KC_HEAD, s, gemm(EPI_F32, e->head_hidden, e->Hhp, e->head_w, e->Hhp, e->logits, e->Cp, n, e->Cp, e->Hhp, e->head_b, nullptr, 0, e->T, 0, s));
@@ -1214,11 +1276,13 @@ int tssp_profile_end(double* ms_per_class, unsigned long long* launches_per_clas
     return 0;
 }
 
-int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out) {
+int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out) {
     TSSP_ENTRY();
     if (cfg == nullptr || out == nullptr) return fail("tssp_create: NULL argument");
-    return engine_create(cfg, device, out);
+    return engine_create(cfg, prefix_tokens, device, out);
 }
+
+int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out) { return tssp_create_ex(cfg, 1, device, out); }
 
 int tssp_destroy(tssp_handle_t h) {
     TSSP_ENTRY();
@@ -1387,6 +1451,7 @@ static int forward_logits(tssp_engine* h, const float* pixels, int n, int pixels
 int tssp_forward_logits(tssp_handle_t h, const float* pixels, int n, int pixels_on_host, const int32_t* skip_attn,
                         float* logits, int out_on_host, void* stream) {
     TSSP_ENGINE_ENTRY(h, "tssp_forward_logits");
+    if (h->cfg.n_classes <= 0) return fail("tssp_forward_logits: model has no classification head: logits unavailable");
     if (logits == nullptr) return fail("tssp_forward_logits: NULL argument");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     return finish_host_batch(h, s, false, forward_logits(h, pixels, n, pixels_on_host, skip_attn, logits, out_on_host, s));
@@ -1543,6 +1608,15 @@ int tssp_op_gemm(int mode, const void* A, int lda, const void* W, int ldw, void*
     if (A == nullptr || W == nullptr || C == nullptr) return fail("tssp_op_gemm: NULL argument");
     return gemm(mode, A, lda, W, ldw, C, ldc, M, N, K, bias, partials, ldp, tokens_per_image, reduce_add, static_cast<cudaStream_t>(stream));
 }
+int tssp_op_gemm_rownorm(const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K, const float* bias,
+                         float* rownorm, int ld_rownorm, int rownorm_chunks, void* stream) {
+    TSSP_ENTRY();
+    if (A == nullptr || W == nullptr || C == nullptr || rownorm == nullptr) return fail("tssp_op_gemm_rownorm: NULL argument");
+    if (rownorm_chunks < 0 || rownorm_chunks > ld_rownorm || rownorm_chunks * 64 > N)
+        return fail("tssp_op_gemm_rownorm: %d chunks of 64 columns with ld_rownorm=%d and N=%d", rownorm_chunks, ld_rownorm, N);
+    return gemm(EPI_BF16_ROWNORM, A, lda, W, ldw, C, ldc, M, N, K, bias, nullptr, 0, 0, 0, static_cast<cudaStream_t>(stream), rownorm,
+                ld_rownorm, rownorm_chunks);
+}
 int tssp_op_score_finish(const float* partials, int ldp, float* norms, int ldn, int n_img, int T, int F, float* scores, void* stream) {
     TSSP_ENTRY();
     if (partials == nullptr || norms == nullptr) return fail("tssp_op_score_finish: NULL argument");
@@ -1570,10 +1644,13 @@ int tssp_debug_attention_trace(long long* device_buf) {
     ++g_launch_epoch;
     return 0;
 }
-int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream) {
+int tssp_op_im2col_ex(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens, void* stream) {
     TSSP_ENTRY();
     if (pixels == nullptr || out_bf16 == nullptr) return fail("tssp_op_im2col: NULL argument");
-    return op_im2col(pixels, out_bf16, n_img, C, H, W, P, static_cast<cudaStream_t>(stream));
+    return op_im2col(pixels, out_bf16, n_img, C, H, W, P, static_cast<cudaStream_t>(stream), prefix_tokens);
+}
+int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream) {
+    return tssp_op_im2col_ex(pixels, out_bf16, n_img, C, H, W, P, 1, stream);
 }
 int tssp_op_cast_bf16(const float* in, int rows, int cols, int ld_in, void* out_bf16, int rows_pad, int cols_pad, int ld_out, void* stream) {
     TSSP_ENTRY();

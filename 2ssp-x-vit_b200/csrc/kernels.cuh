@@ -11,26 +11,29 @@ namespace tssp {
 // fp32 [rows, cols] (pitch ld_in) -> bf16 [rows_pad, cols_pad] (pitch ld_out), zero padded.
 // Used once per weight matrix when a model is loaded (nn.Linear weights are already [N, K] K-major).
 // ------------------------------------------------------------------------------------------------
+// `scale` multiplies every element before the rounding (1 for every matrix except the averaged two-head classifier, which
+// packs both heads at 0.5: a power of two, so bf16(0.5 w) == 0.5 bf16(w) barring subnormals).
 __global__ void cast_pad_bf16_kernel(const float* __restrict__ in, int rows, int cols, int ld_in,
-                                     __nv_bfloat16* __restrict__ out, int rows_pad, int cols_pad, int ld_out) {
+                                     __nv_bfloat16* __restrict__ out, int rows_pad, int cols_pad, int ld_out, float scale) {
     const long long total = static_cast<long long>(rows_pad) * cols_pad;
     for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
          i += static_cast<long long>(gridDim.x) * blockDim.x) {
         const int r = static_cast<int>(i / cols_pad);
         const int c = static_cast<int>(i % cols_pad);
-        const float v = (r < rows && c < cols) ? in[static_cast<size_t>(r) * ld_in + c] : 0.0f;
+        const float v = (r < rows && c < cols) ? in[static_cast<size_t>(r) * ld_in + c] * scale : 0.0f;
         out[static_cast<size_t>(r) * ld_out + c] = __float2bfloat16_rn(v);
     }
 }
 
 // ------------------------------------------------------------------------------------------------
 // Patch extraction for the patch-embedding GEMM (HF ViTPatchEmbeddings: Conv2d(C, D, P, stride P) ==
-// GEMM over non-overlapping patches). pixels fp32 [n, C, H, W] -> A bf16 [n*T, C*P*P] where row
-// img*T + 0 is the (all-zero) CLS slot and row img*T + 1 + (py*G + px) holds patch (py, px) flattened
-// as (c, ky, kx) -- the order of Conv2d.weight.view(D, -1). Each thread converts 8 consecutive kx.
+// GEMM over non-overlapping patches). pixels fp32 [n, C, H, W] -> A bf16 [n*T, C*P*P] where rows
+// img*T + r, r < prefix, are the (all-zero) slots of the prefix tokens (CLS; CLS and distillation for DeiT) and row
+// img*T + prefix + (py*G + px) holds patch (py, px) flattened as (c, ky, kx) -- the order of
+// Conv2d.weight.view(D, -1). Each thread converts 8 consecutive kx.
 // ------------------------------------------------------------------------------------------------
 __global__ void im2col_patches_kernel(const float* __restrict__ pixels, __nv_bfloat16* __restrict__ out, int n_img,
-                                      int C, int H, int W, int P, int T) {
+                                      int C, int H, int W, int P, int T, int prefix) {
     const int G = W / P;
     const int Kp = C * P * P;
     const int k8_per_row = Kp / 8;
@@ -42,8 +45,8 @@ __global__ void im2col_patches_kernel(const float* __restrict__ pixels, __nv_bfl
         const int t = static_cast<int>(row % T);
         const int img = static_cast<int>(row / T);
         uint4 packed = make_uint4(0u, 0u, 0u, 0u);
-        if (t > 0) {
-            const int patch = t - 1;
+        if (t >= prefix) {
+            const int patch = t - prefix;
             const int py = patch / G, px = patch % G;
             const int k = k8 * 8;
             const int c = k / (P * P);
@@ -179,6 +182,78 @@ __global__ void __launch_bounds__(256) layernorm_bf16_slab_kernel(const float* _
             }
             if constexpr (VPL == 2) reinterpret_cast<uint4*>(dst)[i * 32 + lane] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
             else reinterpret_cast<uint2*>(dst)[i * 32 + lane] = make_uint2(pk[0], pk[1]);
+        }
+    }
+}
+
+// The same persistent walk for widths that are a multiple of 64 but not of 128 (D = 192: DeiT-Ti, ViT-Ti): a row is
+// NSLAB slabs of 64 elements, a lane owns two consecutive elements of each slab -- one 64-bit load and one bf16x2 (32-bit)
+// store per slab, so a warp still reads and writes whole 256-byte / 128-byte rows of a slab.
+template <int NSLAB>
+__global__ void __launch_bounds__(256) layernorm_bf16_slab64_kernel(const float* __restrict__ x, long long in_stride,
+                                                                    const float* __restrict__ gamma,
+                                                                    const float* __restrict__ beta,
+                                                                    __nv_bfloat16* __restrict__ out, int rows, float eps,
+                                                                    int reverse, int stream_in) {
+    constexpr int D = NSLAB * 64;
+    const uint64_t in_policy = ptx::l2_policy_evict_first();
+    auto ldx = [&](const float2* p) { return stream_in ? ptx::ld_global_v2_hint(p, in_policy) : *p; };
+    if (reverse) {
+        x += static_cast<size_t>(rows - 1) * in_stride;
+        out += static_cast<size_t>(rows - 1) * D;
+    }
+    const long long xs = reverse ? -in_stride : in_stride;
+    const long long os = reverse ? -static_cast<long long>(D) : static_cast<long long>(D);
+    ptx::griddep_launch_dependents();
+    ptx::griddep_wait();
+    const int lane = threadIdx.x & 31;
+    const int warp_global = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int warp_stride = gridDim.x * (blockDim.x >> 5);
+    const float2* g2 = reinterpret_cast<const float2*>(gamma);
+    const float2* b2 = reinterpret_cast<const float2*>(beta);
+    float2 gm[NSLAB], bt[NSLAB];
+#pragma unroll
+    for (int i = 0; i < NSLAB; ++i) {
+        gm[i] = __ldg(g2 + i * 32 + lane);
+        bt[i] = __ldg(b2 + i * 32 + lane);
+    }
+    float2 nxt[NSLAB];
+    int row = warp_global;
+    if (row < rows) {
+        const float2* src = reinterpret_cast<const float2*>(x + row * xs);
+#pragma unroll
+        for (int i = 0; i < NSLAB; ++i) nxt[i] = ldx(src + i * 32 + lane);
+    }
+    for (; row < rows; row += warp_stride) {
+        float2 v[NSLAB];
+#pragma unroll
+        for (int i = 0; i < NSLAB; ++i) v[i] = nxt[i];
+        const int next_row = row + warp_stride;
+        if (next_row < rows) {
+            const float2* src = reinterpret_cast<const float2*>(x + next_row * xs);
+#pragma unroll
+            for (int i = 0; i < NSLAB; ++i) nxt[i] = ldx(src + i * 32 + lane);
+        }
+        float sum = 0.f;
+#pragma unroll
+        for (int i = 0; i < NSLAB; ++i) sum += v[i].x + v[i].y;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+        const float mean = sum * (1.0f / D);
+        float sq = 0.f;
+#pragma unroll
+        for (int i = 0; i < NSLAB; ++i) {
+            const float a = v[i].x - mean, b = v[i].y - mean;
+            sq += a * a + b * b;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
+        const float rstd = 1.0f / sqrtf(sq * (1.0f / D) + eps);
+        __nv_bfloat16* dst = out + row * os;
+#pragma unroll
+        for (int i = 0; i < NSLAB; ++i) {
+            __nv_bfloat162 pk = __floats2bfloat162_rn((v[i].x - mean) * rstd * gm[i].x + bt[i].x, (v[i].y - mean) * rstd * gm[i].y + bt[i].y);
+            reinterpret_cast<__nv_bfloat162*>(dst)[i * 32 + lane] = pk;
         }
     }
 }

@@ -388,6 +388,11 @@ __device__ __forceinline__ float4 ld_global_v4_hint(const float4* p, uint64_t po
                  : "l"(p), "l"(policy));
     return v;
 }
+__device__ __forceinline__ float2 ld_global_v2_hint(const float2* p, uint64_t policy) {
+    float2 v;
+    asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v2.f32 {%0, %1}, [%2], %3;" : "=f"(v.x), "=f"(v.y) : "l"(p), "l"(policy));
+    return v;
+}
 
 // 3-D tile store shared -> global (bulk async group); elements outside the tensor are not written
 __device__ __forceinline__ void tma_store_3d(const void* tmap, uint32_t smem_src, int32_t c0, int32_t c1, int32_t c2) {

@@ -60,6 +60,18 @@ def gemm(mode: int, a: torch.Tensor, w: torch.Tensor, out: torch.Tensor, bias: t
     return out
 
 
+def gemm_rownorm(a: torch.Tensor, w: torch.Tensor, out: torch.Tensor, bias: torch.Tensor | None, chunks: int) -> torch.Tensor:
+    """The QKV epilogue: out (bf16) = a @ w^T + bias; returns [M, chunks] fp32 sums of squares of 64-column chunks."""
+    _need_cuda(a, w, out, bias)
+    M, K = a.shape
+    N = w.shape[0]
+    rownorm = torch.full((M, chunks), float("nan"), device=a.device, dtype=torch.float32)
+    lib = L.load()
+    L.check(lib.tssp_op_gemm_rownorm(L.ptr(a), a.stride(0), L.ptr(w), w.stride(0), L.ptr(out), out.stride(0), M, N, K, L.ptr(bias),
+                                     L.ptr(rownorm), chunks, chunks, L.current_stream()))
+    return rownorm
+
+
 def score_finish(partials: torch.Tensor, n_img: int, T: int, F: int, scores: torch.Tensor | None = None) -> torch.Tensor:
     """partials [ceil(M/32)*2, ldp] -> per-image norms [n_img, F]; optionally scores[F] += sum over images."""
     _need_cuda(partials, scores)
@@ -93,15 +105,16 @@ def attention(qkv: torch.Tensor, n_img: int, T: int, heads: int) -> torch.Tensor
     return ctx
 
 
-def im2col(pixels: torch.Tensor, patch: int) -> torch.Tensor:
+def im2col(pixels: torch.Tensor, patch: int, prefix: int = 1) -> torch.Tensor:
+    """[n * T, C*P*P] bf16 patch rows, `prefix` zero rows ahead of every image's patches (2 for DeiT)."""
     _need_cuda(pixels)
     if pixels.dtype != torch.float32 or not pixels.is_contiguous():
         raise ValueError("im2col: pixels must be a contiguous float32 tensor [n, C, H, W]")
     n, c, h, w = pixels.shape
-    T = (h // patch) * (w // patch) + 1
+    T = (h // patch) * (w // patch) + prefix
     out = torch.empty(n * T, c * patch * patch, device=pixels.device, dtype=torch.bfloat16)
     lib = L.load()
-    L.check(lib.tssp_op_im2col(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, L.current_stream()))
+    L.check(lib.tssp_op_im2col_ex(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, L.current_stream()))
     return out
 
 

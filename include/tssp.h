@@ -37,11 +37,12 @@ typedef struct tssp_engine* tssp_handle_t;
 
 /* Model anatomy, as discovered by the reference's _get_encoder/_gather_mlp_pairs walkers
  * (src/vit_pruning.py:28-75) on an HF ViTForImageClassification or a timm VisionTransformer.
- * Tokens per image T = (image_size / patch_size)^2 + 1 must lie in [32, 1025]: ViT-x/16 up to 512x512 (T = 1025),
- * ViT-x/8 up to 256x256; tssp_create rejects other shapes before it touches a device. */
+ * Tokens per image T = (image_size / patch_size)^2 + prefix tokens (1 for ViT, 2 for DeiT: see tssp_create_ex) must lie
+ * in [32, 1025]: ViT-x/16 up to 512x512 (T = 1025), ViT-x/8 up to 256x256; tssp_create rejects other shapes before it
+ * touches a device. */
 typedef struct tssp_config {
     int32_t n_blocks;                      /* B: encoder blocks */
-    int32_t hidden;                        /* D: multiple of 128, <= 1024 */
+    int32_t hidden;                        /* D: 192 (DeiT-Ti, ViT-Ti) or a multiple of 128, <= 1024 */
     int32_t heads;                         /* D / heads must be 64 */
     int32_t image_size;                    /* H = W, multiple of patch_size */
     int32_t patch_size;                    /* P: multiple of 8 */
@@ -82,11 +83,25 @@ enum tssp_block_weight_index {
     TSSP_BW_FC2_W, TSSP_BW_FC2_B, /* [D, F] / [D] */
     TSSP_BW_COUNT
 };
+/* Engines with two prefix tokens (tssp_create_ex) take TSSP_WX_COUNT more entries after the per-block ones. */
+enum tssp_weight_ext_index {
+    TSSP_WX_DIST_TOKEN = 0, /* [D] distillation token (required) */
+    TSSP_WX_HEAD_DIST_W,    /* [C, D] distillation head, or NULL: the classifier reads the CLS row only */
+    TSSP_WX_HEAD_DIST_B,    /* [C] or NULL */
+    TSSP_WX_COUNT
+};
 
 int tssp_abi_version(void);
 const char* tssp_last_error(void);
 
 int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out);
+/* Same, for models with `prefix_tokens` (1 or 2) tokens ahead of the patches; tssp_create is this with 1. Two is DeiT
+ * (transformers models/deit/modeling_deit.py DeiTEmbeddings.forward: [CLS, distillation token, patches] + positions;
+ * timm VisionTransformerDistilled): T = G^2 + 2, and the weight table carries the TSSP_WX_* entries. With a distillation
+ * head the logits are (cls_head(row 0) + dist_head(row 1)) / 2, the eval-mode output of
+ * DeiTForImageClassificationWithTeacher.forward and of timm's distilled models; a Sequential head (head_hidden > 0) cannot
+ * be combined with one. Without it (DeiTForImageClassification.forward) the head reads the CLS row only. */
+int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out);
 int tssp_destroy(tssp_handle_t h);
 /* tssp_destroy parks the engine's device buffers in a per-process pool (exact-size reuse by the next tssp_create; capped
  * by TSSP_POOL_MB, default 16384, 0 = no pool); this returns all parked buffers to the driver. */
@@ -151,6 +166,10 @@ int tssp_ffn_gather_batch(int n_blocks, const float* const* fc1_w, const float* 
  * partials, 3 same with pre-activation scores, 4 fp32 (reduce_add: C += ...). A, W bf16; lda/ldw/ldc in elements. */
 int tssp_op_gemm(int mode, const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K,
                  const float* bias, float* partials, int ldp, int tokens_per_image, int reduce_add, void* stream);
+/* the QKV form (mode 5): bf16 C = A W^T + bias, and rownorm[m][c] = sum of squares of the fp32 values of columns
+ * [64c, 64c+64) of row m (|q|^2, |k|^2 per head for the attention kernel) for c < rownorm_chunks */
+int tssp_op_gemm_rownorm(const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K, const float* bias,
+                         float* rownorm, int ld_rownorm, int rownorm_chunks, void* stream);
 int tssp_op_score_finish(const float* partials, int ldp, float* norms, int ldn, int n_img, int T, int F,
                          float* scores, void* stream);
 int tssp_op_layernorm(const float* x, int64_t in_stride, const float* gamma, const float* beta, void* out_bf16,
@@ -159,6 +178,8 @@ int tssp_op_layernorm(const float* x, int64_t in_stride, const float* gamma, con
  * (up to 208 padded keys one kernel holds a whole key row, beyond that a second one streams keys in tiles of 128). */
 int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream);
 int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream);
+/* out[n * T, C*P*P] with T = (H/P)^2 + prefix_tokens: prefix_tokens (1 or 2) zero rows ahead of every image's patches */
+int tssp_op_im2col_ex(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens, void* stream);
 int tssp_op_cast_bf16(const float* in, int rows, int cols, int ld_in, void* out_bf16, int rows_pad, int cols_pad,
                       int ld_out, void* stream);
 int tssp_op_argmax_count(const float* logits, int ld, int n, int C, const int64_t* labels, int32_t* preds,

@@ -20,9 +20,10 @@ W_PATCH_W, W_PATCH_B, W_CLS, W_POS, W_FINAL_LN_W, W_FINAL_LN_B, W_HEAD0_W, W_HEA
 (BW_LN1_W, BW_LN1_B, BW_Q_W, BW_Q_B, BW_K_W, BW_K_B, BW_V_W, BW_V_B, BW_PROJ_W, BW_PROJ_B,
  BW_LN2_W, BW_LN2_B, BW_FC1_W, BW_FC1_B, BW_FC2_W, BW_FC2_B, BW_COUNT) = range(17)
 WX_DIST_TOKEN, WX_HEAD_DIST_W, WX_HEAD_DIST_B, WX_COUNT = range(4)  # engines with two prefix tokens (tssp_create_ex)
+TSSP_MAX_REGISTER_TOKENS = 7
 
 # GEMM epilogue modes (csrc/gemm_tcgen05.cuh: enum GemmMode)
-EPI_BF16, EPI_BF16_GELU, EPI_BF16_GELU_SCORE, EPI_BF16_GELU_SCORE_PRE, EPI_F32, EPI_BF16_ROWNORM = range(6)
+EPI_BF16, EPI_BF16_GELU, EPI_BF16_GELU_SCORE, EPI_BF16_GELU_SCORE_PRE, EPI_F32, EPI_BF16_ROWNORM, EPI_F32_SCALED = range(7)
 
 
 PROFILE_CLASSES = ["fc1_gelu_score", "qkv", "proj", "fc2", "patch_embed", "head", "attention", "layernorm", "score_finish", "misc"]
@@ -47,6 +48,15 @@ class TsspConfig(C.Structure):
     ]
 
 
+class TsspLayout(C.Structure):
+    _fields_ = [
+        ("dist_token", C.c_int32),
+        ("register_tokens", C.c_int32),
+        ("pos_covers_prefix", C.c_int32),
+        ("layer_scale", C.c_int32),
+    ]
+
+
 class TsspError(RuntimeError):
     """A call into libtssp_b200.so failed; the message comes from tssp_last_error()."""
 
@@ -61,6 +71,7 @@ SIGNATURES = {
     "tssp_last_error": (C.c_char_p, []),
     "tssp_create": (_I, [C.POINTER(TsspConfig), _I, C.POINTER(_P)]),
     "tssp_create_ex": (_I, [C.POINTER(TsspConfig), C.c_int32, _I, C.POINTER(_P)]),
+    "tssp_create_layout": (_I, [C.POINTER(TsspConfig), C.POINTER(TsspLayout), _I, C.POINTER(_P)]),
     "tssp_destroy": (_I, [_P]),
     "tssp_trim_pool": (_I, []),
     "tssp_load_weights": (_I, [_P, C.POINTER(_P), _I, _P]),
@@ -78,6 +89,7 @@ SIGNATURES = {
     "tssp_ffn_gather_batch": (_I, [_I, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(C.c_int32), _I, C.POINTER(_P),
                                    C.POINTER(C.c_int32), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), _P]),
     "tssp_op_gemm": (_I, [_I, _P, _I, _P, _I, _P, _I, _I, _I, _I, _P, _P, _I, _I, _I, _P]),
+    "tssp_op_gemm_scaled": (_I, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P, _P, _I, _P]),
     "tssp_op_gemm_rownorm": (_I, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P, _P, _I, _I, _P]),
     "tssp_op_score_finish": (_I, [_P, _I, _P, _I, _I, _I, _I, _P, _P]),
     "tssp_op_layernorm": (_I, [_P, _I64, _P, _P, _P, _I, _I, C.c_float, _P]),

@@ -5,7 +5,12 @@ Mirrors the reference's attribute walking (src/vit_pruning.py:28-75 `_get_encode
 (`.vit.encoder.layer[i].{attention,intermediate,output}`), HF `DeiTModel` / `DeiTForImageClassification` /
 `DeiTForImageClassificationWithTeacher` (`.deit`, the same layer layout; the reference reaches it through
 `model.base_model`) and timm-shaped `VisionTransformer` (`.blocks[i].{norm1,attn,norm2,mlp.fc1,mlp.fc2}`), distilled
-ones (`dist_token`, `head_dist`) included.
+ones (`dist_token`, `head_dist`) included, and those with LayerScale (`.blocks[i].ls1.gamma`, `.ls2.gamma`), register
+tokens (`reg_token`) and class-free position tables (`no_embed_class`): DeiT-III and DINOv2.
+
+The reference walks any timm `VisionTransformer`, so every timm-layout module the engine would not compute exactly is
+refused here by name (`_refuse_timm_extras`) instead of being run without it. HF `Dinov2*` classes fail the reference's
+walk (`layer[i].intermediate`) and fail here the same way.
 """
 from __future__ import annotations
 
@@ -102,8 +107,12 @@ class Anatomy:
     ffn_dims: List[int]
     attn_present: List[bool]
     score_point: int                      # 0 post-GELU (HF hook point), 1 pre-GELU (timm hook point)
-    prefix_tokens: int = 1                # tokens ahead of the patches: 1 (CLS) or 2 (CLS, distillation token: DeiT)
+    prefix_tokens: int = 1                # tokens ahead of the patches: 1 (CLS), 2 (CLS, distillation token: DeiT) or 1 + R
     dist_head: bool = False               # logits = (head(row 0) + dist_head(row 1)) / 2 (globals_ "head_dist_w/_b")
+    dist_token: bool = False              # row 1 is a distillation token (globals_ "dist")
+    register_tokens: int = 0              # R timm register tokens after CLS (globals_ "reg", [R, D])
+    pos_covers_prefix: bool = True        # False: timm no_embed_class, the position table has G^2 rows (patches only)
+    layer_scale: bool = False             # blocks carry "ls1" / "ls2" gammas [D] (timm LayerScale)
     globals_: Dict[str, Optional[torch.Tensor]] = field(default_factory=dict)
     blocks: List[Dict[str, Optional[torch.Tensor]]] = field(default_factory=list)
 
@@ -141,6 +150,47 @@ def _dist_head(main: Tuple, module) -> Tuple[Optional[torch.Tensor], Optional[to
     return _p(module.weight), _p(module.bias)
 
 
+def _is_identity(m) -> bool:
+    return m is None or isinstance(m, nn.Identity)
+
+
+def _refuse_timm_extras(root, blocks) -> None:
+    """AttributeError naming every timm VisionTransformer feature the engine does not compute: a model that has one is
+    refused rather than run without it."""
+    for name in ("norm_pre", "fc_norm"):
+        if not _is_identity(getattr(root, name, None)):
+            raise AttributeError(f"{name} ({type(getattr(root, name)).__name__}) is not supported: only Identity")
+    if not _is_identity(getattr(getattr(root, "patch_embed", None), "norm", None)):
+        raise AttributeError("patch_embed.norm is not supported: only Identity")
+    pool = getattr(root, "global_pool", "token")
+    if pool != "token":
+        raise AttributeError(f"global_pool={pool!r} is not supported: the classifier reads the CLS token ('token') only")
+    if getattr(root, "attn_pool", None) is not None:
+        raise AttributeError("attn_pool is not supported: the classifier reads the CLS token only")
+    if getattr(root, "cls_token", None) is None:
+        raise AttributeError("cls_token is missing: models without a class token are not supported")
+    if getattr(root, "dynamic_img_size", False):
+        raise AttributeError("dynamic_img_size=True is not supported: the engine runs one fixed image size")
+    if getattr(root, "dist_token", None) is not None and getattr(root, "reg_token", None) is not None:
+        raise AttributeError("dist_token together with reg_token is not supported")
+    for i, b in enumerate(blocks):
+        for owner, name in (("attn", "q_norm"), ("attn", "k_norm"), ("attn", "norm"), ("mlp", "norm")):
+            m = getattr(getattr(b, owner, None), name, None)
+            if not _is_identity(m):
+                raise AttributeError(f"blocks[{i}].{owner}.{name} ({type(m).__name__}) is not supported: only Identity")
+
+
+def _layer_scale(block, name: str, index: int) -> Optional[torch.Tensor]:
+    """gamma of timm's LayerScale `block.<name>` (x * gamma), or None when the module is Identity / absent."""
+    m = getattr(block, name, None)
+    if _is_identity(m):
+        return None
+    gamma = getattr(m, "gamma", None)
+    if not isinstance(gamma, torch.Tensor):
+        raise AttributeError(f"blocks[{index}].{name} ({type(m).__name__}) has no gamma: only timm LayerScale is supported")
+    return _p(gamma).reshape(-1)
+
+
 def _hf_root(vit_model):
     for name in ("vit", "deit"):
         if hasattr(vit_model, name):
@@ -155,6 +205,7 @@ def describe(vit_model) -> Anatomy:
     prefix = 1
     hdw = hdb = None
     dist = False
+    n_reg, pos_covers_prefix, layer_scale = 0, True, False
     if kind == "hf":
         vit = _hf_root(vit_model)
         emb = vit.embeddings
@@ -200,6 +251,7 @@ def describe(vit_model) -> Anatomy:
         score_point = 0
     else:
         root = vit_model
+        _refuse_timm_extras(root, blocks)
         conv = root.patch_embed.proj
         final_ln = root.norm
         head = _head(getattr(root, "head", None))
@@ -207,6 +259,11 @@ def describe(vit_model) -> Anatomy:
             prefix = 2
             hdw, hdb = _dist_head(head, getattr(root, "head_dist", None))
             dist = hdw is not None
+        reg = getattr(root, "reg_token", None)
+        if reg is not None:  # timm _pos_embed: [CLS, reg_token rows, patches]
+            n_reg = int(reg.shape[1])
+            prefix += n_reg
+        pos_covers_prefix = not bool(getattr(root, "no_embed_class", False))
         n_classes, head_hidden, h0, hw, hb = head
         first_attn = next((b.attn for b in blocks if has_attention(kind, b)), None)
         heads = int(first_attn.num_heads) if first_attn is not None else hidden // 64
@@ -214,9 +271,12 @@ def describe(vit_model) -> Anatomy:
             "patch_w": _p(conv.weight), "patch_b": _p(conv.bias), "cls": _p(root.cls_token), "pos": _p(root.pos_embed),
             "final_ln_w": _p(final_ln.weight), "final_ln_b": _p(final_ln.bias), "head0_w": h0, "head_w": hw, "head_b": hb,
             "dist": _p(getattr(root, "dist_token", None)), "head_dist_w": hdw, "head_dist_b": hdb,
+            "reg": None if reg is None else _p(reg).reshape(n_reg, hidden),
         }
+        gammas = [(_layer_scale(b, "ls1", i), _layer_scale(b, "ls2", i)) for i, b in enumerate(blocks)]
+        layer_scale = any(g is not None for pair in gammas for g in pair)
         blks = []
-        for b in blocks:
+        for b, (ls1, ls2) in zip(blocks, gammas):
             present = has_attention(kind, b)
             d = {
                 "ln2_w": _p(b.norm2.weight), "ln2_b": _p(b.norm2.bias),
@@ -233,20 +293,28 @@ def describe(vit_model) -> Anatomy:
                     "v_b": None if qkv_b is None else qkv_b[2 * D:3 * D],
                     "proj_w": _p(b.attn.proj.weight), "proj_b": _p(b.attn.proj.bias),
                 })
+            if layer_scale:  # a block without its own LayerScale scales by exactly 1
+                d["ls1"] = (ls1 if ls1 is not None else torch.ones(hidden)) if present else None
+                d["ls2"] = ls2 if ls2 is not None else torch.ones(hidden)
             blks.append(d)
         eps = float(final_ln.eps)
         score_point = 1
+    dist_tok = g.get("dist") is not None
     pw = g["patch_w"]
     channels, patch = int(pw.shape[1]), int(pw.shape[2])
     n_tokens = int(g["pos"].reshape(-1, hidden).shape[0])
-    grid = int(round(max(0, n_tokens - prefix) ** 0.5))
-    if grid * grid + prefix != n_tokens:
-        what = "CLS" if prefix == 1 else "CLS and distillation token"
+    covered = prefix if pos_covers_prefix else 0  # no_embed_class: the table holds the patches' rows only
+    grid = int(round(max(0, n_tokens - covered) ** 0.5))
+    if grid * grid + covered != n_tokens:
+        what = "CLS" if prefix == 1 else ("CLS and distillation token" if dist_tok else f"CLS and {n_reg} register tokens")
+        if not pos_covers_prefix:
+            what = f"nothing (no_embed_class; {what} get no position)"
         raise AttributeError(f"position table with {n_tokens} rows fits neither layout: not a square grid plus {what} "
                              f"({prefix} prefix token{'s' if prefix > 1 else ''})")
     return Anatomy(
         kind=kind, n_blocks=len(blocks), hidden=int(hidden), heads=heads, image_size=grid * patch, patch_size=patch,
         channels=channels, n_classes=int(n_classes), head_hidden=int(head_hidden), ln_eps=eps,
         ffn_dims=[int(p[0].weight.size(0)) for p in pairs], attn_present=[has_attention(kind, b) for b in blocks],
-        score_point=score_point, prefix_tokens=prefix, dist_head=dist, globals_=g, blocks=blks,
+        score_point=score_point, prefix_tokens=prefix, dist_head=dist, dist_token=dist_tok, register_tokens=n_reg,
+        pos_covers_prefix=pos_covers_prefix, layer_scale=layer_scale, globals_=g, blocks=blks,
     )

@@ -126,6 +126,7 @@ struct ProfScope {
 
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline int round_up(int a, int b) { return ceil_div(a, b) * b; }
+constexpr int TSSP_MAX_PREFIX = 1 + TSSP_MAX_REGISTER_TOKENS;  // CLS + register tokens (or CLS + distillation token)
 
 // ------------------------------------------------------------------------------------------------ TMA maps
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -325,10 +326,11 @@ static int launch_gemm_mode(const CUtensorMap& ta, const CUtensorMap& tb, const 
 // C[M,N] (ldc) = A[M,K] (lda) * W[N,K]^T (ldw) with epilogue `mode` (GemmMode)
 static int gemm(int mode, const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K,
                 const float* bias, float* partials, int ldp, int T, int reduce_add, cudaStream_t stream,
-                float* rownorm = nullptr, int ld_rownorm = 0, int rownorm_chunks = 0) {
+                float* rownorm = nullptr, int ld_rownorm = 0, int rownorm_chunks = 0, const float* col_scale = nullptr) {
     if (M <= 0 || N <= 0 || K <= 0) return fail("gemm: empty problem M=%d N=%d K=%d", M, N, K);
     if ((N & 7) || (K & 7)) return fail("gemm: N=%d and K=%d must be multiples of 8", N, K);
-    const bool f32_out = (mode == EPI_F32);
+    const bool f32_out = (mode == EPI_F32 || mode == EPI_F32_SCALED);
+    if (mode == EPI_F32_SCALED && col_scale == nullptr) return fail("gemm: scaled fp32 epilogue needs a column scale");
     const bool score = (mode == EPI_BF16_GELU_SCORE || mode == EPI_BF16_GELU_SCORE_PRE);
     if (score && (partials == nullptr || T < 32 || ldp < N)) return fail("gemm: score epilogue needs partials, ldp >= N and T >= 32 (T=%d)", T);
     const CUtensorMap *ta, *tb, *tc;
@@ -354,9 +356,19 @@ static int gemm(int mode, const void* A, int lda, const void* W, int ldw, void* 
     p.reverse = chain_dir();
     p.trace = g_gemm_trace;
     p.rownorm = rownorm; p.ld_rownorm = ld_rownorm; p.rownorm_chunks = rownorm_chunks;
+    p.col_scale = col_scale;
     if (mode == EPI_BF16_ROWNORM && rownorm == nullptr) return fail("gemm: row-norm epilogue needs an output buffer");
 #define TSSP_GEMM_CASE(m) \
     case m: return pair ? launch_gemm_mode<m, 2>(*ta, *tb, *tc, p, stream) : launch_gemm_mode<m, 1>(*ta, *tb, *tc, p, stream);
+#define TSSP_GEMM_F32_BN(m, bn_)                                                                                   \
+    if (bn == bn_)                                                                                                 \
+        return pair ? launch_gemm_mode<m, 2, bn_>(*ta, *tb, *tc, p, stream) : launch_gemm_mode<m, 1, bn_>(*ta, *tb, *tc, p, stream);
+    if (mode == EPI_F32_SCALED) {  // the fp32 tile widths of EPI_F32 (see above), with the LayerScale factor
+        TSSP_GEMM_F32_BN(EPI_F32_SCALED, GEMM_BN / 2)
+        TSSP_GEMM_F32_BN(EPI_F32_SCALED, 192)
+        TSSP_GEMM_F32_BN(EPI_F32_SCALED, GEMM_BN)
+    }
+#undef TSSP_GEMM_F32_BN
     if (bn == GEMM_BN / 2)  // EPI_F32 only (see above)
         return pair ? launch_gemm_mode<EPI_F32, 2, GEMM_BN / 2>(*ta, *tb, *tc, p, stream) : launch_gemm_mode<EPI_F32, 1, GEMM_BN / 2>(*ta, *tb, *tc, p, stream);
     if (bn == 192)
@@ -392,14 +404,23 @@ static int op_cast(const float* in, int rows, int cols, int ld_in, void* out, in
     return 0;
 }
 
-// prefix: zero rows ahead of every image's patches (1: CLS; 2: CLS and the DeiT distillation token)
+// prefix: zero rows ahead of every image's patches (1: CLS; 2: CLS and the DeiT distillation token; 1 + R: CLS and R
+// register tokens). Rows are patch_width(C, P) = round_up(C*P*P, 8) elements, zero padded past C*P*P.
+static int patch_width(int C, int P) { return round_up(C * P * P, 8); }
 static int op_im2col(const float* pixels, void* out, int n, int C, int H, int W, int P, cudaStream_t s, int prefix = 1) {
-    if (H % P || W % P || (P & 7) || H != W) return fail("im2col: H=%d W=%d P=%d unsupported (square images, P multiple of 8)", H, W, P);
-    if (prefix < 1 || prefix > 2) return fail("im2col: prefix=%d must be 1 or 2", prefix);
+    if (P < 1 || H % P || W % P || H != W) return fail("im2col: H=%d W=%d P=%d unsupported (square images, P dividing them)", H, W, P);
+    if (prefix < 1 || prefix > TSSP_MAX_PREFIX) return fail("im2col: prefix=%d must be in [1,%d]", prefix, TSSP_MAX_PREFIX);
     const int T = (H / P) * (W / P) + prefix;
-    const long long total = static_cast<long long>(n) * T * (C * P * P / 8);
-    im2col_patches_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T, prefix);
-    TSSP_LAUNCH_CHECK("im2col_patches_kernel");
+    const int ld = patch_width(C, P);
+    const long long total = static_cast<long long>(n) * T * (ld / 8);
+    if ((P & 7) == 0) {
+        im2col_patches_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T, prefix);
+        TSSP_LAUNCH_CHECK("im2col_patches_kernel");
+    } else {
+        im2col_patches_padded_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T,
+                                                                          prefix, ld);
+        TSSP_LAUNCH_CHECK("im2col_patches_padded_kernel");
+    }
     return 0;
 }
 
@@ -555,6 +576,7 @@ struct BlockWeights {
     const float *ln1_w, *ln1_b, *ln2_w, *ln2_b;  // fp32 (arena)
     __nv_bfloat16 *qkv_w, *proj_w, *fc1_w, *fc2_w;
     float *qkv_b, *proj_b, *fc1_b, *fc2_b;
+    float *ls1, *ls2; // LayerScale gammas of the attention / MLP branch [D] (layout.layer_scale), else nullptr
     int F, Fp;        // current width and its padding to a multiple of 8
     int F_cap;        // allocated (padded) width
     int score_off;    // column offset of this block in the concatenated score / norm vectors
@@ -580,7 +602,9 @@ struct tssp_engine {
     tssp_config_t cfg;
     int device;
     int T, M_cap, Kp, G;
-    int prefix;     // tokens ahead of the patches: 1 (CLS) or 2 (CLS, DeiT distillation token)
+    tssp_layout_t layout;
+    int prefix;     // tokens ahead of the patches: 1 (CLS) + layout.dist_token + layout.register_tokens
+    int head_rows;  // rows the classifier may read: 2 with a distillation token (CLS, distillation), else 1 (CLS)
     bool dist_head; // a distillation head is loaded: logits = (cls_head(row 0) + dist_head(row 1)) / 2
     int sumF;  // sum of current F over blocks (score vector length)
     int ldn;   // pitch of the per-image norm buffer = sum of F_cap
@@ -605,7 +629,7 @@ struct tssp_engine {
     int next_slot, staged_slot;
     int host_slot;         // slot of the host batch staged by the running entry point (-1: none); see finish_host_batch
     __nv_bfloat16 *patchA, *xn, *qkv, *ctx, *h, *head_hidden;
-    __nv_bfloat16* cls_norm;   // final LayerNorm of the prefix rows: [prefix][max_images][D] (CLS rows, then distillation rows)
+    __nv_bfloat16* cls_norm;   // final LayerNorm of the head rows: [head_rows][max_images][D] (CLS rows, then distillation rows)
     float *x, *partials, *norms, *scores, *logits;
     float* qk_norms;  // [M_cap][2*heads]: |q|^2 and |k|^2 per (token, head), written by the QKV GEMM epilogue
     size_t partials_stride;  // floats between two blocks' partial buffers
@@ -688,24 +712,31 @@ static int dev_alloc(tssp_engine* e, Tp** out, size_t count) {
     return 0;
 }
 
-static int validate(const tssp_config_t& c, int prefix) {
-    if (prefix < 1 || prefix > 2) return fail("config: prefix_tokens=%d must be 1 (CLS) or 2 (CLS and distillation token)", prefix);
+static int validate(const tssp_config_t& c, const tssp_layout_t& l) {
+    if (l.dist_token != 0 && l.dist_token != 1) return fail("layout: dist_token=%d must be 0 or 1", l.dist_token);
+    if (l.register_tokens < 0 || l.register_tokens > TSSP_MAX_REGISTER_TOKENS)
+        return fail("layout: register_tokens=%d must be in [0,%d]", l.register_tokens, TSSP_MAX_REGISTER_TOKENS);
+    if (l.dist_token && l.register_tokens > 0) return fail("layout: a distillation token and register tokens cannot be combined");
+    if (l.pos_covers_prefix != 0 && l.pos_covers_prefix != 1) return fail("layout: pos_covers_prefix=%d must be 0 or 1", l.pos_covers_prefix);
+    if (l.layer_scale != 0 && l.layer_scale != 1) return fail("layout: layer_scale=%d must be 0 or 1", l.layer_scale);
+    const int prefix = 1 + l.dist_token + l.register_tokens;
     if (c.n_blocks < 1 || c.n_blocks > TSSP_MAX_BLOCKS) return fail("config: n_blocks=%d out of range", c.n_blocks);
     if ((c.hidden % 128 && c.hidden != 192) || c.hidden > 1024 || c.hidden < 128)
         return fail("config: hidden=%d must be 192 or a multiple of 128 in [128,1024]", c.hidden);
     if (c.heads * 64 != c.hidden) return fail("config: head_dim must be 64 (hidden=%d heads=%d)", c.hidden, c.heads);
-    if (c.patch_size % 8 || c.image_size % c.patch_size) return fail("config: image %d / patch %d unsupported", c.image_size, c.patch_size);
+    if (c.patch_size < 1 || c.image_size % c.patch_size) return fail("config: image %d / patch %d unsupported", c.image_size, c.patch_size);
     const int G = c.image_size / c.patch_size, T = G * G + prefix;
     if (T < 32 || T > ATL_MAX_T) return fail("config: tokens per image T=%d must be in [32,%d]", T, ATL_MAX_T);
-    if ((c.channels * c.patch_size * c.patch_size) % 8) return fail("config: patch vector length not a multiple of 8");
+    if (c.channels < 1) return fail("config: channels=%d", c.channels);
     if (c.max_images < 1) return fail("config: max_images=%d", c.max_images);
     for (int b = 0; b < c.n_blocks; ++b)
         if (c.ffn_dims[b] < 1) return fail("config: ffn_dims[%d]=%d", b, c.ffn_dims[b]);
     return 0;
 }
 
-static int engine_create(const tssp_config_t* cfg, int prefix, int device, tssp_engine** out) {
-    TSSP_TRY(validate(*cfg, prefix));
+static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, int device, tssp_engine** out) {
+    TSSP_TRY(validate(*cfg, layout));
+    const int prefix = 1 + layout.dist_token + layout.register_tokens;
     int n_dev = 0;
     TSSP_CUDA(cudaGetDeviceCount(&n_dev));
     if (device < 0 || device >= n_dev) return fail("device %d out of range (%d visible)", device, n_dev);
@@ -720,11 +751,13 @@ static int engine_create(const tssp_config_t* cfg, int prefix, int device, tssp_
     e->weights_loaded = false;
     const int D = cfg->hidden, B = cfg->n_blocks;
     e->G = cfg->image_size / cfg->patch_size;
+    e->layout = layout;
     e->prefix = prefix;
+    e->head_rows = 1 + layout.dist_token;
     e->dist_head = false;
     e->T = e->G * e->G + prefix;
     e->M_cap = cfg->max_images * e->T;
-    e->Kp = cfg->channels * cfg->patch_size * cfg->patch_size;
+    e->Kp = patch_width(cfg->channels, cfg->patch_size);
     e->Cp = round_up(cfg->n_classes > 0 ? cfg->n_classes : 8, 8);
     e->Hhp = cfg->head_hidden > 0 ? round_up(cfg->head_hidden, 8) : 0;
     memcpy(e->attn_present, cfg->attn_present, sizeof(e->attn_present));
@@ -739,7 +772,7 @@ static int engine_create(const tssp_config_t* cfg, int prefix, int device, tssp_
     A(&e->head_b, e->Cp);
     e->head_dist_w = nullptr;
     e->head_dist_b = nullptr;
-    if (prefix == 2 && cfg->n_classes > 0) {
+    if (layout.dist_token && cfg->n_classes > 0) {
         A(&e->head_dist_w, static_cast<size_t>(e->Cp) * D);
         A(&e->head_dist_b, e->Cp);
     }
@@ -757,6 +790,8 @@ static int engine_create(const tssp_config_t* cfg, int prefix, int device, tssp_
         A(&w.proj_w, static_cast<size_t>(D) * D); A(&w.proj_b, D);
         A(&w.fc1_w, static_cast<size_t>(w.F_cap) * D); A(&w.fc1_b, w.F_cap);
         A(&w.fc2_w, static_cast<size_t>(D) * w.F_cap); A(&w.fc2_b, D);
+        w.ls1 = w.ls2 = nullptr;
+        if (layout.layer_scale) { A(&w.ls1, D); A(&w.ls2, D); }
     }
     e->ldn = off;
     e->sumF = 0;
@@ -779,7 +814,7 @@ static int engine_create(const tssp_config_t* cfg, int prefix, int device, tssp_
     A(&e->partials, e->partials_stride * B);
     A(&e->norms, static_cast<size_t>(cfg->max_images) * e->ldn);
     A(&e->scores, e->ldn);
-    A(&e->cls_norm, static_cast<size_t>(prefix) * cfg->max_images * D);
+    A(&e->cls_norm, static_cast<size_t>(e->head_rows) * cfg->max_images * D);
     A(&e->head_hidden, static_cast<size_t>(cfg->max_images) * (e->Hhp > 0 ? e->Hhp : 8));
     A(&e->logits, static_cast<size_t>(cfg->max_images) * e->Cp);
     A(&e->preds, cfg->max_images);
@@ -814,15 +849,23 @@ static int engine_create(const tssp_config_t* cfg, int prefix, int device, tssp_
     return 0;
 }
 
-// posmod[0] = cls + pos[0]; with two prefix tokens posmod[1] = dist + pos[1]; posmod[t >= prefix] = pos[t] + conv_bias
-// (so the patch GEMM needs no bias and the prefix rows, whose im2col rows are zero, receive exactly token + pos:
-// HF ViTEmbeddings.forward / DeiTEmbeddings.forward)
-__global__ void build_posmod_kernel(const float* __restrict__ pos, const float* __restrict__ cls, const float* __restrict__ dist,
-                                    const float* __restrict__ conv_b, float* __restrict__ out, int T, int D, int prefix) {
+// posmod[0] = cls + pos[0]; posmod[t < prefix] = tokens[t - 1] + pos[t] (the distillation token or the register tokens);
+// posmod[t >= prefix] = pos[t] + conv_bias (so the patch GEMM needs no bias and the prefix rows, whose im2col rows are
+// zero, receive exactly token + pos: HF ViTEmbeddings.forward / DeiTEmbeddings.forward, timm _pos_embed). With a
+// class-free position table (pos_covers_prefix = 0, timm no_embed_class) pos has G^2 rows: the prefix rows are the
+// bare tokens and patch row t takes pos[t - prefix].
+__global__ void build_posmod_kernel(const float* __restrict__ pos, const float* __restrict__ cls, const float* __restrict__ tokens,
+                                    const float* __restrict__ conv_b, float* __restrict__ out, int T, int D, int prefix,
+                                    int pos_covers_prefix) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= T * D) return;
     const int t = i / D, d = i % D;
-    out[i] = pos[i] + (t < prefix ? (t == 0 ? cls[d] : dist[d]) : (conv_b != nullptr ? conv_b[d] : 0.0f));
+    if (pos_covers_prefix) {
+        out[i] = pos[i] + (t < prefix ? (t == 0 ? cls[d] : tokens[(t - 1) * D + d]) : (conv_b != nullptr ? conv_b[d] : 0.0f));
+    } else {
+        out[i] = t < prefix ? (t == 0 ? cls[d] : tokens[(t - 1) * D + d])
+                            : pos[(t - prefix) * D + d] + (conv_b != nullptr ? conv_b[d] : 0.0f);
+    }
 }
 
 __global__ void copy_pad_f32_kernel(const float* __restrict__ in, int n, float* __restrict__ out, int n_pad, float scale) {
@@ -852,22 +895,35 @@ static int pack_ffn(tssp_engine* e, int b, int F, const float* fc1_w, const floa
 static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cudaStream_t s) {
     const tssp_config_t& c = e->cfg;
     const int D = c.hidden, B = c.n_blocks;
-    const int n_expected = TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT + (e->prefix == 2 ? TSSP_WX_COUNT : 0);
+    const tssp_layout_t& l = e->layout;
+    const int n_ext = l.dist_token ? TSSP_WX_COUNT : 0;
+    const int n_expected = TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT + n_ext + (l.register_tokens > 0 ? 1 : 0) + (l.layer_scale ? 2 * B : 0);
     if (n_entries != n_expected)
-        return fail("load_weights: expected %d pointers for %d prefix token(s), got %d", n_expected, e->prefix, n_entries);
+        return fail("load_weights: expected %d pointers for %d prefix token(s)%s, got %d", n_expected, e->prefix,
+                    l.layer_scale ? " and LayerScale" : "", n_entries);
     auto need = [&](int idx, const char* name) -> int { return t[idx] == nullptr ? fail("load_weights: %s is NULL", name) : 0; };
     TSSP_TRY(need(TSSP_W_PATCH_W, "patch_w")); TSSP_TRY(need(TSSP_W_CLS, "cls_token")); TSSP_TRY(need(TSSP_W_POS, "pos_embed"));
     TSSP_TRY(need(TSSP_W_FINAL_LN_W, "final_ln_w")); TSSP_TRY(need(TSSP_W_FINAL_LN_B, "final_ln_b"));
-    const float* const* x = t + TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT;  // extension entries (two prefix tokens only)
-    const bool dist_head = e->prefix == 2 && x[TSSP_WX_HEAD_DIST_W] != nullptr;
-    if (e->prefix == 2) {
+    const float* const* x = t + TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT;  // extension entries (distillation token only)
+    const float* const* lx = x + n_ext;                                  // layout entries (tssp_create_layout)
+    const float* reg_tokens = l.register_tokens > 0 ? lx[0] : nullptr;
+    const float* const* ls = lx + (l.register_tokens > 0 ? 1 : 0);       // per block LS1, LS2
+    if (l.register_tokens > 0 && reg_tokens == nullptr) return fail("load_weights: register tokens are NULL");
+    if (l.layer_scale)
+        for (int b = 0; b < B; ++b) {
+            if (ls[2 * b + 1] == nullptr) return fail("load_weights: block %d LS2 gamma is NULL", b);
+            if (c.attn_present[b] && ls[2 * b] == nullptr) return fail("load_weights: block %d LS1 gamma is NULL", b);
+        }
+    const bool dist_head = l.dist_token && x[TSSP_WX_HEAD_DIST_W] != nullptr;
+    if (l.dist_token) {
         if (x[TSSP_WX_DIST_TOKEN] == nullptr) return fail("load_weights: distillation token is NULL");
         if (dist_head && c.n_classes <= 0) return fail("load_weights: a distillation head needs n_classes > 0");
         if (dist_head && c.head_hidden > 0) return fail("load_weights: a distillation head cannot be combined with a Sequential head");
     }
-    TSSP_TRY(op_cast(t[TSSP_W_PATCH_W], D, e->Kp, e->Kp, e->patch_w, D, e->Kp, e->Kp, s));
-    build_posmod_kernel<<<ceil_div(e->T * D, 256), 256, 0, s>>>(t[TSSP_W_POS], t[TSSP_W_CLS], e->prefix == 2 ? x[TSSP_WX_DIST_TOKEN] : nullptr,
-                                                               t[TSSP_W_PATCH_B], e->posmod, e->T, D, e->prefix);
+    const int K = c.channels * c.patch_size * c.patch_size;  // Kp = K rounded up to 8: zero columns past K
+    TSSP_TRY(op_cast(t[TSSP_W_PATCH_W], D, K, K, e->patch_w, D, e->Kp, e->Kp, s));
+    build_posmod_kernel<<<ceil_div(e->T * D, 256), 256, 0, s>>>(t[TSSP_W_POS], t[TSSP_W_CLS], l.dist_token ? x[TSSP_WX_DIST_TOKEN] : reg_tokens,
+                                                               t[TSSP_W_PATCH_B], e->posmod, e->T, D, e->prefix, l.pos_covers_prefix);
     TSSP_LAUNCH_CHECK("build_posmod_kernel");
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_W], D, e->final_ln_w, D, s));
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_B], D, e->final_ln_b, D, s));
@@ -912,6 +968,10 @@ static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cud
         }
         TSSP_TRY(pack_ffn(e, b, bw.F, w[TSSP_BW_FC1_W], w[TSSP_BW_FC1_B], w[TSSP_BW_FC2_W], s));
         TSSP_TRY(copy_vec(w[TSSP_BW_FC2_B], D, bw.fc2_b, D, s));
+        if (l.layer_scale) {
+            TSSP_TRY(copy_vec(ls[2 * b], D, bw.ls1, D, s));  // NULL (no attention) -> zeros, never read
+            TSSP_TRY(copy_vec(ls[2 * b + 1], D, bw.ls2, D, s));
+        }
     }
     e->dist_head = dist_head;
     e->weights_loaded = true;
@@ -1106,6 +1166,12 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     const int rows = cls_only ? n : M;              // rows the row-wise part of the block works on
     const int pitch = cls_only ? e->T * D : D;      // their distance in x / ctx
     const bool attn = e->attn_present[b] && !skip_attn;
+    // proj / fc2 add their branch into the residual stream, scaled by the block's LayerScale gamma when the model has one
+    auto residual_gemm = [&](const void* A, int lda, const __nv_bfloat16* W, int ldw, float* xr, int rows_, int K, const float* bias,
+                             const float* gamma) {
+        return gemm(gamma != nullptr ? EPI_F32_SCALED : EPI_F32, A, lda, W, ldw, xr, pitch, rows_, D, K, bias, nullptr, 0, e->T, 1, s,
+                    nullptr, 0, 0, gamma);
+    };
     if (attn) {
         TSSP_PROF(KC_LN, s, op_layernorm(e->x, D, w.ln1_w, w.ln1_b, e->xn, M, D, c.ln_eps, s));
         TSSP_PROF(KC_QKV, s, gemm(EPI_BF16_ROWNORM, e->xn, D, w.qkv_w, D, e->qkv, 3 * D, M, 3 * D, D, w.qkv_b, nullptr, 0, e->T, 0, s,
@@ -1115,15 +1181,14 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     if (cls_only && e->dist_head) {
         for (int r = 0; r < 2; ++r) {
             float* xr = e->x + static_cast<size_t>(r) * D;
-            if (attn) TSSP_PROF(KC_PROJ, s, gemm(EPI_F32, e->ctx + static_cast<size_t>(r) * D, pitch, w.proj_w, D, xr, pitch, n, D, D, w.proj_b,
-                                                 nullptr, 0, e->T, 1, s));
+            if (attn) TSSP_PROF(KC_PROJ, s, residual_gemm(e->ctx + static_cast<size_t>(r) * D, pitch, w.proj_w, D, xr, n, D, w.proj_b, w.ls1));
             TSSP_PROF(KC_LN, s, op_layernorm(xr, pitch, w.ln2_w, w.ln2_b, e->xn, n, D, c.ln_eps, s));
             TSSP_PROF(KC_FC1, s, gemm(EPI_BF16_GELU, e->xn, D, w.fc1_w, D, e->h, w.Fp, n, w.Fp, D, w.fc1_b, nullptr, 0, e->T, 0, s));
-            TSSP_PROF(KC_FC2, s, gemm(EPI_F32, e->h, w.Fp, w.fc2_w, w.Fp, xr, pitch, n, D, w.Fp, w.fc2_b, nullptr, 0, e->T, 1, s));
+            TSSP_PROF(KC_FC2, s, residual_gemm(e->h, w.Fp, w.fc2_w, w.Fp, xr, n, w.Fp, w.fc2_b, w.ls2));
         }
         return 0;
     }
-    if (attn) TSSP_PROF(KC_PROJ, s, gemm(EPI_F32, e->ctx, pitch, w.proj_w, D, e->x, pitch, rows, D, D, w.proj_b, nullptr, 0, e->T, 1, s));
+    if (attn) TSSP_PROF(KC_PROJ, s, residual_gemm(e->ctx, pitch, w.proj_w, D, e->x, rows, D, w.proj_b, w.ls1));
     TSSP_PROF(KC_LN, s, op_layernorm(e->x, pitch, w.ln2_w, w.ln2_b, e->xn, rows, D, c.ln_eps, s, /*stream_in=*/!cls_only));
     if (fc1_mode == FC1_SCORE) {
         const int mode = c.score_point == 1 ? EPI_BF16_GELU_SCORE_PRE : EPI_BF16_GELU_SCORE;
@@ -1134,7 +1199,7 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     } else {
         TSSP_PROF(KC_FC1, s, gemm(EPI_BF16_GELU, e->xn, D, w.fc1_w, D, e->h, w.Fp, rows, w.Fp, D, w.fc1_b, nullptr, 0, e->T, 0, s));
     }
-    if (run_fc2) TSSP_PROF(KC_FC2, s, gemm(EPI_F32, e->h, w.Fp, w.fc2_w, w.Fp, e->x, pitch, rows, D, w.Fp, w.fc2_b, nullptr, 0, e->T, 1, s));
+    if (run_fc2) TSSP_PROF(KC_FC2, s, residual_gemm(e->h, w.Fp, w.fc2_w, w.Fp, e->x, rows, w.Fp, w.fc2_b, w.ls2));
     return 0;
 }
 
@@ -1276,10 +1341,19 @@ int tssp_profile_end(double* ms_per_class, unsigned long long* launches_per_clas
     return 0;
 }
 
-int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out) {
+int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, int device, tssp_handle_t* out) {
     TSSP_ENTRY();
-    if (cfg == nullptr || out == nullptr) return fail("tssp_create: NULL argument");
-    return engine_create(cfg, prefix_tokens, device, out);
+    if (cfg == nullptr || layout == nullptr || out == nullptr) return fail("tssp_create: NULL argument");
+    return engine_create(cfg, *layout, device, out);
+}
+
+int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out) {
+    if (prefix_tokens < 1 || prefix_tokens > 2) {
+        TSSP_ENTRY();
+        return fail("config: prefix_tokens=%d must be 1 (CLS) or 2 (CLS and distillation token)", prefix_tokens);
+    }
+    const tssp_layout_t layout = {prefix_tokens == 2 ? 1 : 0, 0, 1, 0};
+    return tssp_create_layout(cfg, &layout, device, out);
 }
 
 int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out) { return tssp_create_ex(cfg, 1, device, out); }
@@ -1607,6 +1681,13 @@ int tssp_op_gemm(int mode, const void* A, int lda, const void* W, int ldw, void*
     TSSP_ENTRY();
     if (A == nullptr || W == nullptr || C == nullptr) return fail("tssp_op_gemm: NULL argument");
     return gemm(mode, A, lda, W, ldw, C, ldc, M, N, K, bias, partials, ldp, tokens_per_image, reduce_add, static_cast<cudaStream_t>(stream));
+}
+int tssp_op_gemm_scaled(const void* A, int lda, const void* W, int ldw, float* C, int ldc, int M, int N, int K, const float* bias,
+                        const float* col_scale, int reduce_add, void* stream) {
+    TSSP_ENTRY();
+    if (A == nullptr || W == nullptr || C == nullptr || col_scale == nullptr) return fail("tssp_op_gemm_scaled: NULL argument");
+    return gemm(EPI_F32_SCALED, A, lda, W, ldw, C, ldc, M, N, K, bias, nullptr, 0, 0, reduce_add, static_cast<cudaStream_t>(stream),
+                nullptr, 0, 0, col_scale);
 }
 int tssp_op_gemm_rownorm(const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K, const float* bias,
                          float* rownorm, int ld_rownorm, int rownorm_chunks, void* stream) {

@@ -21,6 +21,8 @@
 //                           src/vit_pruning.py:135)
 //       EPI_F32             out fp32 (=|+=) acc + bias; "+=" is a TMA reduce-add into the fp32 residual
 //                           stream, so the residual is never loaded by the SMs   (proj, fc2, patch-embed, head)
+//       EPI_F32_SCALED      out fp32 (=|+=) col_scale[c] * (acc + bias[c])   (proj / fc2 of LayerScale blocks: timm
+//                           LayerScale.forward multiplies the branch output by gamma before the residual add)
 //     Output tiles leave through a 4 KB per-warp staging slot and TMA stores (clipped at the tensor edge).
 #pragma once
 #include <type_traits>
@@ -36,6 +38,7 @@ enum GemmMode : int {
     EPI_BF16_GELU_SCORE_PRE = 3,
     EPI_F32 = 4,
     EPI_BF16_ROWNORM = 5,  // EPI_BF16 + per-(row, 64-column chunk) sum of squares (|q|^2, |k|^2 per head for attention)
+    EPI_F32_SCALED = 6,    // EPI_F32 with a per-column scale applied after the bias (LayerScale)
 };
 
 struct GemmParams {
@@ -53,6 +56,8 @@ struct GemmParams {
     int reverse;            // 1 => walk the tile sequence from the last tile to the first (same tiles, same results):
                             //      a consumer that starts where its producer stopped finds those rows still in L2
     long long* trace;       // diagnostics (tssp_debug_gemm_trace): clock64() stamps of CTA 0, or nullptr
+    const float* col_scale; // EPI_F32_SCALED: [N] per-column factor (kept last: the other instances read the fields above
+                            //      at the same parameter offsets as before it existed)
 };
 
 // Trace layout: 16 int64 per tile, first GEMM_TRACE_TILES tiles of CTA 0. Slots 0-1: MMA thread (accumulator buffer
@@ -83,7 +88,7 @@ struct GemmCfg {
     static constexpr int SMEM_BYTES = 1024 + STAGES * STAGE_BYTES + EPI_WARPS * SLOT_BYTES + BAR_BYTES;
     static constexpr int THREADS = 128 + 32 * EPI_WARPS;
     static constexpr int TMEM_COLS = 2 * BN <= 64 ? 64 : (2 * BN <= 128 ? 128 : (2 * BN <= 256 ? 256 : 512));  // allocations are powers of two
-    static constexpr bool OUT_BF16 = (MODE != EPI_F32);
+    static constexpr bool OUT_BF16 = (MODE != EPI_F32 && MODE != EPI_F32_SCALED);
     static constexpr int CHUNK_COLS = OUT_BF16 ? 64 : 32;  // columns per 128-byte staging row
     static constexpr int CHUNKS = BN / CHUNK_COLS;
     static constexpr int COL_GROUPS = EPI_WARPS / 4;        // column halves handled by different warps
@@ -325,7 +330,22 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
                     tmem_ld_fence(r);
                     if (cc + 1 < Cfg::CHUNKS_PER_WARP) tmem_ld_32x32b_x32_nowait(t_row + tile_col + 32, nx);
                     if (gcol0 < p.N && row0 < p.M) {  // warp-uniform
-                        if (p.bias != nullptr) {
+                        if constexpr (MODE == EPI_F32_SCALED) {
+                            // gamma * (acc + bias) in fp32, then the residual add: timm's order of operations
+#pragma unroll
+                            for (int j = 0; j < 32; j += 4) {
+                                const int gc = gcol0 + j;
+                                if (gc < p.N) {
+                                    const float4 b4 = p.bias != nullptr ? __ldg(reinterpret_cast<const float4*>(p.bias + gc))
+                                                                        : make_float4(0.f, 0.f, 0.f, 0.f);
+                                    const float4 g4 = __ldg(reinterpret_cast<const float4*>(p.col_scale + gc));
+                                    r[j + 0] = __float_as_uint(__fmul_rn(g4.x, __fadd_rn(__uint_as_float(r[j + 0]), b4.x)));
+                                    r[j + 1] = __float_as_uint(__fmul_rn(g4.y, __fadd_rn(__uint_as_float(r[j + 1]), b4.y)));
+                                    r[j + 2] = __float_as_uint(__fmul_rn(g4.z, __fadd_rn(__uint_as_float(r[j + 2]), b4.z)));
+                                    r[j + 3] = __float_as_uint(__fmul_rn(g4.w, __fadd_rn(__uint_as_float(r[j + 3]), b4.w)));
+                                }
+                            }
+                        } else if (p.bias != nullptr) {
 #pragma unroll
                             for (int j = 0; j < 32; j += 4) {
                                 const int gc = gcol0 + j;

@@ -28,7 +28,8 @@ __global__ void cast_pad_bf16_kernel(const float* __restrict__ in, int rows, int
 // ------------------------------------------------------------------------------------------------
 // Patch extraction for the patch-embedding GEMM (HF ViTPatchEmbeddings: Conv2d(C, D, P, stride P) ==
 // GEMM over non-overlapping patches). pixels fp32 [n, C, H, W] -> A bf16 [n*T, C*P*P] where rows
-// img*T + r, r < prefix, are the (all-zero) slots of the prefix tokens (CLS; CLS and distillation for DeiT) and row
+// img*T + r, r < prefix, are the (all-zero) slots of the prefix tokens (CLS, then a DeiT distillation token or timm
+// register tokens) and row
 // img*T + prefix + (py*G + px) holds patch (py, px) flattened as (c, ky, kx) -- the order of
 // Conv2d.weight.view(D, -1). Each thread converts 8 consecutive kx.
 // ------------------------------------------------------------------------------------------------
@@ -65,6 +66,54 @@ __global__ void im2col_patches_kernel(const float* __restrict__ pixels, __nv_bfl
             packed.w = *reinterpret_cast<uint32_t*>(&p3);
         }
         *reinterpret_cast<uint4*>(out + static_cast<size_t>(row) * Kp + k8 * 8) = packed;
+    }
+}
+
+// The same for patches whose width is not a multiple of 8 (P = 14: DINOv2): rows of `ld` = round_up(C*P*P, 8) elements,
+// the columns past C*P*P written as zeros (the patch weight is padded the same way, so they add nothing to the GEMM).
+// A patch row of 14 floats starts only 8-byte aligned, so each thread converts its 8 columns as four pairs: with P even a
+// pair never straddles two patch rows and is one 64-bit load; with P odd the pair is two scalar loads.
+__global__ void im2col_patches_padded_kernel(const float* __restrict__ pixels, __nv_bfloat16* __restrict__ out, int n_img,
+                                             int C, int H, int W, int P, int T, int prefix, int ld) {
+    const int G = W / P;
+    const int PP = P * P;
+    const int K = C * PP;
+    const int k8_per_row = ld / 8;
+    const long long total = static_cast<long long>(n_img) * T * k8_per_row;
+    for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+         i += static_cast<long long>(gridDim.x) * blockDim.x) {
+        const int k8 = static_cast<int>(i % k8_per_row);
+        const long long row = i / k8_per_row;
+        const int t = static_cast<int>(row % T);
+        const int img = static_cast<int>(row / T);
+        uint32_t w[4] = {0u, 0u, 0u, 0u};
+        if (t >= prefix) {
+            const int patch = t - prefix;
+            const int py = patch / G, px = patch % G;
+            const float* base = pixels + static_cast<size_t>(img) * C * H * W + static_cast<size_t>(py * P) * W + px * P;
+            auto at = [&](int k) {
+                const int c = k / PP, r = k - c * PP, ky = r / P, kx = r - ky * P;
+                return base + (static_cast<size_t>(c) * H + ky) * W + kx;
+            };
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int k = k8 * 8 + 2 * q;
+                float v0 = 0.0f, v1 = 0.0f;
+                if ((P & 1) == 0) {
+                    if (k < K) {  // K even: k + 1 < K as well
+                        const float2 f = __ldg(reinterpret_cast<const float2*>(at(k)));
+                        v0 = f.x;
+                        v1 = f.y;
+                    }
+                } else {
+                    if (k < K) v0 = __ldg(at(k));
+                    if (k + 1 < K) v1 = __ldg(at(k + 1));
+                }
+                __nv_bfloat162 p2 = __floats2bfloat162_rn(v0, v1);
+                w[q] = *reinterpret_cast<uint32_t*>(&p2);
+            }
+        }
+        *reinterpret_cast<uint4*>(out + static_cast<size_t>(row) * ld + k8 * 8) = make_uint4(w[0], w[1], w[2], w[3]);
     }
 }
 

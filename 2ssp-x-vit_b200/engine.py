@@ -14,7 +14,7 @@ from . import _lib as L
 from .anatomy import Anatomy, describe
 
 _GLOBAL_ORDER = ["patch_w", "patch_b", "cls", "pos", "final_ln_w", "final_ln_b", "head0_w", "head_w", "head_b"]
-_EXT_ORDER = ["dist", "head_dist_w", "head_dist_b"]  # engines with two prefix tokens (include/tssp.h: tssp_weight_ext_index)
+_EXT_ORDER = ["dist", "head_dist_w", "head_dist_b"]  # engines with a distillation token (include/tssp.h: tssp_weight_ext_index)
 _BLOCK_ORDER = ["ln1_w", "ln1_b", "q_w", "q_b", "k_w", "k_b", "v_w", "v_b", "proj_w", "proj_b",
                 "ln2_w", "ln2_b", "fc1_w", "fc1_b", "fc2_w", "fc2_b"]
 
@@ -49,7 +49,8 @@ class Engine:
             cfg.attn_present[i] = 1 if a.attn_present[i] else 0
         self._handle = C.c_void_p()
         with torch.cuda.device(self.device):
-            L.check(self.lib.tssp_create_ex(C.byref(cfg), a.prefix_tokens, self.device.index, C.byref(self._handle)))
+            layout = L.TsspLayout(int(a.dist_token), a.register_tokens, int(a.pos_covers_prefix), int(a.layer_scale))
+            L.check(self.lib.tssp_create_layout(C.byref(cfg), C.byref(layout), self.device.index, C.byref(self._handle)))
         self.ffn_dims = list(a.ffn_dims)
         self.load_weights(a)
         self.anatomy.globals_.clear()
@@ -68,8 +69,13 @@ class Engine:
         entries = [self._dev32(a.globals_.get(k), keep) for k in _GLOBAL_ORDER]
         for blk in a.blocks:
             entries += [self._dev32(blk.get(k), keep) for k in _BLOCK_ORDER]
-        if a.prefix_tokens == 2:
+        if a.dist_token:
             entries += [self._dev32(a.globals_.get(k), keep) for k in _EXT_ORDER]
+        if a.register_tokens > 0:  # then the layout entries of tssp_create_layout
+            entries.append(self._dev32(a.globals_["reg"], keep))
+        if a.layer_scale:
+            for blk in a.blocks:
+                entries += [self._dev32(blk.get("ls1"), keep), self._dev32(blk.get("ls2"), keep)]
         table = (C.c_void_p * len(entries))(*entries)
         with torch.cuda.device(self.device):
             L.check(self.lib.tssp_load_weights(self._handle, table, len(entries), L.current_stream()))

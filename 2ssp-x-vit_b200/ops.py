@@ -60,6 +60,20 @@ def gemm(mode: int, a: torch.Tensor, w: torch.Tensor, out: torch.Tensor, bias: t
     return out
 
 
+def gemm_scaled(a: torch.Tensor, w: torch.Tensor, out: torch.Tensor, bias: torch.Tensor | None, col_scale: torch.Tensor, *,
+                reduce_add: bool = False) -> torch.Tensor:
+    """The LayerScale epilogue: out (fp32) (=|+=) col_scale * (a @ w^T + bias), column-wise."""
+    _need_cuda(a, w, out, bias, col_scale)
+    if out.dtype != torch.float32 or col_scale.dtype != torch.float32:
+        raise ValueError("gemm_scaled: out and col_scale must be float32")
+    M, K = a.shape
+    N = w.shape[0]
+    lib = L.load()
+    L.check(lib.tssp_op_gemm_scaled(L.ptr(a), a.stride(0), L.ptr(w), w.stride(0), L.ptr(out), out.stride(0), M, N, K, L.ptr(bias),
+                                    L.ptr(col_scale), 1 if reduce_add else 0, L.current_stream()))
+    return out
+
+
 def gemm_rownorm(a: torch.Tensor, w: torch.Tensor, out: torch.Tensor, bias: torch.Tensor | None, chunks: int) -> torch.Tensor:
     """The QKV epilogue: out (bf16) = a @ w^T + bias; returns [M, chunks] fp32 sums of squares of 64-column chunks."""
     _need_cuda(a, w, out, bias)
@@ -106,13 +120,14 @@ def attention(qkv: torch.Tensor, n_img: int, T: int, heads: int) -> torch.Tensor
 
 
 def im2col(pixels: torch.Tensor, patch: int, prefix: int = 1) -> torch.Tensor:
-    """[n * T, C*P*P] bf16 patch rows, `prefix` zero rows ahead of every image's patches (2 for DeiT)."""
+    """[n * T, Kp] bf16 patch rows, `prefix` zero rows ahead of every image's patches (2 for DeiT, 1 + R with R register
+    tokens); Kp = C*P*P rounded up to a multiple of 8, the columns past C*P*P zero (P = 14: 588 -> 592)."""
     _need_cuda(pixels)
     if pixels.dtype != torch.float32 or not pixels.is_contiguous():
         raise ValueError("im2col: pixels must be a contiguous float32 tensor [n, C, H, W]")
     n, c, h, w = pixels.shape
     T = (h // patch) * (w // patch) + prefix
-    out = torch.empty(n * T, c * patch * patch, device=pixels.device, dtype=torch.bfloat16)
+    out = torch.empty(n * T, (c * patch * patch + 7) // 8 * 8, device=pixels.device, dtype=torch.bfloat16)
     lib = L.load()
     L.check(lib.tssp_op_im2col_ex(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, L.current_stream()))
     return out

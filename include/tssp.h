@@ -37,15 +37,17 @@ typedef struct tssp_engine* tssp_handle_t;
 
 /* Model anatomy, as discovered by the reference's _get_encoder/_gather_mlp_pairs walkers
  * (src/vit_pruning.py:28-75) on an HF ViTForImageClassification or a timm VisionTransformer.
- * Tokens per image T = (image_size / patch_size)^2 + prefix tokens (1 for ViT, 2 for DeiT: see tssp_create_ex) must lie
- * in [32, 1025]: ViT-x/16 up to 512x512 (T = 1025), ViT-x/8 up to 256x256; tssp_create rejects other shapes before it
+ * Tokens per image T = (image_size / patch_size)^2 + prefix tokens (1 for ViT, 2 for DeiT: see tssp_create_ex; 1 + R with
+ * R register tokens: see tssp_create_layout) must lie in [32, 1025]: ViT-x/16 up to 512x512 (T = 1025), ViT-x/8 up to
+ * 256x256, ViT-x/14 up to 448x448; tssp_create rejects other shapes (DINOv2 at its native 518x518: T = 1370) before it
  * touches a device. */
 typedef struct tssp_config {
     int32_t n_blocks;                      /* B: encoder blocks */
     int32_t hidden;                        /* D: 192 (DeiT-Ti, ViT-Ti) or a multiple of 128, <= 1024 */
     int32_t heads;                         /* D / heads must be 64 */
     int32_t image_size;                    /* H = W, multiple of patch_size */
-    int32_t patch_size;                    /* P: multiple of 8 */
+    int32_t patch_size;                    /* P: any size dividing image_size; the patch vector C_in*P*P is zero padded
+                                              to a multiple of 8 inside the engine (P = 14: 588 -> 592) */
     int32_t channels;                      /* C_in (3) */
     int32_t n_classes;                     /* classifier outputs (0: no head, logits/eval unavailable) */
     int32_t head_hidden;                   /* 0: Linear head; >0: Sequential(Linear(D,h,bias=False), GELU, Linear(h,C))
@@ -91,6 +93,24 @@ enum tssp_weight_ext_index {
     TSSP_WX_COUNT
 };
 
+/* Prefix-token and residual-branch layout of timm VisionTransformer models beyond ViT / DeiT (timm
+ * vision_transformer.py: VisionTransformer._pos_embed, LayerScale, Block.forward). */
+#define TSSP_MAX_REGISTER_TOKENS 7
+typedef struct tssp_layout {
+    int32_t dist_token;        /* 1: DeiT distillation token after CLS (what tssp_create_ex(..., 2, ...) means) */
+    int32_t register_tokens;   /* R timm register tokens after CLS (reg_token [1, R, D]), 0..7; not with dist_token */
+    int32_t pos_covers_prefix; /* 1: pos table [T, D] covers the prefix rows (ViT, DeiT, DINOv2);
+                                  0: pos table [G^2, D] for the patches only, the prefix rows get no position
+                                  (timm no_embed_class: DeiT-III, DINOv2 with registers) */
+    int32_t layer_scale;       /* 1: every block scales its attention and MLP outputs by ls1.gamma / ls2.gamma before the
+                                  residual add: x += gamma * (proj(a) + b), in fp32 */
+} tssp_layout_t;
+/* Entries appended to the weight table of an engine made by tssp_create_layout, after the TSSP_WX_* ones (present only
+ * with dist_token), in this order:
+ *   register_tokens > 0: one entry, the register tokens [R, D] (row-major, reg_token[0]);
+ *   layer_scale = 1:     2 * n_blocks entries, per block LS1 [D] (attention branch; NULL for a block without attention)
+ *                        then LS2 [D] (MLP branch). */
+
 int tssp_abi_version(void);
 const char* tssp_last_error(void);
 
@@ -102,6 +122,9 @@ int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out);
  * DeiTForImageClassificationWithTeacher.forward and of timm's distilled models; a Sequential head (head_hidden > 0) cannot
  * be combined with one. Without it (DeiTForImageClassification.forward) the head reads the CLS row only. */
 int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out);
+/* The general form: tssp_create is this with the layout {0, 0, 1, 0}, tssp_create_ex with {prefix_tokens == 2, 0, 1, 0}.
+ * T = G^2 + 1 + dist_token + register_tokens. Models with register tokens feed the classifier from the CLS row. */
+int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, int device, tssp_handle_t* out);
 int tssp_destroy(tssp_handle_t h);
 /* tssp_destroy parks the engine's device buffers in a per-process pool (exact-size reuse by the next tssp_create; capped
  * by TSSP_POOL_MB, default 16384, 0 = no pool); this returns all parked buffers to the driver. */
@@ -163,11 +186,15 @@ int tssp_ffn_gather_batch(int n_blocks, const float* const* fc1_w, const float* 
 
 /* ---- kernel-level entry points (used by the parity tests and by the engine itself) ---- */
 /* C[M,N] = A[M,K] * W[N,K]^T with a fused epilogue; mode: 0 bf16(acc+bias), 1 bf16 gelu, 2 bf16 gelu + score
- * partials, 3 same with pre-activation scores, 4 fp32 (reduce_add: C += ...). A, W bf16; lda/ldw/ldc in elements. */
+ * partials, 3 same with pre-activation scores, 4 fp32 (reduce_add: C += ...). A, W bf16; lda/ldw/ldc in elements.
+ * K is a multiple of 8; past K the operands' tiles are zero filled, so any such K works (the padded patch vector). */
 int tssp_op_gemm(int mode, const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K,
                  const float* bias, float* partials, int ldp, int tokens_per_image, int reduce_add, void* stream);
 /* the QKV form (mode 5): bf16 C = A W^T + bias, and rownorm[m][c] = sum of squares of the fp32 values of columns
  * [64c, 64c+64) of row m (|q|^2, |k|^2 per head for the attention kernel) for c < rownorm_chunks */
+/* the LayerScale form (mode 6): fp32 C (=|+=) col_scale[c] * (A W^T + bias)[., c] */
+int tssp_op_gemm_scaled(const void* A, int lda, const void* W, int ldw, float* C, int ldc, int M, int N, int K, const float* bias,
+                        const float* col_scale, int reduce_add, void* stream);
 int tssp_op_gemm_rownorm(const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K, const float* bias,
                          float* rownorm, int ld_rownorm, int rownorm_chunks, void* stream);
 int tssp_op_score_finish(const float* partials, int ldp, float* norms, int ldn, int n_img, int T, int F,
@@ -178,7 +205,8 @@ int tssp_op_layernorm(const float* x, int64_t in_stride, const float* gamma, con
  * (up to 208 padded keys one kernel holds a whole key row, beyond that a second one streams keys in tiles of 128). */
 int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream);
 int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream);
-/* out[n * T, C*P*P] with T = (H/P)^2 + prefix_tokens: prefix_tokens (1 or 2) zero rows ahead of every image's patches */
+/* out[n * T, Kp] with T = (H/P)^2 + prefix_tokens and Kp = round_up(C*P*P, 8): prefix_tokens (1..8) zero rows ahead of
+ * every image's patches, columns past C*P*P zero (the padded patch vector of patch sizes that are not a multiple of 8) */
 int tssp_op_im2col_ex(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens, void* stream);
 int tssp_op_cast_bf16(const float* in, int rows, int cols, int ld_in, void* out_bf16, int rows_pad, int cols_pad,
                       int ld_out, void* stream);

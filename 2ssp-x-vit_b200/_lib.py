@@ -23,7 +23,10 @@ WX_DIST_TOKEN, WX_HEAD_DIST_W, WX_HEAD_DIST_B, WX_COUNT = range(4)  # engines wi
 TSSP_MAX_REGISTER_TOKENS = 7
 
 # GEMM epilogue modes (csrc/gemm_tcgen05.cuh: enum GemmMode)
-EPI_BF16, EPI_BF16_GELU, EPI_BF16_GELU_SCORE, EPI_BF16_GELU_SCORE_PRE, EPI_F32, EPI_BF16_ROWNORM, EPI_F32_SCALED = range(7)
+(EPI_BF16, EPI_BF16_GELU, EPI_BF16_GELU_SCORE, EPI_BF16_GELU_SCORE_PRE, EPI_F32, EPI_BF16_ROWNORM, EPI_F32_SCALED,
+ EPI_BF16_QGELU, EPI_BF16_QGELU_SCORE_PRE) = range(9)
+# MLP activations of tssp_model_opts_t.ffn_act
+FFN_ACTS = {"gelu": 0, "quick_gelu": 1}
 
 
 PROFILE_CLASSES = ["fc1_gelu_score", "qkv", "proj", "fc2", "patch_embed", "head", "attention", "layernorm", "score_finish", "misc"]
@@ -57,6 +60,13 @@ class TsspLayout(C.Structure):
     ]
 
 
+class TsspModelOpts(C.Structure):
+    _fields_ = [
+        ("pre_norm", C.c_int32),
+        ("ffn_act", C.c_int32),
+    ]
+
+
 class TsspError(RuntimeError):
     """A call into libtssp_b200.so failed; the message comes from tssp_last_error()."""
 
@@ -72,6 +82,7 @@ SIGNATURES = {
     "tssp_create": (_I, [C.POINTER(TsspConfig), _I, C.POINTER(_P)]),
     "tssp_create_ex": (_I, [C.POINTER(TsspConfig), C.c_int32, _I, C.POINTER(_P)]),
     "tssp_create_layout": (_I, [C.POINTER(TsspConfig), C.POINTER(TsspLayout), _I, C.POINTER(_P)]),
+    "tssp_create_model": (_I, [C.POINTER(TsspConfig), C.POINTER(TsspLayout), C.POINTER(TsspModelOpts), _I, C.POINTER(_P)]),
     "tssp_destroy": (_I, [_P]),
     "tssp_trim_pool": (_I, []),
     "tssp_load_weights": (_I, [_P, C.POINTER(_P), _I, _P]),
@@ -93,6 +104,7 @@ SIGNATURES = {
     "tssp_op_gemm_rownorm": (_I, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P, _P, _I, _I, _P]),
     "tssp_op_score_finish": (_I, [_P, _I, _P, _I, _I, _I, _I, _P, _P]),
     "tssp_op_layernorm": (_I, [_P, _I64, _P, _P, _P, _I, _I, C.c_float, _P]),
+    "tssp_op_layernorm_f32": (_I, [_P, _I64, _P, _P, _P, _I64, _I, _I, C.c_float, _P]),
     "tssp_op_attention": (_I, [_P, _P, _I, _I, _I, _I, _P]),
     "tssp_op_im2col": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
     "tssp_op_im2col_ex": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),

@@ -6,11 +6,12 @@ Mirrors the reference's attribute walking (src/vit_pruning.py:28-75 `_get_encode
 `DeiTForImageClassificationWithTeacher` (`.deit`, the same layer layout; the reference reaches it through
 `model.base_model`) and timm-shaped `VisionTransformer` (`.blocks[i].{norm1,attn,norm2,mlp.fc1,mlp.fc2}`), distilled
 ones (`dist_token`, `head_dist`) included, and those with LayerScale (`.blocks[i].ls1.gamma`, `.ls2.gamma`), register
-tokens (`reg_token`) and class-free position tables (`no_embed_class`): DeiT-III and DINOv2.
+tokens (`reg_token`) and class-free position tables (`no_embed_class`): DeiT-III and DINOv2, and those with a pre-norm
+(`norm_pre`, timm `pre_norm=True`) and QuickGELU (`blocks[i].mlp.act`): the CLIP image towers.
 
 The reference walks any timm `VisionTransformer`, so every timm-layout module the engine would not compute exactly is
-refused here by name (`_refuse_timm_extras`) instead of being run without it. HF `Dinov2*` classes fail the reference's
-walk (`layer[i].intermediate`) and fail here the same way.
+refused here by name (`_refuse_timm_extras`, `_ffn_act`) instead of being run without it. HF `Dinov2*` classes fail the
+reference's walk (`layer[i].intermediate`) and fail here the same way.
 """
 from __future__ import annotations
 
@@ -113,6 +114,8 @@ class Anatomy:
     register_tokens: int = 0              # R timm register tokens after CLS (globals_ "reg", [R, D])
     pos_covers_prefix: bool = True        # False: timm no_embed_class, the position table has G^2 rows (patches only)
     layer_scale: bool = False             # blocks carry "ls1" / "ls2" gammas [D] (timm LayerScale)
+    pre_norm: bool = False                # LayerNorm over every token before block 0 (globals_ "norm_pre_w" / "norm_pre_b")
+    ffn_act: str = "gelu"                 # MLP activation of every block: "gelu" (erf) or "quick_gelu" (x * sigmoid(1.702 x))
     globals_: Dict[str, Optional[torch.Tensor]] = field(default_factory=dict)
     blocks: List[Dict[str, Optional[torch.Tensor]]] = field(default_factory=list)
 
@@ -157,9 +160,8 @@ def _is_identity(m) -> bool:
 def _refuse_timm_extras(root, blocks) -> None:
     """AttributeError naming every timm VisionTransformer feature the engine does not compute: a model that has one is
     refused rather than run without it."""
-    for name in ("norm_pre", "fc_norm"):
-        if not _is_identity(getattr(root, name, None)):
-            raise AttributeError(f"{name} ({type(getattr(root, name)).__name__}) is not supported: only Identity")
+    if not _is_identity(getattr(root, "fc_norm", None)):
+        raise AttributeError(f"fc_norm ({type(root.fc_norm).__name__}) is not supported: only Identity")
     if not _is_identity(getattr(getattr(root, "patch_embed", None), "norm", None)):
         raise AttributeError("patch_embed.norm is not supported: only Identity")
     pool = getattr(root, "global_pool", "token")
@@ -178,6 +180,59 @@ def _refuse_timm_extras(root, blocks) -> None:
             m = getattr(getattr(b, owner, None), name, None)
             if not _is_identity(m):
                 raise AttributeError(f"blocks[{i}].{owner}.{name} ({type(m).__name__}) is not supported: only Identity")
+
+
+def _norm_pre(root, hidden: int) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """(weight, bias) of timm's `norm_pre` LayerNorm (pre_norm=True: CLIP towers), or (None, None) when it is Identity. A
+    non-affine LayerNorm is taken as ones / zeros. The engine carries one LayerNorm eps, that of `norm`."""
+    m = getattr(root, "norm_pre", None)
+    if _is_identity(m):
+        return None, None
+    if not isinstance(m, nn.LayerNorm) or tuple(m.normalized_shape) != (hidden,):  # timm's LayerNorm subclasses nn.LayerNorm
+        raise AttributeError(f"norm_pre ({type(m).__name__}) is not supported: only Identity or nn.LayerNorm({hidden})")
+    if float(m.eps) != float(root.norm.eps):
+        raise AttributeError(f"norm_pre.eps={m.eps} differs from norm.eps={root.norm.eps}: the engine applies one LayerNorm eps")
+    w = _p(m.weight) if m.weight is not None else torch.ones(hidden)
+    b = _p(m.bias) if m.bias is not None else torch.zeros(hidden)
+    return w, b
+
+
+def _act_kind(act) -> Optional[str]:
+    """'gelu' (erf), 'quick_gelu', or None for any other module. timm cannot be imported here, so its activation classes
+    are matched by name: timm.layers.GELU wraps F.gelu (erf), QuickGELU is x * sigmoid(1.702 x)."""
+    if isinstance(act, nn.GELU):
+        return "gelu" if act.approximate == "none" else None
+    name = type(act).__name__
+    return {"GELU": "gelu", "QuickGELU": "quick_gelu"}.get(name)
+
+
+def ffn_act_signature(vit_model) -> tuple:
+    """Per block: the class of `mlp.act` and its `approximate` setting (timm layout; () for HF models, whose activation
+    is a config string). Parameter-free, so the parameter signature of a cached engine does not see a swapped module."""
+    try:
+        kind, blocks = get_blocks(vit_model)
+    except AttributeError:
+        return ()
+    if kind != "timm":
+        return ()
+    acts = [getattr(getattr(b, "mlp", None), "act", None) for b in blocks]
+    return tuple((type(a), getattr(a, "approximate", None)) for a in acts)
+
+
+def _ffn_act(blocks) -> str:
+    """The one MLP activation of every block: AttributeError naming the block for any other module or a mix of kinds."""
+    kinds = []
+    for i, b in enumerate(blocks):
+        act = getattr(b.mlp, "act", None)
+        kind = _act_kind(act)
+        if kind is None:
+            what = type(act).__name__ + (f", approximate={act.approximate!r}" if isinstance(act, nn.GELU) else "")
+            raise AttributeError(f"blocks[{i}].mlp.act ({what}) is not supported: only erf GELU or QuickGELU")
+        if kinds and kind != kinds[0]:
+            raise AttributeError(f"blocks[{i}].mlp.act ({type(act).__name__}) differs from blocks[0].mlp.act "
+                                 f"({type(blocks[0].mlp.act).__name__}): every block must use the same activation")
+        kinds.append(kind)
+    return kinds[0]
 
 
 def _layer_scale(block, name: str, index: int) -> Optional[torch.Tensor]:
@@ -206,6 +261,7 @@ def describe(vit_model) -> Anatomy:
     hdw = hdb = None
     dist = False
     n_reg, pos_covers_prefix, layer_scale = 0, True, False
+    ffn_act = "gelu"
     if kind == "hf":
         vit = _hf_root(vit_model)
         emb = vit.embeddings
@@ -252,6 +308,8 @@ def describe(vit_model) -> Anatomy:
     else:
         root = vit_model
         _refuse_timm_extras(root, blocks)
+        ffn_act = _ffn_act(blocks)
+        npw, npb = _norm_pre(root, hidden)
         conv = root.patch_embed.proj
         final_ln = root.norm
         head = _head(getattr(root, "head", None))
@@ -272,6 +330,7 @@ def describe(vit_model) -> Anatomy:
             "final_ln_w": _p(final_ln.weight), "final_ln_b": _p(final_ln.bias), "head0_w": h0, "head_w": hw, "head_b": hb,
             "dist": _p(getattr(root, "dist_token", None)), "head_dist_w": hdw, "head_dist_b": hdb,
             "reg": None if reg is None else _p(reg).reshape(n_reg, hidden),
+            "norm_pre_w": npw, "norm_pre_b": npb,
         }
         gammas = [(_layer_scale(b, "ls1", i), _layer_scale(b, "ls2", i)) for i, b in enumerate(blocks)]
         layer_scale = any(g is not None for pair in gammas for g in pair)
@@ -316,5 +375,6 @@ def describe(vit_model) -> Anatomy:
         channels=channels, n_classes=int(n_classes), head_hidden=int(head_hidden), ln_eps=eps,
         ffn_dims=[int(p[0].weight.size(0)) for p in pairs], attn_present=[has_attention(kind, b) for b in blocks],
         score_point=score_point, prefix_tokens=prefix, dist_head=dist, dist_token=dist_tok, register_tokens=n_reg,
-        pos_covers_prefix=pos_covers_prefix, layer_scale=layer_scale, globals_=g, blocks=blks,
+        pos_covers_prefix=pos_covers_prefix, layer_scale=layer_scale, pre_norm=g.get("norm_pre_w") is not None,
+        ffn_act=ffn_act, globals_=g, blocks=blks,
     )

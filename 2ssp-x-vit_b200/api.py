@@ -25,7 +25,8 @@ import torch.nn as nn
 from . import _lib as L
 from . import distributed as D
 from . import ops
-from .anatomy import (attention_module, gather_mlp_pairs, get_blocks, get_encoder, has_attention, install_bypass)
+from .anatomy import (attention_module, ffn_act_signature, gather_mlp_pairs, get_blocks, get_encoder, has_attention,
+                      install_bypass)
 from .engine import Engine, _cuda_device
 
 __all__ = [
@@ -87,7 +88,8 @@ _ENGINES: "weakref.WeakKeyDictionary[nn.Module, Dict[str, Any]]" = weakref.WeakK
 
 def _signature(model) -> tuple:
     """What a cached engine's weights were packed from: address, in-place version and shape of every parameter (a rebound
-    Parameter changes the address, an in-place update the version, a view of the same storage the shape)."""
+    Parameter changes the address, an in-place update the version, a view of the same storage the shape), and the MLP
+    activation of every block (a parameter-free module: a swapped `mlp.act` changes nothing above)."""
     sig = []
     stack = [model]  # a plain walk of the module tree: model.parameters() spends 4x as long building names and a de-dup set
     while stack:
@@ -96,6 +98,7 @@ def _signature(model) -> tuple:
             if p is not None:
                 sig.append((p.data_ptr(), p._version, p.shape))
         stack.extend(m for m in mod._modules.values() if m is not None)
+    sig.append(ffn_act_signature(model))
     return tuple(sig)
 
 

@@ -331,7 +331,7 @@ static int gemm(int mode, const void* A, int lda, const void* W, int ldw, void* 
     if ((N & 7) || (K & 7)) return fail("gemm: N=%d and K=%d must be multiples of 8", N, K);
     const bool f32_out = (mode == EPI_F32 || mode == EPI_F32_SCALED);
     if (mode == EPI_F32_SCALED && col_scale == nullptr) return fail("gemm: scaled fp32 epilogue needs a column scale");
-    const bool score = (mode == EPI_BF16_GELU_SCORE || mode == EPI_BF16_GELU_SCORE_PRE);
+    const bool score = gemm_mode_scores(mode);
     if (score && (partials == nullptr || T < 32 || ldp < N)) return fail("gemm: score epilogue needs partials, ldp >= N and T >= 32 (T=%d)", T);
     const CUtensorMap *ta, *tb, *tc;
     TSSP_TRY(get_tmap(&ta, A, false, K, M, static_cast<uint64_t>(lda) * 2, 64, 128));
@@ -380,6 +380,8 @@ static int gemm(int mode, const void* A, int lda, const void* W, int ldw, void* 
         TSSP_GEMM_CASE(EPI_BF16_GELU_SCORE_PRE)
         TSSP_GEMM_CASE(EPI_F32)
         TSSP_GEMM_CASE(EPI_BF16_ROWNORM)
+        TSSP_GEMM_CASE(EPI_BF16_QGELU)
+        TSSP_GEMM_CASE(EPI_BF16_QGELU_SCORE_PRE)
 #undef TSSP_GEMM_CASE
         default: return fail("gemm: unknown epilogue mode %d", mode);
     }
@@ -424,10 +426,13 @@ static int op_im2col(const float* pixels, void* out, int n, int C, int H, int W,
     return 0;
 }
 
-static int op_layernorm(const float* x, long long in_stride, const float* g, const float* b, void* out, int rows, int D, float eps, cudaStream_t s,
-                        bool stream_in = false) {
+// out: bf16 rows of pitch D, or (f32_out) fp32 rows of pitch out_stride; an fp32 out may be x itself
+static int op_layernorm_any(const float* x, long long in_stride, const float* g, const float* b, void* out, bool f32_out,
+                            long long out_stride, int rows, int D, float eps, cudaStream_t s, bool stream_in) {
     if (((D & 127) && D != 192) || D > 1024) return fail("layernorm: D=%d must be 192 or a multiple of 128 <= 1024", D);
     if (in_stride & 3) return fail("layernorm: row pitch %lld must be a multiple of 4 elements", in_stride);
+    if (f32_out && ((out_stride & 3) || out_stride < D))
+        return fail("layernorm: output row pitch %lld must be a multiple of 4 elements and >= D=%d", out_stride, D);
     if (rows <= 0) return 0;
     // persistent: resident CTAs per SM. Narrow rows need more warps for the same bytes in flight; at D = 1024 the kernel
     // holds 150 registers (row, prefetched row, gamma, beta), so 12 warps fit as three CTAs of 128 threads but only 8
@@ -438,12 +443,16 @@ static int op_layernorm(const float* x, long long in_stride, const float* g, con
     const int ctas = ceil_div(rows, threads / 32);
     const int grid = ctas < per_sm * num_sms() ? ctas : per_sm * num_sms();
     __nv_bfloat16* o = static_cast<__nv_bfloat16*>(out);
+    float* of = static_cast<float*>(out);
     const int rev = chain_dir();
     const int hint = stream_in ? 1 : 0;
+#define TSSP_LN_LAUNCH(kbf16, kf32)                                                                                                 \
+    TSSP_CUDA(f32_out ? launch_pdl(kf32, dim3(grid), dim3(threads), 0, s, x, in_stride, g, b, of, out_stride, rows, eps, rev, hint) \
+                      : launch_pdl(kbf16, dim3(grid), dim3(threads), 0, s, x, in_stride, g, b, o, rows, eps, rev, hint))
 #define TSSP_LN_CASE(d, NS, VPL) \
-    case d: TSSP_CUDA(launch_pdl(layernorm_bf16_slab_kernel<NS, VPL>, dim3(grid), dim3(threads), 0, s, x, in_stride, g, b, o, rows, eps, rev, hint)); break;
+    case d: TSSP_LN_LAUNCH((layernorm_bf16_slab_kernel<NS, VPL>), (layernorm_f32_slab_kernel<NS, VPL>)); break;
     switch (D) {
-        case 192: TSSP_CUDA(launch_pdl(layernorm_bf16_slab64_kernel<3>, dim3(grid), dim3(threads), 0, s, x, in_stride, g, b, o, rows, eps, rev, hint)); break;
+        case 192: TSSP_LN_LAUNCH(layernorm_bf16_slab64_kernel<3>, layernorm_f32_slab64_kernel<3>); break;
         TSSP_LN_CASE(128, 1, 1)
         TSSP_LN_CASE(256, 1, 2)
         TSSP_LN_CASE(384, 3, 1)
@@ -455,8 +464,18 @@ static int op_layernorm(const float* x, long long in_stride, const float* g, con
         default: return fail("layernorm: D=%d has no kernel instance", D);
     }
 #undef TSSP_LN_CASE
-    TSSP_LAUNCH_CHECK("layernorm_bf16_slab_kernel");
+#undef TSSP_LN_LAUNCH
+    TSSP_LAUNCH_CHECK(f32_out ? "layernorm_f32_slab_kernel" : "layernorm_bf16_slab_kernel");
     return 0;
+}
+
+static int op_layernorm(const float* x, long long in_stride, const float* g, const float* b, void* out, int rows, int D, float eps, cudaStream_t s,
+                        bool stream_in = false) {
+    return op_layernorm_any(x, in_stride, g, b, out, false, D, rows, D, eps, s, stream_in);
+}
+static int op_layernorm_f32(const float* x, long long in_stride, const float* g, const float* b, float* out, long long out_stride, int rows,
+                            int D, float eps, cudaStream_t s) {
+    return op_layernorm_any(x, in_stride, g, b, out, true, out_stride, rows, D, eps, s, false);
 }
 
 // 3-D tensor map over a token-major bf16 activation viewed as [n_img][T][width] (width = 3D for the fused qkv, D for
@@ -603,6 +622,7 @@ struct tssp_engine {
     int device;
     int T, M_cap, Kp, G;
     tssp_layout_t layout;
+    tssp_model_opts_t opts;
     int prefix;     // tokens ahead of the patches: 1 (CLS) + layout.dist_token + layout.register_tokens
     int head_rows;  // rows the classifier may read: 2 with a distillation token (CLS, distillation), else 1 (CLS)
     bool dist_head; // a distillation head is loaded: logits = (cls_head(row 0) + dist_head(row 1)) / 2
@@ -616,6 +636,7 @@ struct tssp_engine {
     // global weights
     __nv_bfloat16 *patch_w, *head0_w, *head_w, *head_dist_w;  // with a distillation head both heads are packed at 0.5 scale
     float *posmod, *final_ln_w, *final_ln_b, *head_b, *head_dist_b;
+    float *norm_pre_w, *norm_pre_b;  // opts.pre_norm: LayerNorm over every token before block 0, else nullptr
     int Cp, Hhp;  // padded classes / head hidden
     // workspace
     float* pixels[2];          // double-buffered staging of host pixel batches
@@ -712,7 +733,12 @@ static int dev_alloc(tssp_engine* e, Tp** out, size_t count) {
     return 0;
 }
 
-static int validate(const tssp_config_t& c, const tssp_layout_t& l) {
+static int validate(const tssp_config_t& c, const tssp_layout_t& l, const tssp_model_opts_t& o) {
+    if (o.pre_norm != 0 && o.pre_norm != 1) return fail("options: pre_norm=%d must be 0 or 1", o.pre_norm);
+    if (o.ffn_act != TSSP_FFN_GELU && o.ffn_act != TSSP_FFN_QUICK_GELU)
+        return fail("options: ffn_act=%d must be %d (erf GELU) or %d (QuickGELU)", o.ffn_act, TSSP_FFN_GELU, TSSP_FFN_QUICK_GELU);
+    if (o.ffn_act == TSSP_FFN_QUICK_GELU && c.score_point != 1)
+        return fail("options: QuickGELU is scored before the activation only (score_point=1, got %d)", c.score_point);
     if (l.dist_token != 0 && l.dist_token != 1) return fail("layout: dist_token=%d must be 0 or 1", l.dist_token);
     if (l.register_tokens < 0 || l.register_tokens > TSSP_MAX_REGISTER_TOKENS)
         return fail("layout: register_tokens=%d must be in [0,%d]", l.register_tokens, TSSP_MAX_REGISTER_TOKENS);
@@ -734,8 +760,9 @@ static int validate(const tssp_config_t& c, const tssp_layout_t& l) {
     return 0;
 }
 
-static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, int device, tssp_engine** out) {
-    TSSP_TRY(validate(*cfg, layout));
+static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, const tssp_model_opts_t& opts, int device,
+                         tssp_engine** out) {
+    TSSP_TRY(validate(*cfg, layout, opts));
     const int prefix = 1 + layout.dist_token + layout.register_tokens;
     int n_dev = 0;
     TSSP_CUDA(cudaGetDeviceCount(&n_dev));
@@ -752,6 +779,7 @@ static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, 
     const int D = cfg->hidden, B = cfg->n_blocks;
     e->G = cfg->image_size / cfg->patch_size;
     e->layout = layout;
+    e->opts = opts;
     e->prefix = prefix;
     e->head_rows = 1 + layout.dist_token;
     e->dist_head = false;
@@ -772,6 +800,12 @@ static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, 
     A(&e->head_b, e->Cp);
     e->head_dist_w = nullptr;
     e->head_dist_b = nullptr;
+    e->norm_pre_w = nullptr;
+    e->norm_pre_b = nullptr;
+    if (opts.pre_norm) {
+        A(&e->norm_pre_w, D);
+        A(&e->norm_pre_b, D);
+    }
     if (layout.dist_token && cfg->n_classes > 0) {
         A(&e->head_dist_w, static_cast<size_t>(e->Cp) * D);
         A(&e->head_dist_b, e->Cp);
@@ -897,10 +931,11 @@ static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cud
     const int D = c.hidden, B = c.n_blocks;
     const tssp_layout_t& l = e->layout;
     const int n_ext = l.dist_token ? TSSP_WX_COUNT : 0;
-    const int n_expected = TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT + n_ext + (l.register_tokens > 0 ? 1 : 0) + (l.layer_scale ? 2 * B : 0);
+    const int n_layout = (l.register_tokens > 0 ? 1 : 0) + (l.layer_scale ? 2 * B : 0);
+    const int n_expected = TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT + n_ext + n_layout + (e->opts.pre_norm ? 2 : 0);
     if (n_entries != n_expected)
-        return fail("load_weights: expected %d pointers for %d prefix token(s)%s, got %d", n_expected, e->prefix,
-                    l.layer_scale ? " and LayerScale" : "", n_entries);
+        return fail("load_weights: expected %d pointers for %d prefix token(s)%s%s, got %d", n_expected, e->prefix,
+                    l.layer_scale ? " and LayerScale" : "", e->opts.pre_norm ? " and a pre-norm" : "", n_entries);
     auto need = [&](int idx, const char* name) -> int { return t[idx] == nullptr ? fail("load_weights: %s is NULL", name) : 0; };
     TSSP_TRY(need(TSSP_W_PATCH_W, "patch_w")); TSSP_TRY(need(TSSP_W_CLS, "cls_token")); TSSP_TRY(need(TSSP_W_POS, "pos_embed"));
     TSSP_TRY(need(TSSP_W_FINAL_LN_W, "final_ln_w")); TSSP_TRY(need(TSSP_W_FINAL_LN_B, "final_ln_b"));
@@ -908,7 +943,9 @@ static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cud
     const float* const* lx = x + n_ext;                                  // layout entries (tssp_create_layout)
     const float* reg_tokens = l.register_tokens > 0 ? lx[0] : nullptr;
     const float* const* ls = lx + (l.register_tokens > 0 ? 1 : 0);       // per block LS1, LS2
+    const float* const* pn = lx + n_layout;                              // option entries (tssp_create_model): norm_pre
     if (l.register_tokens > 0 && reg_tokens == nullptr) return fail("load_weights: register tokens are NULL");
+    if (e->opts.pre_norm && (pn[0] == nullptr || pn[1] == nullptr)) return fail("load_weights: norm_pre weight or bias is NULL");
     if (l.layer_scale)
         for (int b = 0; b < B; ++b) {
             if (ls[2 * b + 1] == nullptr) return fail("load_weights: block %d LS2 gamma is NULL", b);
@@ -927,6 +964,10 @@ static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cud
     TSSP_LAUNCH_CHECK("build_posmod_kernel");
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_W], D, e->final_ln_w, D, s));
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_B], D, e->final_ln_b, D, s));
+    if (e->opts.pre_norm) {
+        TSSP_TRY(copy_vec(pn[0], D, e->norm_pre_w, D, s));
+        TSSP_TRY(copy_vec(pn[1], D, e->norm_pre_b, D, s));
+    }
     if (c.n_classes > 0 && dist_head) {
         // (cls_head(x0) + dist_head(x1)) / 2 as two GEMMs into the same logits (run_head): both heads at half scale
         TSSP_TRY(need(TSSP_W_HEAD_W, "head_w"));
@@ -1133,7 +1174,8 @@ static int run_im2col(tssp_engine* e, const float* dev_pixels, int n, cudaStream
     return 0;
 }
 
-// embeddings: x = [cls | patches W^T + b] + pos      (HF ViTEmbeddings / ViTPatchEmbeddings)
+// embeddings: x = [cls | patches W^T + b] + pos      (HF ViTEmbeddings / ViTPatchEmbeddings); with a pre-norm (timm
+// pre_norm=True: CLIP towers) x = norm_pre(x), in place, before block 0 (and so before the Stage-2 snapshot of block 0)
 static int run_embed(tssp_engine* e, int n, cudaStream_t s) {
     e->launch.chain_dir = 0;  // every batch starts its chain in the same direction
     const tssp_config_t& c = e->cfg;
@@ -1144,6 +1186,7 @@ static int run_embed(tssp_engine* e, int n, cudaStream_t s) {
         TSSP_LAUNCH_CHECK("broadcast_rows_kernel");
     }
     TSSP_PROF(KC_PATCH, s, gemm(EPI_F32, e->patchA, e->Kp, e->patch_w, e->Kp, e->x, D, M, D, e->Kp, nullptr, nullptr, 0, e->T, 1, s));
+    if (e->opts.pre_norm) TSSP_PROF(KC_LN, s, op_layernorm_f32(e->x, D, e->norm_pre_w, e->norm_pre_b, e->x, D, M, D, c.ln_eps, s));
     return 0;
 }
 
@@ -1166,6 +1209,8 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     const int rows = cls_only ? n : M;              // rows the row-wise part of the block works on
     const int pitch = cls_only ? e->T * D : D;      // their distance in x / ctx
     const bool attn = e->attn_present[b] && !skip_attn;
+    const bool qgelu = e->opts.ffn_act == TSSP_FFN_QUICK_GELU;
+    const int fc1_plain = qgelu ? EPI_BF16_QGELU : EPI_BF16_GELU;
     // proj / fc2 add their branch into the residual stream, scaled by the block's LayerScale gamma when the model has one
     auto residual_gemm = [&](const void* A, int lda, const __nv_bfloat16* W, int ldw, float* xr, int rows_, int K, const float* bias,
                              const float* gamma) {
@@ -1183,7 +1228,7 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
             float* xr = e->x + static_cast<size_t>(r) * D;
             if (attn) TSSP_PROF(KC_PROJ, s, residual_gemm(e->ctx + static_cast<size_t>(r) * D, pitch, w.proj_w, D, xr, n, D, w.proj_b, w.ls1));
             TSSP_PROF(KC_LN, s, op_layernorm(xr, pitch, w.ln2_w, w.ln2_b, e->xn, n, D, c.ln_eps, s));
-            TSSP_PROF(KC_FC1, s, gemm(EPI_BF16_GELU, e->xn, D, w.fc1_w, D, e->h, w.Fp, n, w.Fp, D, w.fc1_b, nullptr, 0, e->T, 0, s));
+            TSSP_PROF(KC_FC1, s, gemm(fc1_plain, e->xn, D, w.fc1_w, D, e->h, w.Fp, n, w.Fp, D, w.fc1_b, nullptr, 0, e->T, 0, s));
             TSSP_PROF(KC_FC2, s, residual_gemm(e->h, w.Fp, w.fc2_w, w.Fp, xr, n, w.Fp, w.fc2_b, w.ls2));
         }
         return 0;
@@ -1191,13 +1236,14 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     if (attn) TSSP_PROF(KC_PROJ, s, residual_gemm(e->ctx, pitch, w.proj_w, D, e->x, rows, D, w.proj_b, w.ls1));
     TSSP_PROF(KC_LN, s, op_layernorm(e->x, pitch, w.ln2_w, w.ln2_b, e->xn, rows, D, c.ln_eps, s, /*stream_in=*/!cls_only));
     if (fc1_mode == FC1_SCORE) {
-        const int mode = c.score_point == 1 ? EPI_BF16_GELU_SCORE_PRE : EPI_BF16_GELU_SCORE;
+        // QuickGELU engines score before the activation only (validate)
+        const int mode = c.score_point == 1 ? (qgelu ? EPI_BF16_QGELU_SCORE_PRE : EPI_BF16_GELU_SCORE_PRE) : EPI_BF16_GELU_SCORE;
         // per-block partial sums of squares; the square roots and the image sums are taken once per batch
         // for all blocks together (finish_scores)
         TSSP_PROF(KC_FC1, s, gemm(mode, e->xn, D, w.fc1_w, D, e->h, w.Fp, M, w.Fp, D, w.fc1_b,
                                   e->partials + static_cast<size_t>(b) * e->partials_stride, w.Fp, e->T, 0, s));
     } else {
-        TSSP_PROF(KC_FC1, s, gemm(EPI_BF16_GELU, e->xn, D, w.fc1_w, D, e->h, w.Fp, rows, w.Fp, D, w.fc1_b, nullptr, 0, e->T, 0, s));
+        TSSP_PROF(KC_FC1, s, gemm(fc1_plain, e->xn, D, w.fc1_w, D, e->h, w.Fp, rows, w.Fp, D, w.fc1_b, nullptr, 0, e->T, 0, s));
     }
     if (run_fc2) TSSP_PROF(KC_FC2, s, residual_gemm(e->h, w.Fp, w.fc2_w, w.Fp, e->x, rows, w.Fp, w.fc2_b, w.ls2));
     return 0;
@@ -1341,10 +1387,16 @@ int tssp_profile_end(double* ms_per_class, unsigned long long* launches_per_clas
     return 0;
 }
 
-int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, int device, tssp_handle_t* out) {
+int tssp_create_model(const tssp_config_t* cfg, const tssp_layout_t* layout, const tssp_model_opts_t* opts, int device,
+                      tssp_handle_t* out) {
     TSSP_ENTRY();
-    if (cfg == nullptr || layout == nullptr || out == nullptr) return fail("tssp_create: NULL argument");
-    return engine_create(cfg, *layout, device, out);
+    if (cfg == nullptr || layout == nullptr || opts == nullptr || out == nullptr) return fail("tssp_create: NULL argument");
+    return engine_create(cfg, *layout, *opts, device, out);
+}
+
+int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, int device, tssp_handle_t* out) {
+    const tssp_model_opts_t opts = {0, TSSP_FFN_GELU};
+    return tssp_create_model(cfg, layout, &opts, device, out);
 }
 
 int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out) {
@@ -1707,6 +1759,12 @@ int tssp_op_layernorm(const float* x, int64_t in_stride, const float* gamma, con
     TSSP_ENTRY();
     if (x == nullptr || gamma == nullptr || beta == nullptr || out_bf16 == nullptr) return fail("tssp_op_layernorm: NULL argument");
     return op_layernorm(x, in_stride, gamma, beta, out_bf16, rows, D, eps, static_cast<cudaStream_t>(stream));
+}
+int tssp_op_layernorm_f32(const float* x, int64_t in_stride, const float* gamma, const float* beta, float* out_f32, int64_t out_stride,
+                          int rows, int D, float eps, void* stream) {
+    TSSP_ENTRY();
+    if (x == nullptr || gamma == nullptr || beta == nullptr || out_f32 == nullptr) return fail("tssp_op_layernorm_f32: NULL argument");
+    return op_layernorm_f32(x, in_stride, gamma, beta, out_f32, out_stride, rows, D, eps, static_cast<cudaStream_t>(stream));
 }
 int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream) {
     TSSP_ENTRY();

@@ -23,6 +23,8 @@
 //                           stream, so the residual is never loaded by the SMs   (proj, fc2, patch-embed, head)
 //       EPI_F32_SCALED      out fp32 (=|+=) col_scale[c] * (acc + bias[c])   (proj / fc2 of LayerScale blocks: timm
 //                           LayerScale.forward multiplies the branch output by gamma before the residual add)
+//       EPI_BF16_QGELU, EPI_BF16_QGELU_SCORE_PRE   EPI_BF16_GELU / EPI_BF16_GELU_SCORE_PRE with QuickGELU,
+//                           x * sigmoid(1.702 x), in place of erf GELU (fc1 of the OpenAI CLIP image towers)
 //     Output tiles leave through a 4 KB per-warp staging slot and TMA stores (clipped at the tensor edge).
 #pragma once
 #include <type_traits>
@@ -39,7 +41,14 @@ enum GemmMode : int {
     EPI_F32 = 4,
     EPI_BF16_ROWNORM = 5,  // EPI_BF16 + per-(row, 64-column chunk) sum of squares (|q|^2, |k|^2 per head for attention)
     EPI_F32_SCALED = 6,    // EPI_F32 with a per-column scale applied after the bias (LayerScale)
+    EPI_BF16_QGELU = 7,    // EPI_BF16_GELU with QuickGELU
+    EPI_BF16_QGELU_SCORE_PRE = 8,  // EPI_BF16_GELU_SCORE_PRE with QuickGELU (the squares are taken before the activation)
 };
+
+// epilogues that write Stage-1 score partials (32-row sub-tile, image segment, neuron)
+__host__ __device__ constexpr bool gemm_mode_scores(int mode) {
+    return mode == EPI_BF16_GELU_SCORE || mode == EPI_BF16_GELU_SCORE_PRE || mode == EPI_BF16_QGELU_SCORE_PRE;
+}
 
 struct GemmParams {
     int M;                  // valid rows of A / C (rows >= M are never scored; stores clip at the tensor map)
@@ -135,6 +144,20 @@ __device__ __forceinline__ void gelu_erf_x2(float& x0, float& x1) {
     const uint64_t q = pack_f32x2(ex2_approx(p0), ex2_approx(p1));
     const uint64_t r = fma_f32x2(pack_f32x2(-a0, -a1), q, pack_f32x2(fmaxf(x0, 0.0f), fmaxf(x1, 0.0f)));
     unpack_f32x2(r, x0, x1);
+}
+
+// quickgelu(x) = x * sigmoid(1.702 x) = x / (1 + 2^(-1.702 log2(e) x)): one MUFU.EX2 and one MUFU.RCP per element, plus
+// an FMUL and an FADD with immediate operands and the final FMUL. (The same with packed FMUL2 / FADD2 needs the constants in
+// register pairs: in the 168-register epilogue it spilled 12 bytes more than this form, in both modes.) Both approximations are within a few fp32 ulps, so the result is
+// within a fraction of a bf16 ulp of the exact value for |x| <= 50 (below about -51, 1 + 2^y exceeds 2^126 and the
+// reciprocal flushes to zero: the result is -0 instead of a value under 1e-36). The one-MUFU form
+// 0.5 x (1 + tanh.approx(0.851 x)) is not used: tanh.approx has about 2^-11 relative error and 1 + tanh cancels for
+// negative x (4 % off at x = -3).
+__device__ __forceinline__ void quick_gelu_x2(float& x0, float& x1) {
+    using namespace ptx;
+    constexpr float K = -2.45546696f;  // -1.702 * log2(e)
+    x0 = x0 * rcp_approx(1.0f + ex2_approx(K * x0));
+    x1 = x1 * rcp_approx(1.0f + ex2_approx(K * x1));
 }
 
 __device__ __forceinline__ float bf16_lo(uint32_t w) { return __uint_as_float(w << 16); }
@@ -309,7 +332,7 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
             };
             // image segmentation of this warp's 32 rows (SCORE modes)
             int seg_split = 0, seg_end = 0;
-            if constexpr (MODE == EPI_BF16_GELU_SCORE || MODE == EPI_BF16_GELU_SCORE_PRE) {
+            if constexpr (gemm_mode_scores(MODE)) {
                 const int valid = min(32, max(0, p.M - row0));
                 const int img0 = row0 / p.tokens_per_image;
                 seg_end = valid;
@@ -382,7 +405,8 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
 
                 if constexpr (Cfg::OUT_BF16) {
                     constexpr bool GELU = (MODE == EPI_BF16_GELU || MODE == EPI_BF16_GELU_SCORE || MODE == EPI_BF16_GELU_SCORE_PRE);
-                    constexpr bool PRE = (MODE == EPI_BF16_GELU_SCORE_PRE);
+                    constexpr bool QGELU = (MODE == EPI_BF16_QGELU || MODE == EPI_BF16_QGELU_SCORE_PRE);
+                    constexpr bool PRE = (MODE == EPI_BF16_GELU_SCORE_PRE || MODE == EPI_BF16_QGELU_SCORE_PRE);
                     // non-PRE modes stage each half as soon as it is packed, so only 16 packed words are ever live;
                     // the PRE mode (rare path) keeps the whole chunk twice: pre-activation values and activations
                     uint32_t packed[PRE ? 32 : 16];
@@ -436,6 +460,10 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
                             if constexpr (GELU) {
                                 gelu_erf_x2(v0, v1);
                                 gelu_erf_x2(v2, v3);
+                            }
+                            if constexpr (QGELU) {
+                                quick_gelu_x2(v0, v1);
+                                quick_gelu_x2(v2, v3);
                             }
                             packed[po + j / 2] = pack_bf16x2(v0, v1);
                             packed[po + j / 2 + 1] = pack_bf16x2(v2, v3);
@@ -516,7 +544,7 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
                     // was measured: no faster)
                     if constexpr (MODE == EPI_BF16_GELU_SCORE) score_pass();
                     GEMM_TRACE(e == 0 && lane == 0, it, cc == 0 ? 9 : 14);
-                    if constexpr (MODE == EPI_BF16_GELU_SCORE || MODE == EPI_BF16_GELU_SCORE_PRE) {
+                    if constexpr (gemm_mode_scores(MODE)) {
                         const int gc = gcol0 + 2 * lane;
                         if (gc < p.N && row0 < p.M) {
                             const size_t sub = static_cast<size_t>(row0 >> 5);

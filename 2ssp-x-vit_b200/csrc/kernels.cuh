@@ -131,7 +131,8 @@ __global__ void broadcast_rows_kernel(const float* __restrict__ table, float* __
 }
 
 // ------------------------------------------------------------------------------------------------
-// LayerNorm over the last dim, fp32 in (row pitch in_stride elements) -> bf16 out (pitch D); D % 128 == 0, D <= 1024.
+// LayerNorm over the last dim, fp32 in (row pitch in_stride elements) -> bf16 out (pitch D) or fp32 out (any pitch);
+// D % 128 == 0, D <= 1024, or D = 192.
 // ------------------------------------------------------------------------------------------------
 // Persistent LayerNorm: a fixed grid (a multiple of the SM count) walks the rows, one warp per row, and every warp has the
 // NEXT row's loads in flight while it reduces / normalises / stores the current one. A row is NSLAB slabs of 128 * VPL
@@ -140,12 +141,13 @@ __global__ void broadcast_rows_kernel(const float* __restrict__ table, float* __
 //   VPL = 1 (odd multiples of 128: ViT-S 384): one 128-bit load and one 64-bit store per slab.
 // gamma / beta stay in registers (re-reading them from L1 at D = 1024 to save 64 registers was measured slower -- the
 // launcher gives that width three CTAs of 128 threads per SM instead).
-template <int NSLAB, int VPL>
-__global__ void __launch_bounds__(256) layernorm_bf16_slab_kernel(const float* __restrict__ x, long long in_stride,
-                                                                  const float* __restrict__ gamma,
-                                                                  const float* __restrict__ beta,
-                                                                  __nv_bfloat16* __restrict__ out, int rows, float eps,
-                                                                  int reverse, int stream_in) {
+// OutT = float: the same rows in fp32 (the pre-norm of CLIP towers, written back into the residual stream). Statistics and
+// arithmetic are the same, so bf16(fp32 output) is the bf16 output bit for bit; out may equal x (a warp has loaded a whole
+// row before it stores any of it, and no other warp touches that row).
+template <int NSLAB, int VPL, typename OutT>
+__device__ __forceinline__ void layernorm_slab_rows(const float* x, long long in_stride, const float* __restrict__ gamma,
+                                                    const float* __restrict__ beta, OutT* out, long long out_stride, int rows,
+                                                    float eps, int reverse, int stream_in) {
     constexpr int D = NSLAB * 128 * VPL;
     // stream_in: x is loaded with an L2 evict-first policy, so the normalised rows this kernel writes (what the next
     // GEMM starts on) are what stays in L2, not the residual rows it has finished with
@@ -153,10 +155,10 @@ __global__ void __launch_bounds__(256) layernorm_bf16_slab_kernel(const float* _
     auto ldx = [&](const float4* p) { return stream_in ? ptx::ld_global_v4_hint(p, in_policy) : *p; };
     if (reverse) {  // walk the rows from the last to the first: re-base the pointers on the last row, negative pitch
         x += static_cast<size_t>(rows - 1) * in_stride;
-        out += static_cast<size_t>(rows - 1) * D;
+        out += static_cast<size_t>(rows - 1) * out_stride;
     }
     const long long xs = reverse ? -in_stride : in_stride;
-    const long long os = reverse ? -static_cast<long long>(D) : static_cast<long long>(D);
+    const long long os = reverse ? -out_stride : out_stride;
     ptx::griddep_launch_dependents();
     ptx::griddep_wait();
     const int lane = threadIdx.x & 31;
@@ -216,7 +218,7 @@ __global__ void __launch_bounds__(256) layernorm_bf16_slab_kernel(const float* _
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
         const float rstd = 1.0f / sqrtf(sq * (1.0f / D) + eps);
-        __nv_bfloat16* dst = out + row * os;
+        OutT* dst = out + row * os;
 #pragma unroll
         for (int i = 0; i < NSLAB; ++i) {
             uint32_t pk[2 * VPL];
@@ -224,35 +226,57 @@ __global__ void __launch_bounds__(256) layernorm_bf16_slab_kernel(const float* _
             for (int h = 0; h < VPL; ++h) {
                 const float4 g = gm[i][h];
                 const float4 bb = bt[i][h];
-                __nv_bfloat162 lo = __floats2bfloat162_rn((v[i][h].x - mean) * rstd * g.x + bb.x, (v[i][h].y - mean) * rstd * g.y + bb.y);
-                __nv_bfloat162 hi = __floats2bfloat162_rn((v[i][h].z - mean) * rstd * g.z + bb.z, (v[i][h].w - mean) * rstd * g.w + bb.w);
-                pk[2 * h] = *reinterpret_cast<uint32_t*>(&lo);
-                pk[2 * h + 1] = *reinterpret_cast<uint32_t*>(&hi);
+                // the same expressions in both forms, so that both contract to the same FFMAs
+                if constexpr (sizeof(OutT) == 4) {
+                    reinterpret_cast<float4*>(dst)[(i * 32 + lane) * VPL + h] =
+                        make_float4((v[i][h].x - mean) * rstd * g.x + bb.x, (v[i][h].y - mean) * rstd * g.y + bb.y,
+                                    (v[i][h].z - mean) * rstd * g.z + bb.z, (v[i][h].w - mean) * rstd * g.w + bb.w);
+                } else {
+                    __nv_bfloat162 lo = __floats2bfloat162_rn((v[i][h].x - mean) * rstd * g.x + bb.x, (v[i][h].y - mean) * rstd * g.y + bb.y);
+                    __nv_bfloat162 hi = __floats2bfloat162_rn((v[i][h].z - mean) * rstd * g.z + bb.z, (v[i][h].w - mean) * rstd * g.w + bb.w);
+                    pk[2 * h] = *reinterpret_cast<uint32_t*>(&lo);
+                    pk[2 * h + 1] = *reinterpret_cast<uint32_t*>(&hi);
+                }
             }
-            if constexpr (VPL == 2) reinterpret_cast<uint4*>(dst)[i * 32 + lane] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-            else reinterpret_cast<uint2*>(dst)[i * 32 + lane] = make_uint2(pk[0], pk[1]);
+            if constexpr (sizeof(OutT) == 2) {
+                if constexpr (VPL == 2) reinterpret_cast<uint4*>(dst)[i * 32 + lane] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+                else reinterpret_cast<uint2*>(dst)[i * 32 + lane] = make_uint2(pk[0], pk[1]);
+            }
         }
     }
+}
+
+template <int NSLAB, int VPL>
+__global__ void __launch_bounds__(256) layernorm_bf16_slab_kernel(const float* __restrict__ x, long long in_stride,
+                                                                  const float* __restrict__ gamma,
+                                                                  const float* __restrict__ beta,
+                                                                  __nv_bfloat16* __restrict__ out, int rows, float eps,
+                                                                  int reverse, int stream_in) {
+    layernorm_slab_rows<NSLAB, VPL>(x, in_stride, gamma, beta, out, NSLAB * 128 * VPL, rows, eps, reverse, stream_in);
+}
+template <int NSLAB, int VPL>
+__global__ void __launch_bounds__(256) layernorm_f32_slab_kernel(const float* x, long long in_stride, const float* __restrict__ gamma,
+                                                                 const float* __restrict__ beta, float* out, long long out_stride,
+                                                                 int rows, float eps, int reverse, int stream_in) {
+    layernorm_slab_rows<NSLAB, VPL>(x, in_stride, gamma, beta, out, out_stride, rows, eps, reverse, stream_in);
 }
 
 // The same persistent walk for widths that are a multiple of 64 but not of 128 (D = 192: DeiT-Ti, ViT-Ti): a row is
 // NSLAB slabs of 64 elements, a lane owns two consecutive elements of each slab -- one 64-bit load and one bf16x2 (32-bit)
 // store per slab, so a warp still reads and writes whole 256-byte / 128-byte rows of a slab.
-template <int NSLAB>
-__global__ void __launch_bounds__(256) layernorm_bf16_slab64_kernel(const float* __restrict__ x, long long in_stride,
-                                                                    const float* __restrict__ gamma,
-                                                                    const float* __restrict__ beta,
-                                                                    __nv_bfloat16* __restrict__ out, int rows, float eps,
-                                                                    int reverse, int stream_in) {
+template <int NSLAB, typename OutT>
+__device__ __forceinline__ void layernorm_slab64_rows(const float* x, long long in_stride, const float* __restrict__ gamma,
+                                                      const float* __restrict__ beta, OutT* out, long long out_stride, int rows,
+                                                      float eps, int reverse, int stream_in) {
     constexpr int D = NSLAB * 64;
     const uint64_t in_policy = ptx::l2_policy_evict_first();
     auto ldx = [&](const float2* p) { return stream_in ? ptx::ld_global_v2_hint(p, in_policy) : *p; };
     if (reverse) {
         x += static_cast<size_t>(rows - 1) * in_stride;
-        out += static_cast<size_t>(rows - 1) * D;
+        out += static_cast<size_t>(rows - 1) * out_stride;
     }
     const long long xs = reverse ? -in_stride : in_stride;
-    const long long os = reverse ? -static_cast<long long>(D) : static_cast<long long>(D);
+    const long long os = reverse ? -out_stride : out_stride;
     ptx::griddep_launch_dependents();
     ptx::griddep_wait();
     const int lane = threadIdx.x & 31;
@@ -298,13 +322,33 @@ __global__ void __launch_bounds__(256) layernorm_bf16_slab64_kernel(const float*
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
         const float rstd = 1.0f / sqrtf(sq * (1.0f / D) + eps);
-        __nv_bfloat16* dst = out + row * os;
+        OutT* dst = out + row * os;
 #pragma unroll
         for (int i = 0; i < NSLAB; ++i) {
-            __nv_bfloat162 pk = __floats2bfloat162_rn((v[i].x - mean) * rstd * gm[i].x + bt[i].x, (v[i].y - mean) * rstd * gm[i].y + bt[i].y);
-            reinterpret_cast<__nv_bfloat162*>(dst)[i * 32 + lane] = pk;
+            if constexpr (sizeof(OutT) == 4) {
+                reinterpret_cast<float2*>(dst)[i * 32 + lane] =
+                    make_float2((v[i].x - mean) * rstd * gm[i].x + bt[i].x, (v[i].y - mean) * rstd * gm[i].y + bt[i].y);
+            } else {
+                __nv_bfloat162 pk = __floats2bfloat162_rn((v[i].x - mean) * rstd * gm[i].x + bt[i].x, (v[i].y - mean) * rstd * gm[i].y + bt[i].y);
+                reinterpret_cast<__nv_bfloat162*>(dst)[i * 32 + lane] = pk;
+            }
         }
     }
+}
+
+template <int NSLAB>
+__global__ void __launch_bounds__(256) layernorm_bf16_slab64_kernel(const float* __restrict__ x, long long in_stride,
+                                                                    const float* __restrict__ gamma,
+                                                                    const float* __restrict__ beta,
+                                                                    __nv_bfloat16* __restrict__ out, int rows, float eps,
+                                                                    int reverse, int stream_in) {
+    layernorm_slab64_rows<NSLAB>(x, in_stride, gamma, beta, out, NSLAB * 64, rows, eps, reverse, stream_in);
+}
+template <int NSLAB>
+__global__ void __launch_bounds__(256) layernorm_f32_slab64_kernel(const float* x, long long in_stride, const float* __restrict__ gamma,
+                                                                   const float* __restrict__ beta, float* out, long long out_stride,
+                                                                   int rows, float eps, int reverse, int stream_in) {
+    layernorm_slab64_rows<NSLAB>(x, in_stride, gamma, beta, out, out_stride, rows, eps, reverse, stream_in);
 }
 
 constexpr int ATT_HD = 64;  // head dimension of every supported ViT (attention_tcgen05.cuh)

@@ -419,6 +419,11 @@ __device__ __forceinline__ float ex2_approx(float x) {
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
 }
+__device__ __forceinline__ float rcp_approx(float x) {
+    float y;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
 
 // Shared-memory matrix descriptor for a K-major bf16 operand tile written by TMA with SWIZZLE_128B:
 // rows are 128 B (64 bf16) apart, 8-row groups are 1024 B apart (SBO), LBO unused for swizzled K-major.

@@ -50,7 +50,12 @@ class Engine:
         self._handle = C.c_void_p()
         with torch.cuda.device(self.device):
             layout = L.TsspLayout(int(a.dist_token), a.register_tokens, int(a.pos_covers_prefix), int(a.layer_scale))
-            L.check(self.lib.tssp_create_layout(C.byref(cfg), C.byref(layout), self.device.index, C.byref(self._handle)))
+            if a.pre_norm or a.ffn_act != "gelu":
+                opts = L.TsspModelOpts(int(a.pre_norm), L.FFN_ACTS[a.ffn_act])
+                L.check(self.lib.tssp_create_model(C.byref(cfg), C.byref(layout), C.byref(opts), self.device.index,
+                                                   C.byref(self._handle)))
+            else:
+                L.check(self.lib.tssp_create_layout(C.byref(cfg), C.byref(layout), self.device.index, C.byref(self._handle)))
         self.ffn_dims = list(a.ffn_dims)
         self.load_weights(a)
         self.anatomy.globals_.clear()
@@ -76,6 +81,8 @@ class Engine:
         if a.layer_scale:
             for blk in a.blocks:
                 entries += [self._dev32(blk.get("ls1"), keep), self._dev32(blk.get("ls2"), keep)]
+        if a.pre_norm:  # then the option entries of tssp_create_model
+            entries += [self._dev32(a.globals_["norm_pre_w"], keep), self._dev32(a.globals_["norm_pre_b"], keep)]
         table = (C.c_void_p * len(entries))(*entries)
         with torch.cuda.device(self.device):
             L.check(self.lib.tssp_load_weights(self._handle, table, len(entries), L.current_stream()))

@@ -43,7 +43,7 @@ def _aligned(t):
 def gemm(mode: int, a: torch.Tensor, w: torch.Tensor, out: torch.Tensor, bias: torch.Tensor | None = None, *,
          m: int | None = None, partials: torch.Tensor | None = None, tokens_per_image: int = 0,
          reduce_add: bool = False) -> torch.Tensor:
-    """out[M,N] (=|+=) epilogue(a[M,K] @ w[N,K]^T + bias). a, w bf16; out bf16 (modes 0-3) or fp32 (mode 4)."""
+    """out[M,N] (=|+=) epilogue(a[M,K] @ w[N,K]^T + bias). a, w bf16; out bf16 (modes 0-3, 5, 7, 8) or fp32 (mode 4)."""
     _need_cuda(a, w, out, bias, partials)
     if a.dtype != torch.bfloat16 or w.dtype != torch.bfloat16:
         raise ValueError(f"gemm: operands must be bfloat16, got {a.dtype} and {w.dtype}")
@@ -105,6 +105,21 @@ def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: flo
     out = torch.empty(rows, D, device=x.device, dtype=torch.bfloat16)
     lib = L.load()
     L.check(lib.tssp_op_layernorm(L.ptr(x), stride, L.ptr(gamma), L.ptr(beta), L.ptr(out), rows, D, float(eps), L.current_stream()))
+    return out
+
+
+def layernorm_f32(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, out: torch.Tensor | None = None) -> torch.Tensor:
+    """The LayerNorm with fp32 output rows (the pre-norm of CLIP towers); `out` may be `x` itself (in place)."""
+    _need_cuda(x, gamma, beta, out)
+    if x.dtype != torch.float32 or x.stride(1) != 1:
+        raise ValueError("layernorm_f32: x must be float32 with unit stride in the last dimension")
+    D = gamma.numel()
+    out = torch.empty(x.shape[0], D, device=x.device, dtype=torch.float32) if out is None else out
+    if out.dtype != torch.float32 or out.stride(1) != 1:
+        raise ValueError("layernorm_f32: out must be float32 with unit stride in the last dimension")
+    lib = L.load()
+    L.check(lib.tssp_op_layernorm_f32(L.ptr(x), x.stride(0), L.ptr(gamma), L.ptr(beta), L.ptr(out), out.stride(0), x.shape[0], D,
+                                      float(eps), L.current_stream()))
     return out
 
 

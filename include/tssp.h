@@ -111,6 +111,17 @@ typedef struct tssp_layout {
  *   layer_scale = 1:     2 * n_blocks entries, per block LS1 [D] (attention branch; NULL for a block without attention)
  *                        then LS2 [D] (MLP branch). */
 
+/* Model options beyond the token layout, for the timm CLIP image towers (timm vision_transformer.py: VisionTransformer with
+ * pre_norm=True, act_layer='quick_gelu'; OpenAI and LAION ViT-B/32, B/16, L/14, L/14@336 and their fine-tunes). */
+#define TSSP_FFN_GELU 0        /* erf GELU (nn.GELU(), HF "gelu") */
+#define TSSP_FFN_QUICK_GELU 1  /* QuickGELU, x * sigmoid(1.702 x) (timm QuickGELU); needs score_point = 1 */
+typedef struct tssp_model_opts {
+    int32_t pre_norm; /* 1: a LayerNorm (timm norm_pre, eps = ln_eps) over every token after the position embedding and
+                         before block 0; its weight and bias [D] are the last two entries of the weight table */
+    int32_t ffn_act;  /* TSSP_FFN_GELU or TSSP_FFN_QUICK_GELU: the activation between fc1 and fc2 of every block (a
+                         Sequential classification head keeps erf GELU) */
+} tssp_model_opts_t;
+
 int tssp_abi_version(void);
 const char* tssp_last_error(void);
 
@@ -125,6 +136,11 @@ int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, 
 /* The general form: tssp_create is this with the layout {0, 0, 1, 0}, tssp_create_ex with {prefix_tokens == 2, 0, 1, 0}.
  * T = G^2 + 1 + dist_token + register_tokens. Models with register tokens feed the classifier from the CLS row. */
 int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, int device, tssp_handle_t* out);
+/* The most general form: tssp_create_layout is this with the options {0, TSSP_FFN_GELU}. With pre_norm = 1 the weight table
+ * ends with norm_pre weight [D], norm_pre bias [D], after every entry tssp_create_layout's table has. Invalid options are
+ * refused before any device is touched. */
+int tssp_create_model(const tssp_config_t* cfg, const tssp_layout_t* layout, const tssp_model_opts_t* opts, int device,
+                      tssp_handle_t* out);
 int tssp_destroy(tssp_handle_t h);
 /* tssp_destroy parks the engine's device buffers in a per-process pool (exact-size reuse by the next tssp_create; capped
  * by TSSP_POOL_MB, default 16384, 0 = no pool); this returns all parked buffers to the driver. */
@@ -186,7 +202,8 @@ int tssp_ffn_gather_batch(int n_blocks, const float* const* fc1_w, const float* 
 
 /* ---- kernel-level entry points (used by the parity tests and by the engine itself) ---- */
 /* C[M,N] = A[M,K] * W[N,K]^T with a fused epilogue; mode: 0 bf16(acc+bias), 1 bf16 gelu, 2 bf16 gelu + score
- * partials, 3 same with pre-activation scores, 4 fp32 (reduce_add: C += ...). A, W bf16; lda/ldw/ldc in elements.
+ * partials, 3 same with pre-activation scores, 4 fp32 (reduce_add: C += ...), 7 bf16 quickgelu(acc+bias), 8 the same with
+ * pre-activation score partials (those of mode 3 for the same operands). A, W bf16; lda/ldw/ldc in elements.
  * K is a multiple of 8; past K the operands' tiles are zero filled, so any such K works (the padded patch vector). */
 int tssp_op_gemm(int mode, const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K,
                  const float* bias, float* partials, int ldp, int tokens_per_image, int reduce_add, void* stream);
@@ -201,6 +218,10 @@ int tssp_op_score_finish(const float* partials, int ldp, float* norms, int ldn, 
                          float* scores, void* stream);
 int tssp_op_layernorm(const float* x, int64_t in_stride, const float* gamma, const float* beta, void* out_bf16,
                       int rows, int D, float eps, void* stream);
+/* the same LayerNorm with fp32 rows of pitch out_stride (a multiple of 4, >= D); out_f32 may be x (in place). Rounded to
+ * bf16, its output is tssp_op_layernorm's bit for bit. */
+int tssp_op_layernorm_f32(const float* x, int64_t in_stride, const float* gamma, const float* beta, float* out_f32,
+                          int64_t out_stride, int rows, int D, float eps, void* stream);
 /* ctx[n*T, D] = softmax(Q K^T / 8) V per (image, head) from the fused qkv[n*T, 3D]; head_dim 64, 16 <= T <= 1025
  * (up to 208 padded keys one kernel holds a whole key row, beyond that a second one streams keys in tiles of 128). */
 int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream);

@@ -67,6 +67,30 @@ class TsspModelOpts(C.Structure):
     ]
 
 
+# pixel formats of tssp_pixel_input_t.format
+PIXELS_F32, PIXELS_U8 = 0, 1
+TSSP_MAX_PIXEL_CHANNELS = 4
+
+
+class TsspPixelInput(C.Structure):
+    _fields_ = [
+        ("format", C.c_int32),
+        ("rescale", C.c_float),
+        ("mean", C.c_float * TSSP_MAX_PIXEL_CHANNELS),
+        ("std", C.c_float * TSSP_MAX_PIXEL_CHANNELS),
+    ]
+
+
+def pixel_input(fmt: int, mean=(), std=(), rescale: float = 1.0) -> TsspPixelInput:
+    """A tssp_pixel_input_t; mean / std hold one value per channel (at most four), the rest stay 0 / 1."""
+    out = TsspPixelInput()
+    out.format, out.rescale = fmt, rescale
+    for c in range(TSSP_MAX_PIXEL_CHANNELS):
+        out.mean[c] = mean[c] if c < len(mean) else 0.0
+        out.std[c] = std[c] if c < len(std) else 1.0
+    return out
+
+
 class TsspError(RuntimeError):
     """A call into libtssp_b200.so failed; the message comes from tssp_last_error()."""
 
@@ -88,6 +112,7 @@ SIGNATURES = {
     "tssp_load_weights": (_I, [_P, C.POINTER(_P), _I, _P]),
     "tssp_update_ffn": (_I, [_P, _I, _I, _P, _P, _P, _P]),
     "tssp_set_attention": (_I, [_P, C.POINTER(C.c_int32)]),
+    "tssp_set_pixel_input": (_I, [_P, C.POINTER(TsspPixelInput)]),
     "tssp_s1_reset": (_I, [_P, _P]),
     "tssp_s1_batch": (_I, [_P, _P, _I, _I, _P, _P]),
     "tssp_s1_scores": (_I, [_P, _P, _I, _P]),
@@ -108,6 +133,7 @@ SIGNATURES = {
     "tssp_op_attention": (_I, [_P, _P, _I, _I, _I, _I, _P]),
     "tssp_op_im2col": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
     "tssp_op_im2col_ex": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "tssp_op_im2col_u8": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, C.POINTER(TsspPixelInput), _P]),
     "tssp_op_cast_bf16": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P]),
     "tssp_op_argmax_count": (_I, [_P, _I, _I, _I, _P, _P, _P, _P]),
     "tssp_op_stable_rank_f64": (_I, [_P, _I, _I, _I, _P, _P]),

@@ -12,6 +12,7 @@ There is no CPU fallback: a model or device that is not CUDA raises TsspError.
 from __future__ import annotations
 
 import json
+import math
 import os
 import re
 import weakref
@@ -25,7 +26,7 @@ import torch.nn as nn
 from . import _lib as L
 from . import distributed as D
 from . import ops
-from .anatomy import (attention_module, ffn_act_signature, gather_mlp_pairs, get_blocks, get_encoder, has_attention,
+from .anatomy import (attention_module, describe, ffn_act_signature, gather_mlp_pairs, get_blocks, get_encoder, has_attention,
                       install_bypass)
 from .engine import Engine, _cuda_device
 
@@ -36,6 +37,7 @@ __all__ = [
     "save_ffn_importances", "save_ffn_masks", "save_attention_indices", "save_framework_export",
     "load_ffn_mask", "mask_to_importance", "apply_ffn_mask", "attention_removal_counts", "attention_removal_iterative",
     "measure_latency", "engine_for", "release_engine", "trim_pool",
+    "set_pixel_normalization", "clear_pixel_normalization", "normalize_pixels",
 ]
 
 # reference-named helpers (src/vit_pruning.py:28-75)
@@ -84,6 +86,9 @@ def _count_ffn_params_per_block(vit_model) -> List[int]:
 
 # ------------------------------------------------------------------------------------------ engine cache
 _ENGINES: "weakref.WeakKeyDictionary[nn.Module, Dict[str, Any]]" = weakref.WeakKeyDictionary()
+# model -> (mean, std, rescale) registered by set_pixel_normalization; applied to every engine engine_for returns, so an
+# engine rebuilt after a pruning step or a parameter change keeps it
+_PIXEL_NORMS: "weakref.WeakKeyDictionary[nn.Module, tuple]" = weakref.WeakKeyDictionary()
 
 
 def _signature(model) -> tuple:
@@ -110,10 +115,12 @@ def engine_for(model, device="cuda", batch_hint: int = 128, need_cache: bool = F
     if slot is not None:
         eng: Engine = slot["engine"]
         if slot["sig"] == sig and eng.device == dev and (eng.cache_blocks or not need_cache):
+            eng.set_pixel_normalization(_PIXEL_NORMS.get(model))
             return eng
         eng.close()
     cap = min(max(int(batch_hint), 16), 256)
     eng = Engine(model, device=dev, max_images=cap, cache_blocks=need_cache)
+    eng.set_pixel_normalization(_PIXEL_NORMS.get(model))
     _ENGINES[model] = {"engine": eng, "sig": sig}
     return eng
 
@@ -133,6 +140,52 @@ def trim_pool() -> None:
     or reclaim that memory (up to TSSP_POOL_MB, default 16 GB): call this before fine-tuning the pruned model in the
     same process, or when torch reports out-of-memory."""
     L.check(L.load().tssp_trim_pool())
+
+
+def set_pixel_normalization(model, mean: Sequence[float], std: Sequence[float], rescale: float = 1 / 255) -> None:
+    """Let `model`'s batches arrive as uint8 [n, C, H, W] (what JPEG decoders produce) and normalise them on the device:
+    x = (float(u) * rescale - mean[c]) / std[c] in fp32, the per-channel arithmetic of HF image processors and timm
+    transforms. Every result is then bit for bit that of the fp32 batch `normalize_pixels(u, mean, std, rescale)`, and
+    each image crosses PCIe as a quarter of the bytes. fp32 batches are unaffected. Pass the processor's numbers
+    (e.g. image_mean / image_std of an HF processor). Raises ValueError, before any device work, unless there is one
+    finite mean and one finite std > 0 per channel (at most four channels) and rescale is finite."""
+    import ctypes as C
+    channels = describe(model).channels
+    f32 = lambda v: C.c_float(float(v)).value  # noqa: E731  (the values the device computes with)
+    mean = [f32(m) for m in mean]
+    std = [f32(s) for s in std]
+    rescale = f32(rescale)
+    if not 1 <= channels <= L.TSSP_MAX_PIXEL_CHANNELS:
+        raise ValueError(f"uint8 pixel input supports 1 to {L.TSSP_MAX_PIXEL_CHANNELS} channels; the model has {channels}")
+    if len(mean) != channels or len(std) != channels:
+        raise ValueError(f"mean and std need one value per channel ({channels}), got {len(mean)} and {len(std)}")
+    if not all(math.isfinite(v) for v in mean + std + [rescale]):
+        raise ValueError(f"mean, std and rescale must be finite, got mean={mean} std={std} rescale={rescale}")
+    if not all(s > 0 for s in std):
+        raise ValueError(f"std must be > 0 in every channel, got {std}")
+    _PIXEL_NORMS[model] = (tuple(mean), tuple(std), rescale)
+    slot = _ENGINES.get(model)
+    if slot is not None:
+        slot["engine"].set_pixel_normalization(_PIXEL_NORMS[model])
+
+
+def clear_pixel_normalization(model) -> None:
+    """Undo set_pixel_normalization: uint8 batches of `model` are converted with .float() again, without normalisation."""
+    _PIXEL_NORMS.pop(model, None)
+    slot = _ENGINES.get(model)
+    if slot is not None:
+        slot["engine"].set_pixel_normalization(None)
+
+
+def normalize_pixels(pixels: torch.Tensor, mean: Sequence[float], std: Sequence[float], rescale: float = 1 / 255) -> torch.Tensor:
+    """The fp32 image a uint8 batch [n, C, H, W] stands for under set_pixel_normalization:
+    (u.float() * rescale - mean[c]) / std[c], each operation in fp32, on the batch's device."""
+    C = pixels.shape[1]
+    dev = pixels.device
+    r = torch.tensor(float(rescale), dtype=torch.float32, device=dev)
+    m = torch.tensor([float(v) for v in mean], dtype=torch.float32, device=dev).view(1, C, 1, 1)
+    s = torch.tensor([float(v) for v in std], dtype=torch.float32, device=dev).view(1, C, 1, 1)
+    return (pixels.float() * r - m) / s
 
 
 def _engine_in_step(model):

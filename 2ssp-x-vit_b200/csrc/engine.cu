@@ -426,6 +426,48 @@ static int op_im2col(const float* pixels, void* out, int n, int C, int H, int W,
     return 0;
 }
 
+// The normalisation of uint8 pixels (TSSP_PIXELS_U8) for a model with C channels: refused unless it can be applied.
+static int check_pixel_norm(const tssp_pixel_input_t& in, int C, const char* where) {
+    if (C < 1 || C > TSSP_MAX_PIXEL_CHANNELS)
+        return fail("%s: uint8 pixels need 1 to %d channels, got C=%d", where, TSSP_MAX_PIXEL_CHANNELS, C);
+    if (!std::isfinite(in.rescale)) return fail("%s: rescale=%g is not finite", where, in.rescale);
+    for (int c = 0; c < C; ++c) {
+        if (!std::isfinite(in.mean[c])) return fail("%s: mean[%d]=%g is not finite", where, c, in.mean[c]);
+        if (!std::isfinite(in.std[c]) || !(in.std[c] > 0.0f)) return fail("%s: std[%d]=%g must be finite and > 0", where, c, in.std[c]);
+    }
+    return 0;
+}
+
+// im2col of uint8 pixels, normalised per channel on the way in (kernels.cuh: the fp32 kernels' bits for the normalised image)
+static int op_im2col_u8(const uint8_t* pixels, void* out, int n, int C, int H, int W, int P, const tssp_pixel_input_t& norm,
+                        cudaStream_t s, int prefix) {
+    if (P < 1 || H % P || W % P || H != W) return fail("im2col: H=%d W=%d P=%d unsupported (square images, P dividing them)", H, W, P);
+    if (prefix < 1 || prefix > TSSP_MAX_PREFIX) return fail("im2col: prefix=%d must be in [1,%d]", prefix, TSSP_MAX_PREFIX);
+    TSSP_TRY(check_pixel_norm(norm, C, "im2col (uint8 pixels)"));
+    const uintptr_t align = (P & 7) == 0 ? 8 : ((P & 1) == 0 ? 2 : 1);  // the 8-byte / 2-byte loads of the two kernels
+    if (reinterpret_cast<uintptr_t>(pixels) % align != 0)
+        return fail("im2col (uint8 pixels): pointer %p is not %d-byte aligned, as the loads at P=%d need", static_cast<const void*>(pixels),
+                    static_cast<int>(align), P);
+    PixelNorm pn;
+    pn.rescale = norm.rescale;
+    for (int c = 0; c < 4; ++c) {
+        pn.mean[c] = c < C ? norm.mean[c] : 0.0f;
+        pn.std[c] = c < C ? norm.std[c] : 1.0f;
+    }
+    const int T = (H / P) * (W / P) + prefix;
+    const int ld = patch_width(C, P);
+    const long long total = static_cast<long long>(n) * T * (ld / 8);
+    if ((P & 7) == 0) {
+        im2col_patches_u8_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T, prefix, pn);
+        TSSP_LAUNCH_CHECK("im2col_patches_u8_kernel");
+    } else {
+        im2col_patches_padded_u8_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T,
+                                                                             prefix, ld, pn);
+        TSSP_LAUNCH_CHECK("im2col_patches_padded_u8_kernel");
+    }
+    return 0;
+}
+
 // out: bf16 rows of pitch D, or (f32_out) fp32 rows of pitch out_stride; an fp32 out may be x itself
 static int op_layernorm_any(const float* x, long long in_stride, const float* g, const float* b, void* out, bool f32_out,
                             long long out_stride, int rows, int D, float eps, cudaStream_t s, bool stream_in) {
@@ -639,7 +681,8 @@ struct tssp_engine {
     float *norm_pre_w, *norm_pre_b;  // opts.pre_norm: LayerNorm over every token before block 0, else nullptr
     int Cp, Hhp;  // padded classes / head hidden
     // workspace
-    float* pixels[2];          // double-buffered staging of host pixel batches
+    float* pixels[2];          // double-buffered staging of host pixel batches (fp32-sized: a uint8 batch fits too)
+    tssp_pixel_input_t pix;    // format of the pixels the batch entry points are handed (tssp_set_pixel_input)
     long long* labels[2];      // ... and of their labels (same slot, same copy stream)
     long long* labels_dev;     // device-resident labels are copied here on the caller's stream: captured chains then only
                                // ever reference engine-owned label buffers (a fresh tensor per batch would force a re-capture)
@@ -863,6 +906,7 @@ static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, 
         return rc;
     }
     e->next_slot = 0;
+    e->pix = tssp_pixel_input_t{TSSP_PIXELS_F32, 1.0f, {0.0f, 0.0f, 0.0f, 0.0f}, {1.0f, 1.0f, 1.0f, 1.0f}};
     e->staged_slot = -1;
     e->host_slot = -1;
     e->s1_fresh = false;
@@ -1029,7 +1073,9 @@ static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cud
 // `bounds` (optional): up to three ascending image counts 0 < b0 < b1 < b2 < n; the pixels are copied as n_bounds + 1
 // consecutive parts, ev_part[i] fires when the images below bounds[i] have landed, and only the FIRST part is waited
 // for on `s` here -- the caller waits for the others as it reaches them.
-static int stage_batch(tssp_engine* e, const float* pixels, const int64_t* labels, int n, int on_host, const float** dev_pixels,
+static size_t pixel_bytes(const tssp_engine* e) { return e->pix.format == TSSP_PIXELS_U8 ? 1 : sizeof(float); }
+
+static int stage_batch(tssp_engine* e, const void* pixels, const int64_t* labels, int n, int on_host, const void** dev_pixels,
                        const long long** dev_labels, cudaStream_t s, const int* bounds = nullptr, int n_bounds = 0, int* slot_out = nullptr) {
     if (n < 1 || n > e->cfg.max_images) return fail("batch of %d images outside [1, max_images=%d]", n, e->cfg.max_images);
     if (!e->weights_loaded) return fail("weights have not been loaded");
@@ -1045,7 +1091,7 @@ static int stage_batch(tssp_engine* e, const float* pixels, const int64_t* label
         }
         return 0;
     }
-    const size_t bytes = static_cast<size_t>(n) * e->cfg.channels * e->cfg.image_size * e->cfg.image_size * sizeof(float);
+    const size_t bytes = static_cast<size_t>(n) * e->cfg.channels * e->cfg.image_size * e->cfg.image_size * pixel_bytes(e);
     const int slot = e->next_slot;
     e->next_slot ^= 1;
     e->host_slot = slot;  // from here on the caller's buffers are in use until finish_host_batch()
@@ -1164,9 +1210,14 @@ static unsigned long long block_mask(const int32_t* flags, int B) {
 // ---- launch sequences ----------------------------------------------------------------------------
 // patch extraction (HF ViTPatchEmbeddings as a GEMM over non-overlapping patches): the one kernel that reads the
 // caller's / the staged pixels, kept outside the captured chains so that those do not depend on where a batch lives
-static int run_im2col(tssp_engine* e, const float* dev_pixels, int n, cudaStream_t s) {
+static int run_im2col(tssp_engine* e, const void* dev_pixels, int n, cudaStream_t s) {
     const tssp_config_t& c = e->cfg;
-    TSSP_PROF(KC_MISC, s, op_im2col(dev_pixels, e->patchA, n, c.channels, c.image_size, c.image_size, c.patch_size, s, e->prefix));
+    if (e->pix.format == TSSP_PIXELS_U8)
+        TSSP_PROF(KC_MISC, s, op_im2col_u8(static_cast<const uint8_t*>(dev_pixels), e->patchA, n, c.channels, c.image_size, c.image_size,
+                                           c.patch_size, e->pix, s, e->prefix));
+    else
+        TSSP_PROF(KC_MISC, s, op_im2col(static_cast<const float*>(dev_pixels), e->patchA, n, c.channels, c.image_size, c.image_size,
+                                        c.patch_size, s, e->prefix));
     if (e->staged_slot >= 0) {  // the host-staged pixel buffer may be refilled once im2col has read it
         TSSP_CUDA(cudaEventRecord(e->ev_consumed[e->staged_slot], s));
         e->staged_slot = -1;
@@ -1464,6 +1515,16 @@ int tssp_set_attention(tssp_handle_t h, const int32_t* present) {
     return 0;
 }
 
+int tssp_set_pixel_input(tssp_handle_t h, const tssp_pixel_input_t* input) {
+    TSSP_ENGINE_ENTRY(h, "tssp_set_pixel_input");
+    if (input == nullptr) return fail("tssp_set_pixel_input: NULL argument");
+    if (input->format != TSSP_PIXELS_F32 && input->format != TSSP_PIXELS_U8)
+        return fail("tssp_set_pixel_input: format=%d must be %d (fp32) or %d (uint8)", input->format, TSSP_PIXELS_F32, TSSP_PIXELS_U8);
+    if (input->format == TSSP_PIXELS_U8) TSSP_TRY(check_pixel_norm(*input, h->cfg.channels, "tssp_set_pixel_input"));
+    h->pix = *input;
+    return 0;
+}
+
 int tssp_s1_reset(tssp_handle_t h, void* stream) {
     TSSP_ENGINE_ENTRY(h, "tssp_s1_reset");
     TSSP_CUDA(cudaMemsetAsync(h->scores, 0, sizeof(float) * h->ldn, static_cast<cudaStream_t>(stream)));
@@ -1473,7 +1534,7 @@ int tssp_s1_reset(tssp_handle_t h, void* stream) {
 
 // Stage-1 forward of n device-resident images: patch extraction, then ONE captured chain (embeddings, the blocks up
 // to the last fc1, score finisher)
-static int s1_sweep(tssp_engine* h, const float* px, int n, float* img_norms, cudaStream_t s) {
+static int s1_sweep(tssp_engine* h, const void* px, int n, float* img_norms, cudaStream_t s) {
     TSSP_TRY(run_im2col(h, px, n, s));
     const GraphKey key{GK_S1, n, h->cfg.score_point, 0ull, nullptr, nullptr};
     TSSP_TRY(run_graphed(h, key, s, [&](cudaStream_t gs) -> int {
@@ -1511,7 +1572,7 @@ static int s1_split_bounds(const tssp_engine* h, int n, int* bounds) {
 }
 
 static int s1_batch(tssp_engine* h, const float* pixels, int n, int pixels_on_host, float* img_norms, cudaStream_t s) {
-    const float* px = nullptr;
+    const void* px = nullptr;
     const bool fresh = h->s1_fresh;
     h->s1_fresh = false;
     int bounds[3];
@@ -1519,13 +1580,13 @@ static int s1_batch(tssp_engine* h, const float* pixels, int n, int pixels_on_ho
     if (nb > 0) {
         int slot = -1;
         TSSP_TRY(stage_batch(h, pixels, nullptr, n, 1, &px, nullptr, s, bounds, nb, &slot));
-        const size_t img_elems = static_cast<size_t>(h->cfg.channels) * h->cfg.image_size * h->cfg.image_size;
+        const size_t img_bytes = static_cast<size_t>(h->cfg.channels) * h->cfg.image_size * h->cfg.image_size * pixel_bytes(h);
         int begin = 0;
         for (int i = 0; i <= nb; ++i) {
             const int end = i < nb ? bounds[i] : n;
             if (i > 0) TSSP_CUDA(cudaStreamWaitEvent(s, i < nb ? h->ev_part[i] : h->ev_copied[slot], 0));
             h->staged_slot = (i == nb) ? slot : -1;  // the staging buffer is released by the last sub-batch
-            TSSP_TRY(s1_sweep(h, px + img_elems * begin, end - begin,
+            TSSP_TRY(s1_sweep(h, static_cast<const char*>(px) + img_bytes * begin, end - begin,
                               img_norms != nullptr ? img_norms + static_cast<size_t>(begin) * h->sumF : nullptr, s));
             begin = end;
         }
@@ -1562,7 +1623,7 @@ int tssp_s1_scores(tssp_handle_t h, float* scores, int out_on_host, void* stream
 
 static int forward_logits(tssp_engine* h, const float* pixels, int n, int pixels_on_host, const int32_t* skip_attn,
                           float* logits, int out_on_host, cudaStream_t s) {
-    const float* px = nullptr;
+    const void* px = nullptr;
     TSSP_TRY(stage_batch(h, pixels, nullptr, n, pixels_on_host, &px, nullptr, s));
     TSSP_TRY(run_im2col(h, px, n, s));
     const GraphKey key{GK_FORWARD, n, 0, block_mask(skip_attn, h->cfg.n_blocks), nullptr, nullptr};
@@ -1585,7 +1646,7 @@ int tssp_forward_logits(tssp_handle_t h, const float* pixels, int n, int pixels_
 
 static int eval_batch(tssp_engine* h, const float* pixels, const int64_t* labels, int n, int on_host, const int32_t* skip_attn,
                       unsigned long long* correct_dev, cudaStream_t s) {
-    const float* px = nullptr;
+    const void* px = nullptr;
     const long long* lb = nullptr;
     TSSP_TRY(stage_batch(h, pixels, labels, n, on_host, &px, &lb, s));
     TSSP_TRY(run_im2col(h, px, n, s));
@@ -1614,7 +1675,7 @@ static int s2_batch(tssp_engine* h, const float* pixels, const int64_t* labels, 
                     int run_baseline, cudaStream_t s) {
     if (!h->cfg.cache_blocks) return fail("tssp_s2_batch: engine was created without cache_blocks");
     const int B = h->cfg.n_blocks;
-    const float* px = nullptr;
+    const void* px = nullptr;
     const long long* lb = nullptr;
     TSSP_TRY(stage_batch(h, pixels, labels, n, on_host, &px, &lb, s));
     TSSP_TRY(run_im2col(h, px, n, s));
@@ -1787,6 +1848,12 @@ int tssp_op_im2col_ex(const float* pixels, void* out_bf16, int n_img, int C, int
     TSSP_ENTRY();
     if (pixels == nullptr || out_bf16 == nullptr) return fail("tssp_op_im2col: NULL argument");
     return op_im2col(pixels, out_bf16, n_img, C, H, W, P, static_cast<cudaStream_t>(stream), prefix_tokens);
+}
+int tssp_op_im2col_u8(const uint8_t* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens,
+                      const tssp_pixel_input_t* norm, void* stream) {
+    TSSP_ENTRY();
+    if (pixels == nullptr || out_bf16 == nullptr || norm == nullptr) return fail("tssp_op_im2col_u8: NULL argument");
+    return op_im2col_u8(pixels, out_bf16, n_img, C, H, W, P, *norm, static_cast<cudaStream_t>(stream), prefix_tokens);
 }
 int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream) {
     return tssp_op_im2col_ex(pixels, out_bf16, n_img, C, H, W, P, 1, stream);

@@ -117,6 +117,127 @@ __global__ void im2col_patches_padded_kernel(const float* __restrict__ pixels, _
     }
 }
 
+// uint8 pixels [n, C, H, W] (C <= 4) normalised on the way in: x = (float(u) * rescale - mean[c]) / std[c], each step one
+// IEEE fp32 operation (no FMA contraction, correctly rounded division), so the bf16 written is the one the fp32 kernels
+// above write for the fp32 image (u.float() * rescale - mean) / std computed by torch.
+struct PixelNorm {
+    float rescale;
+    float mean[4];
+    float std[4];
+};
+
+__device__ __forceinline__ float normalize_u8(uint32_t u, float rescale, float mean, float std) {
+    return __fdiv_rn(__fsub_rn(__fmul_rn(static_cast<float>(u), rescale), mean), std);
+}
+
+// v[c] with constant indices only: a runtime index into a kernel parameter would copy the struct to local memory.
+__device__ __forceinline__ float pick4(const float (&v)[4], int c) { return c == 0 ? v[0] : c == 1 ? v[1] : c == 2 ? v[2] : v[3]; }
+
+// The bf16 a pixel becomes depends only on (channel, byte): every block first fills a table of those C * 256 values in
+// shared memory, then looks pixels up. One correctly rounded division per pixel made the kernel issue-bound, slower than
+// the fp32 kernel it replaces. Every thread of the block reaches the barrier (the kernels do not return early).
+__device__ __forceinline__ void fill_u8_table(uint16_t (&lut)[4][256], const PixelNorm& norm, int C) {
+    for (int j = threadIdx.x; j < C * 256; j += blockDim.x) {
+        const int c = j >> 8;
+        const float x = normalize_u8(static_cast<uint32_t>(j & 255), norm.rescale, pick4(norm.mean, c), pick4(norm.std, c));
+        lut[c][j & 255] = __bfloat16_as_ushort(__float2bfloat16_rn(x));
+    }
+    __syncthreads();
+}
+
+// Two table entries as one bf16x2 word, the first in the low half (as __floats2bfloat162_rn packs them).
+__device__ __forceinline__ uint32_t pack2(uint16_t lo, uint16_t hi) { return static_cast<uint32_t>(lo) | (static_cast<uint32_t>(hi) << 16); }
+
+// im2col_patches_kernel for uint8 pixels (P a multiple of 8): each thread's 8 columns are one 8-byte load.
+__global__ void im2col_patches_u8_kernel(const uint8_t* __restrict__ pixels, __nv_bfloat16* __restrict__ out, int n_img,
+                                         int C, int H, int W, int P, int T, int prefix, const PixelNorm norm) {
+    __shared__ uint16_t lut[4][256];
+    fill_u8_table(lut, norm, C);
+    const int G = W / P;
+    const int Kp = C * P * P;
+    const int k8_per_row = Kp / 8;
+    const long long total = static_cast<long long>(n_img) * T * k8_per_row;
+    for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+         i += static_cast<long long>(gridDim.x) * blockDim.x) {
+        const int k8 = static_cast<int>(i % k8_per_row);
+        const long long row = i / k8_per_row;
+        const int t = static_cast<int>(row % T);
+        const int img = static_cast<int>(row / T);
+        uint4 packed = make_uint4(0u, 0u, 0u, 0u);
+        if (t >= prefix) {
+            const int patch = t - prefix;
+            const int py = patch / G, px = patch % G;
+            const int k = k8 * 8;
+            const int c = k / (P * P);
+            const int ky = (k / P) % P;
+            const int kx = k % P;
+            const uint8_t* src = pixels + ((static_cast<size_t>(img) * C + c) * H + (py * P + ky)) * W + px * P + kx;
+            const uint2 raw = __ldg(reinterpret_cast<const uint2*>(src));
+            const uint16_t* tc = lut[c];
+            packed.x = pack2(tc[raw.x & 0xffu], tc[(raw.x >> 8) & 0xffu]);
+            packed.y = pack2(tc[(raw.x >> 16) & 0xffu], tc[raw.x >> 24]);
+            packed.z = pack2(tc[raw.y & 0xffu], tc[(raw.y >> 8) & 0xffu]);
+            packed.w = pack2(tc[(raw.y >> 16) & 0xffu], tc[raw.y >> 24]);
+        }
+        *reinterpret_cast<uint4*>(out + static_cast<size_t>(row) * Kp + k8 * 8) = packed;
+    }
+}
+
+// im2col_patches_padded_kernel for uint8 pixels: with P even a column pair is one 2-byte load inside one channel (C*P*P
+// and P*P are even), with P odd two byte loads, each looked up in its own channel's table.
+__global__ void im2col_patches_padded_u8_kernel(const uint8_t* __restrict__ pixels, __nv_bfloat16* __restrict__ out, int n_img,
+                                                int C, int H, int W, int P, int T, int prefix, int ld, const PixelNorm norm) {
+    __shared__ uint16_t lut[4][256];
+    fill_u8_table(lut, norm, C);
+    const int G = W / P;
+    const int PP = P * P;
+    const int K = C * PP;
+    const int k8_per_row = ld / 8;
+    const long long total = static_cast<long long>(n_img) * T * k8_per_row;
+    for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+         i += static_cast<long long>(gridDim.x) * blockDim.x) {
+        const int k8 = static_cast<int>(i % k8_per_row);
+        const long long row = i / k8_per_row;
+        const int t = static_cast<int>(row % T);
+        const int img = static_cast<int>(row / T);
+        uint32_t w[4] = {0u, 0u, 0u, 0u};
+        if (t >= prefix) {
+            const int patch = t - prefix;
+            const int py = patch / G, px = patch % G;
+            const uint8_t* base = pixels + static_cast<size_t>(img) * C * H * W + static_cast<size_t>(py * P) * W + px * P;
+            auto at = [&](int k, int& c) {
+                c = k / PP;
+                const int r = k - c * PP, ky = r / P, kx = r - ky * P;
+                return base + (static_cast<size_t>(c) * H + ky) * W + kx;
+            };
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int k = k8 * 8 + 2 * q;
+                uint16_t v0 = 0, v1 = 0;  // bf16 +0
+                int c0 = 0, c1 = 0;
+                if ((P & 1) == 0) {
+                    if (k < K) {  // K even: k + 1 < K as well
+                        const uint32_t pair = __ldg(reinterpret_cast<const unsigned short*>(at(k, c0)));
+                        v0 = lut[c0][pair & 0xffu];
+                        v1 = lut[c0][pair >> 8];
+                    }
+                } else {
+                    if (k < K) {
+                        const uint8_t* p0 = at(k, c0);
+                        v0 = lut[c0][__ldg(p0)];
+                    }
+                    if (k + 1 < K) {
+                        const uint8_t* p1 = at(k + 1, c1);
+                        v1 = lut[c1][__ldg(p1)];
+                    }
+                }
+                w[q] = pack2(v0, v1);
+            }
+        }
+        *reinterpret_cast<uint4*>(out + static_cast<size_t>(row) * ld + k8 * 8) = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+}
+
 // x[img*T + t, :] = table[t, :]   (table = position embeddings with the CLS token / conv bias folded in)
 __global__ void broadcast_rows_kernel(const float* __restrict__ table, float* __restrict__ x, int n_img, int T, int D) {
     const int d4 = D / 4;

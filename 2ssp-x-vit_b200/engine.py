@@ -57,6 +57,8 @@ class Engine:
             else:
                 L.check(self.lib.tssp_create_layout(C.byref(cfg), C.byref(layout), self.device.index, C.byref(self._handle)))
         self.ffn_dims = list(a.ffn_dims)
+        self.pixel_norm = None                # (mean, std, rescale): see set_pixel_normalization
+        self._pixel_format = (L.PIXELS_F32, None)  # what the library engine reads its `pixels` pointers as
         self.load_weights(a)
         self.anatomy.globals_.clear()
         self.anatomy.blocks.clear()  # do not keep parameter references alive
@@ -100,9 +102,25 @@ class Engine:
         arr = (C.c_int32 * len(present))(*[1 if p else 0 for p in present])
         L.check(self.lib.tssp_set_attention(self._handle, arr))
 
+    def set_pixel_normalization(self, norm) -> None:
+        """norm = (mean, std, rescale), one mean and std per channel: uint8 batches are then sent as bytes and normalised on
+        the device, (float(u) * rescale - mean[c]) / std[c] in fp32. None: uint8 batches are converted with .float() on the
+        host and not normalised. fp32 batches are fed as they are either way."""
+        self.pixel_norm = None if norm is None else (tuple(float(m) for m in norm[0]), tuple(float(s) for s in norm[1]), float(norm[2]))
+
+    def _use_format(self, u8: bool) -> None:
+        want = (L.PIXELS_U8, self.pixel_norm) if u8 else (L.PIXELS_F32, None)
+        if want != self._pixel_format:
+            mean, std, rescale = self.pixel_norm if u8 else ((), (), 1.0)
+            L.check(self.lib.tssp_set_pixel_input(self._handle, C.byref(L.pixel_input(want[0], mean, std, rescale))))
+            self._pixel_format = want
+
     # ------------------------------------------------------------------ batches
     def _pixels(self, px: torch.Tensor) -> torch.Tensor:
-        if px.dtype != torch.float32:
+        """The batch as the engine reads it; also sets the engine's pixel format for it (uint8 stays uint8 only with a
+        normalisation set)."""
+        u8 = px.dtype == torch.uint8 and self.pixel_norm is not None
+        if px.dtype != torch.float32 and not u8:
             px = px.float()
         a = self.anatomy
         if px.dim() != 4 or px.shape[1] != a.channels or px.shape[2] != a.image_size or px.shape[3] != a.image_size:
@@ -110,6 +128,7 @@ class Engine:
                              f"([n,{a.channels},{a.image_size},{a.image_size}])")
         if px.is_cuda and px.device != self.device:
             px = px.to(self.device)
+        self._use_format(u8)
         return px.contiguous()
 
     def _chunks(self, n: int):

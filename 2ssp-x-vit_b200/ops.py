@@ -134,17 +134,26 @@ def attention(qkv: torch.Tensor, n_img: int, T: int, heads: int) -> torch.Tensor
     return ctx
 
 
-def im2col(pixels: torch.Tensor, patch: int, prefix: int = 1) -> torch.Tensor:
+def im2col(pixels: torch.Tensor, patch: int, prefix: int = 1, *, mean=None, std=None, rescale: float = 1 / 255) -> torch.Tensor:
     """[n * T, Kp] bf16 patch rows, `prefix` zero rows ahead of every image's patches (2 for DeiT, 1 + R with R register
-    tokens); Kp = C*P*P rounded up to a multiple of 8, the columns past C*P*P zero (P = 14: 588 -> 592)."""
+    tokens); Kp = C*P*P rounded up to a multiple of 8, the columns past C*P*P zero (P = 14: 588 -> 592).
+    uint8 pixels (C <= 4) need `mean` and `std` per channel and are normalised in the kernel, (float(u) * rescale -
+    mean[c]) / std[c] in fp32: the bits of the fp32 form on api.normalize_pixels(pixels, mean, std, rescale)."""
     _need_cuda(pixels)
-    if pixels.dtype != torch.float32 or not pixels.is_contiguous():
-        raise ValueError("im2col: pixels must be a contiguous float32 tensor [n, C, H, W]")
+    u8 = pixels.dtype == torch.uint8
+    if not (u8 or pixels.dtype == torch.float32) or not pixels.is_contiguous():
+        raise ValueError("im2col: pixels must be a contiguous float32 or uint8 tensor [n, C, H, W]")
+    if u8 and (mean is None or std is None):
+        raise ValueError("im2col: uint8 pixels need the per-channel mean and std they are normalised with")
     n, c, h, w = pixels.shape
     T = (h // patch) * (w // patch) + prefix
     out = torch.empty(n * T, (c * patch * patch + 7) // 8 * 8, device=pixels.device, dtype=torch.bfloat16)
     lib = L.load()
-    L.check(lib.tssp_op_im2col_ex(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, L.current_stream()))
+    if u8:
+        norm = L.pixel_input(L.PIXELS_U8, [float(v) for v in mean], [float(v) for v in std], float(rescale))
+        L.check(lib.tssp_op_im2col_u8(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, norm, L.current_stream()))
+    else:
+        L.check(lib.tssp_op_im2col_ex(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, L.current_stream()))
     return out
 
 

@@ -141,6 +141,27 @@ int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, in
  * refused before any device is touched. */
 int tssp_create_model(const tssp_config_t* cfg, const tssp_layout_t* layout, const tssp_model_opts_t* opts, int device,
                       tssp_handle_t* out);
+
+/* Pixel input format of an engine's batch entry points (tssp_s1_batch, tssp_forward_logits, tssp_eval_batch,
+ * tssp_s2_batch). TSSP_PIXELS_F32 (the default): `pixels` is fp32 [n, C, H, W], fed to the patch embedding as it is.
+ * TSSP_PIXELS_U8: `pixels` is uint8 [n, C, H, W] (the bytes a JPEG decoder produces; C <= 4), read through the same
+ * `const float*` parameter, and every pixel is normalised on the device as x = (float(u) * rescale - mean[c]) / std[c]
+ * in IEEE fp32, one rounding per operation: the bits of the fp32 batch normalised that way on the host, at a quarter of
+ * the host-to-device bytes. A device-resident uint8 batch must be 8-byte aligned when the patch size is a multiple of
+ * 8, 2-byte aligned when it is even. Host uint8 batches follow the same lifetime rule as fp32 ones. */
+#define TSSP_PIXELS_F32 0
+#define TSSP_PIXELS_U8 1
+#define TSSP_MAX_PIXEL_CHANNELS 4
+typedef struct tssp_pixel_input {
+    int32_t format; /* TSSP_PIXELS_F32 or TSSP_PIXELS_U8 */
+    float rescale;  /* U8: multiplies every byte first (1/255 for the usual [0, 1] scaling) */
+    float mean[TSSP_MAX_PIXEL_CHANNELS]; /* U8: per channel, entries past the model's channels are ignored */
+    float std[TSSP_MAX_PIXEL_CHANNELS];  /* U8: per channel, > 0 */
+} tssp_pixel_input_t;
+/* Sets the format of the following batches. Under U8 the values must be finite, std > 0 and the model's channels in
+ * [1, 4]; an invalid input is refused and the engine keeps its previous format. Needs no new device memory (a uint8 batch
+ * is staged in the fp32 slots) and no new graph captures (the patch extraction runs outside the captured chains). */
+int tssp_set_pixel_input(tssp_handle_t h, const tssp_pixel_input_t* input);
 int tssp_destroy(tssp_handle_t h);
 /* tssp_destroy parks the engine's device buffers in a per-process pool (exact-size reuse by the next tssp_create; capped
  * by TSSP_POOL_MB, default 16384, 0 = no pool); this returns all parked buffers to the driver. */
@@ -160,12 +181,14 @@ int tssp_set_attention(tssp_handle_t h, const int32_t* present);
 int tssp_s1_reset(tssp_handle_t h, void* stream);
 /* img_norms (optional, device, [n][sum_b F_b] fp32): per-image norms of this batch, for GPU-count-invariant
  * reductions across data-parallel ranks. */
+/* pixels: fp32 [n, C, H, W], or uint8 under TSSP_PIXELS_U8 (tssp_set_pixel_input) */
 int tssp_s1_batch(tssp_handle_t h, const float* pixels, int n, int pixels_on_host, float* img_norms, void* stream);
 /* scores: [sum_b F_b] fp32, blocks concatenated. Synchronises `stream` when out_on_host. */
 int tssp_s1_scores(tssp_handle_t h, float* scores, int out_on_host, void* stream);
 
 /* ---- forward / top-1 -- replaces the forward + argmax/compare of evaluate_top1 (src/vit_pruning.py:325-373).
- *      skip_attn (optional, [B]): 1 = evaluate with that block's attention removed (zero bypass). */
+ *      skip_attn (optional, [B]): 1 = evaluate with that block's attention removed (zero bypass).
+ *      pixels: fp32 [n, C, H, W], or uint8 under TSSP_PIXELS_U8 (tssp_set_pixel_input), here and in tssp_eval_batch. */
 int tssp_forward_logits(tssp_handle_t h, const float* pixels, int n, int pixels_on_host, const int32_t* skip_attn,
                         float* logits, int out_on_host, void* stream);
 /* adds the number of correct top-1 predictions of this batch to *correct (device uint64). */
@@ -181,7 +204,8 @@ int tssp_eval_batch(tssp_handle_t h, const float* pixels, const int64_t* labels,
  *      across ranks); run_baseline is a set of flags: TSSP_S2_COUNT_BASELINE (1) adds the baseline pass to counts[0]
  *      (0 leaves counts[0] untouched; the cache pass still runs), TSSP_S2_WITH_SCORES (2) makes the baseline pass also
  *      accumulate the Stage-1 score sums of the batch exactly as tssp_s1_batch would (call tssp_s1_reset first, read
- *      them with tssp_s1_scores): fit() of mask_conjunction.py:359-362 runs both passes over the same images. */
+ *      them with tssp_s1_scores): fit() of mask_conjunction.py:359-362 runs both passes over the same images.
+ *      pixels: fp32 [n, C, H, W], or uint8 under TSSP_PIXELS_U8 (tssp_set_pixel_input). */
 #define TSSP_S2_COUNT_BASELINE 1
 #define TSSP_S2_WITH_SCORES 2
 int tssp_s2_reset(tssp_handle_t h, void* stream);
@@ -229,6 +253,11 @@ int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H,
 /* out[n * T, Kp] with T = (H/P)^2 + prefix_tokens and Kp = round_up(C*P*P, 8): prefix_tokens (1..8) zero rows ahead of
  * every image's patches, columns past C*P*P zero (the padded patch vector of patch sizes that are not a multiple of 8) */
 int tssp_op_im2col_ex(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens, void* stream);
+/* the same from uint8 pixels [n_img, C, H, W], C in [1, 4], normalised as under TSSP_PIXELS_U8 with norm's rescale, mean
+ * and std (its format is ignored): bit for bit tssp_op_im2col_ex of the fp32 image (float(u) * rescale - mean) / std.
+ * pixels must be 8-byte aligned when P is a multiple of 8, 2-byte aligned when P is even. */
+int tssp_op_im2col_u8(const uint8_t* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens,
+                      const tssp_pixel_input_t* norm, void* stream);
 int tssp_op_cast_bf16(const float* in, int rows, int cols, int ld_in, void* out_bf16, int rows_pad, int cols_pad,
                       int ld_out, void* stream);
 int tssp_op_argmax_count(const float* logits, int ld, int n, int C, const int64_t* labels, int32_t* preds,

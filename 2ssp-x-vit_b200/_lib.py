@@ -10,22 +10,22 @@ import os
 from pathlib import Path
 
 TSSP_MAX_BLOCKS = 64
-TSSP_ABI_VERSION = 1
+TSSP_ABI_VERSION = 2
 
 _PKG_DIR = Path(__file__).resolve().parent
 LIB_PATH = _PKG_DIR / "lib" / "libtssp_b200.so"
 
 # weight table layout (include/tssp.h: enum tssp_weight_index / tssp_block_weight_index)
-W_PATCH_W, W_PATCH_B, W_CLS, W_POS, W_FINAL_LN_W, W_FINAL_LN_B, W_HEAD0_W, W_HEAD_W, W_HEAD_B, W_GLOBAL_COUNT = range(10)
+(W_PATCH_W, W_PATCH_B, W_CLS, W_POS, W_FINAL_LN_W, W_FINAL_LN_B, W_HEAD0_W, W_HEAD_W, W_HEAD_B,
+ W_DIST_TOKEN, W_HEAD_DIST_W, W_HEAD_DIST_B, W_REG_TOKENS, W_NORM_PRE_W, W_NORM_PRE_B, W_GLOBAL_COUNT) = range(16)
 (BW_LN1_W, BW_LN1_B, BW_Q_W, BW_Q_B, BW_K_W, BW_K_B, BW_V_W, BW_V_B, BW_PROJ_W, BW_PROJ_B,
- BW_LN2_W, BW_LN2_B, BW_FC1_W, BW_FC1_B, BW_FC2_W, BW_FC2_B, BW_COUNT) = range(17)
-WX_DIST_TOKEN, WX_HEAD_DIST_W, WX_HEAD_DIST_B, WX_COUNT = range(4)  # engines with two prefix tokens (tssp_create_ex)
+ BW_LN2_W, BW_LN2_B, BW_FC1_W, BW_FC1_B, BW_FC2_W, BW_FC2_B, BW_LS1, BW_LS2, BW_COUNT) = range(19)
 TSSP_MAX_REGISTER_TOKENS = 7
 
 # GEMM epilogue modes (csrc/gemm_tcgen05.cuh: enum GemmMode)
 (EPI_BF16, EPI_BF16_GELU, EPI_BF16_GELU_SCORE, EPI_BF16_GELU_SCORE_PRE, EPI_F32, EPI_BF16_ROWNORM, EPI_F32_SCALED,
  EPI_BF16_QGELU, EPI_BF16_QGELU_SCORE_PRE) = range(9)
-# MLP activations of tssp_model_opts_t.ffn_act
+# MLP activations of tssp_config_t.ffn_act
 FFN_ACTS = {"gelu": 0, "quick_gelu": 1}
 
 
@@ -46,24 +46,14 @@ class TsspConfig(C.Structure):
         ("score_point", C.c_int32),
         ("cache_blocks", C.c_int32),
         ("ln_eps", C.c_float),
-        ("ffn_dims", C.c_int32 * TSSP_MAX_BLOCKS),
-        ("attn_present", C.c_int32 * TSSP_MAX_BLOCKS),
-    ]
-
-
-class TsspLayout(C.Structure):
-    _fields_ = [
         ("dist_token", C.c_int32),
         ("register_tokens", C.c_int32),
-        ("pos_covers_prefix", C.c_int32),
+        ("pos_patches_only", C.c_int32),
         ("layer_scale", C.c_int32),
-    ]
-
-
-class TsspModelOpts(C.Structure):
-    _fields_ = [
         ("pre_norm", C.c_int32),
         ("ffn_act", C.c_int32),
+        ("ffn_dims", C.c_int32 * TSSP_MAX_BLOCKS),
+        ("attn_present", C.c_int32 * TSSP_MAX_BLOCKS),
     ]
 
 
@@ -104,9 +94,6 @@ SIGNATURES = {
     "tssp_abi_version": (_I, []),
     "tssp_last_error": (C.c_char_p, []),
     "tssp_create": (_I, [C.POINTER(TsspConfig), _I, C.POINTER(_P)]),
-    "tssp_create_ex": (_I, [C.POINTER(TsspConfig), C.c_int32, _I, C.POINTER(_P)]),
-    "tssp_create_layout": (_I, [C.POINTER(TsspConfig), C.POINTER(TsspLayout), _I, C.POINTER(_P)]),
-    "tssp_create_model": (_I, [C.POINTER(TsspConfig), C.POINTER(TsspLayout), C.POINTER(TsspModelOpts), _I, C.POINTER(_P)]),
     "tssp_destroy": (_I, [_P]),
     "tssp_trim_pool": (_I, []),
     "tssp_load_weights": (_I, [_P, C.POINTER(_P), _I, _P]),
@@ -131,9 +118,7 @@ SIGNATURES = {
     "tssp_op_layernorm": (_I, [_P, _I64, _P, _P, _P, _I, _I, C.c_float, _P]),
     "tssp_op_layernorm_f32": (_I, [_P, _I64, _P, _P, _P, _I64, _I, _I, C.c_float, _P]),
     "tssp_op_attention": (_I, [_P, _P, _I, _I, _I, _I, _P]),
-    "tssp_op_im2col": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
-    "tssp_op_im2col_ex": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P]),
-    "tssp_op_im2col_u8": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, C.POINTER(TsspPixelInput), _P]),
+    "tssp_op_im2col": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, C.POINTER(TsspPixelInput), _P]),
     "tssp_op_cast_bf16": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P]),
     "tssp_op_argmax_count": (_I, [_P, _I, _I, _I, _P, _P, _P, _P]),
     "tssp_op_stable_rank_f64": (_I, [_P, _I, _I, _I, _P, _P]),

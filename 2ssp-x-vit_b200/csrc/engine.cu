@@ -409,25 +409,11 @@ static int op_cast(const float* in, int rows, int cols, int ld_in, void* out, in
 // prefix: zero rows ahead of every image's patches (1: CLS; 2: CLS and the DeiT distillation token; 1 + R: CLS and R
 // register tokens). Rows are patch_width(C, P) = round_up(C*P*P, 8) elements, zero padded past C*P*P.
 static int patch_width(int C, int P) { return round_up(C * P * P, 8); }
-static int op_im2col(const float* pixels, void* out, int n, int C, int H, int W, int P, cudaStream_t s, int prefix = 1) {
-    if (P < 1 || H % P || W % P || H != W) return fail("im2col: H=%d W=%d P=%d unsupported (square images, P dividing them)", H, W, P);
-    if (prefix < 1 || prefix > TSSP_MAX_PREFIX) return fail("im2col: prefix=%d must be in [1,%d]", prefix, TSSP_MAX_PREFIX);
-    const int T = (H / P) * (W / P) + prefix;
-    const int ld = patch_width(C, P);
-    const long long total = static_cast<long long>(n) * T * (ld / 8);
-    if ((P & 7) == 0) {
-        im2col_patches_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T, prefix);
-        TSSP_LAUNCH_CHECK("im2col_patches_kernel");
-    } else {
-        im2col_patches_padded_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T,
-                                                                          prefix, ld);
-        TSSP_LAUNCH_CHECK("im2col_patches_padded_kernel");
-    }
-    return 0;
-}
-
-// The normalisation of uint8 pixels (TSSP_PIXELS_U8) for a model with C channels: refused unless it can be applied.
-static int check_pixel_norm(const tssp_pixel_input_t& in, int C, const char* where) {
+// The pixel format of an im2col input (tssp_pixel_input_t): refused unless its normalisation can be applied to C channels.
+static int check_pixel_input(const tssp_pixel_input_t& in, int C, const char* where) {
+    if (in.format != TSSP_PIXELS_F32 && in.format != TSSP_PIXELS_U8)
+        return fail("%s: format=%d must be %d (fp32) or %d (uint8)", where, in.format, TSSP_PIXELS_F32, TSSP_PIXELS_U8);
+    if (in.format == TSSP_PIXELS_F32) return 0;
     if (C < 1 || C > TSSP_MAX_PIXEL_CHANNELS)
         return fail("%s: uint8 pixels need 1 to %d channels, got C=%d", where, TSSP_MAX_PIXEL_CHANNELS, C);
     if (!std::isfinite(in.rescale)) return fail("%s: rescale=%g is not finite", where, in.rescale);
@@ -438,31 +424,44 @@ static int check_pixel_norm(const tssp_pixel_input_t& in, int C, const char* whe
     return 0;
 }
 
-// im2col of uint8 pixels, normalised per channel on the way in (kernels.cuh: the fp32 kernels' bits for the normalised image)
-static int op_im2col_u8(const uint8_t* pixels, void* out, int n, int C, int H, int W, int P, const tssp_pixel_input_t& norm,
-                        cudaStream_t s, int prefix) {
+// in == nullptr or TSSP_PIXELS_F32: fp32 pixels. TSSP_PIXELS_U8: uint8 pixels, normalised per channel on the way in
+// (kernels.cuh: the fp32 kernels' bits for the normalised image).
+static int op_im2col(const void* pixels, void* out, int n, int C, int H, int W, int P, int prefix, const tssp_pixel_input_t* in,
+                     cudaStream_t s) {
     if (P < 1 || H % P || W % P || H != W) return fail("im2col: H=%d W=%d P=%d unsupported (square images, P dividing them)", H, W, P);
     if (prefix < 1 || prefix > TSSP_MAX_PREFIX) return fail("im2col: prefix=%d must be in [1,%d]", prefix, TSSP_MAX_PREFIX);
-    TSSP_TRY(check_pixel_norm(norm, C, "im2col (uint8 pixels)"));
-    const uintptr_t align = (P & 7) == 0 ? 8 : ((P & 1) == 0 ? 2 : 1);  // the 8-byte / 2-byte loads of the two kernels
-    if (reinterpret_cast<uintptr_t>(pixels) % align != 0)
-        return fail("im2col (uint8 pixels): pointer %p is not %d-byte aligned, as the loads at P=%d need", static_cast<const void*>(pixels),
-                    static_cast<int>(align), P);
-    PixelNorm pn;
-    pn.rescale = norm.rescale;
-    for (int c = 0; c < 4; ++c) {
-        pn.mean[c] = c < C ? norm.mean[c] : 0.0f;
-        pn.std[c] = c < C ? norm.std[c] : 1.0f;
-    }
+    if (in != nullptr) TSSP_TRY(check_pixel_input(*in, C, "im2col"));
+    const bool u8 = in != nullptr && in->format == TSSP_PIXELS_U8;
     const int T = (H / P) * (W / P) + prefix;
     const int ld = patch_width(C, P);
     const long long total = static_cast<long long>(n) * T * (ld / 8);
+    __nv_bfloat16* o = static_cast<__nv_bfloat16*>(out);
+    if (!u8) {
+        const float* px = static_cast<const float*>(pixels);
+        if ((P & 7) == 0) {
+            im2col_patches_kernel<<<grid_for(total, 256), 256, 0, s>>>(px, o, n, C, H, W, P, T, prefix);
+            TSSP_LAUNCH_CHECK("im2col_patches_kernel");
+        } else {
+            im2col_patches_padded_kernel<<<grid_for(total, 256), 256, 0, s>>>(px, o, n, C, H, W, P, T, prefix, ld);
+            TSSP_LAUNCH_CHECK("im2col_patches_padded_kernel");
+        }
+        return 0;
+    }
+    const uintptr_t align = (P & 7) == 0 ? 8 : ((P & 1) == 0 ? 2 : 1);  // the 8-byte / 2-byte loads of the two kernels
+    if (reinterpret_cast<uintptr_t>(pixels) % align != 0)
+        return fail("im2col (uint8 pixels): pointer %p is not %d-byte aligned, as the loads at P=%d need", pixels, static_cast<int>(align), P);
+    PixelNorm pn;
+    pn.rescale = in->rescale;
+    for (int c = 0; c < 4; ++c) {
+        pn.mean[c] = c < C ? in->mean[c] : 0.0f;
+        pn.std[c] = c < C ? in->std[c] : 1.0f;
+    }
+    const uint8_t* px = static_cast<const uint8_t*>(pixels);
     if ((P & 7) == 0) {
-        im2col_patches_u8_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T, prefix, pn);
+        im2col_patches_u8_kernel<<<grid_for(total, 256), 256, 0, s>>>(px, o, n, C, H, W, P, T, prefix, pn);
         TSSP_LAUNCH_CHECK("im2col_patches_u8_kernel");
     } else {
-        im2col_patches_padded_u8_kernel<<<grid_for(total, 256), 256, 0, s>>>(pixels, static_cast<__nv_bfloat16*>(out), n, C, H, W, P, T,
-                                                                             prefix, ld, pn);
+        im2col_patches_padded_u8_kernel<<<grid_for(total, 256), 256, 0, s>>>(px, o, n, C, H, W, P, T, prefix, ld, pn);
         TSSP_LAUNCH_CHECK("im2col_patches_padded_u8_kernel");
     }
     return 0;
@@ -637,7 +636,7 @@ struct BlockWeights {
     const float *ln1_w, *ln1_b, *ln2_w, *ln2_b;  // fp32 (arena)
     __nv_bfloat16 *qkv_w, *proj_w, *fc1_w, *fc2_w;
     float *qkv_b, *proj_b, *fc1_b, *fc2_b;
-    float *ls1, *ls2; // LayerScale gammas of the attention / MLP branch [D] (layout.layer_scale), else nullptr
+    float *ls1, *ls2; // LayerScale gammas of the attention / MLP branch [D] (cfg.layer_scale), else nullptr
     int F, Fp;        // current width and its padding to a multiple of 8
     int F_cap;        // allocated (padded) width
     int score_off;    // column offset of this block in the concatenated score / norm vectors
@@ -663,9 +662,7 @@ struct tssp_engine {
     tssp_config_t cfg;
     int device;
     int T, M_cap, Kp, G;
-    tssp_layout_t layout;
-    tssp_model_opts_t opts;
-    int prefix;     // tokens ahead of the patches: 1 (CLS) + layout.dist_token + layout.register_tokens
+    int prefix;     // tokens ahead of the patches: 1 (CLS) + cfg.dist_token + cfg.register_tokens
     int head_rows;  // rows the classifier may read: 2 with a distillation token (CLS, distillation), else 1 (CLS)
     bool dist_head; // a distillation head is loaded: logits = (cls_head(row 0) + dist_head(row 1)) / 2
     int sumF;  // sum of current F over blocks (score vector length)
@@ -678,7 +675,7 @@ struct tssp_engine {
     // global weights
     __nv_bfloat16 *patch_w, *head0_w, *head_w, *head_dist_w;  // with a distillation head both heads are packed at 0.5 scale
     float *posmod, *final_ln_w, *final_ln_b, *head_b, *head_dist_b;
-    float *norm_pre_w, *norm_pre_b;  // opts.pre_norm: LayerNorm over every token before block 0, else nullptr
+    float *norm_pre_w, *norm_pre_b;  // cfg.pre_norm: LayerNorm over every token before block 0, else nullptr
     int Cp, Hhp;  // padded classes / head hidden
     // workspace
     float* pixels[2];          // double-buffered staging of host pixel batches (fp32-sized: a uint8 batch fits too)
@@ -776,19 +773,19 @@ static int dev_alloc(tssp_engine* e, Tp** out, size_t count) {
     return 0;
 }
 
-static int validate(const tssp_config_t& c, const tssp_layout_t& l, const tssp_model_opts_t& o) {
-    if (o.pre_norm != 0 && o.pre_norm != 1) return fail("options: pre_norm=%d must be 0 or 1", o.pre_norm);
-    if (o.ffn_act != TSSP_FFN_GELU && o.ffn_act != TSSP_FFN_QUICK_GELU)
-        return fail("options: ffn_act=%d must be %d (erf GELU) or %d (QuickGELU)", o.ffn_act, TSSP_FFN_GELU, TSSP_FFN_QUICK_GELU);
-    if (o.ffn_act == TSSP_FFN_QUICK_GELU && c.score_point != 1)
-        return fail("options: QuickGELU is scored before the activation only (score_point=1, got %d)", c.score_point);
-    if (l.dist_token != 0 && l.dist_token != 1) return fail("layout: dist_token=%d must be 0 or 1", l.dist_token);
-    if (l.register_tokens < 0 || l.register_tokens > TSSP_MAX_REGISTER_TOKENS)
-        return fail("layout: register_tokens=%d must be in [0,%d]", l.register_tokens, TSSP_MAX_REGISTER_TOKENS);
-    if (l.dist_token && l.register_tokens > 0) return fail("layout: a distillation token and register tokens cannot be combined");
-    if (l.pos_covers_prefix != 0 && l.pos_covers_prefix != 1) return fail("layout: pos_covers_prefix=%d must be 0 or 1", l.pos_covers_prefix);
-    if (l.layer_scale != 0 && l.layer_scale != 1) return fail("layout: layer_scale=%d must be 0 or 1", l.layer_scale);
-    const int prefix = 1 + l.dist_token + l.register_tokens;
+static int validate(const tssp_config_t& c) {
+    if (c.dist_token != 0 && c.dist_token != 1) return fail("config: dist_token=%d must be 0 or 1", c.dist_token);
+    if (c.register_tokens < 0 || c.register_tokens > TSSP_MAX_REGISTER_TOKENS)
+        return fail("config: register_tokens=%d must be in [0,%d]", c.register_tokens, TSSP_MAX_REGISTER_TOKENS);
+    if (c.dist_token && c.register_tokens > 0) return fail("config: a distillation token and register tokens cannot be combined");
+    if (c.pos_patches_only != 0 && c.pos_patches_only != 1) return fail("config: pos_patches_only=%d must be 0 or 1", c.pos_patches_only);
+    if (c.layer_scale != 0 && c.layer_scale != 1) return fail("config: layer_scale=%d must be 0 or 1", c.layer_scale);
+    if (c.pre_norm != 0 && c.pre_norm != 1) return fail("config: pre_norm=%d must be 0 or 1", c.pre_norm);
+    if (c.ffn_act != TSSP_FFN_GELU && c.ffn_act != TSSP_FFN_QUICK_GELU)
+        return fail("config: ffn_act=%d must be %d (erf GELU) or %d (QuickGELU)", c.ffn_act, TSSP_FFN_GELU, TSSP_FFN_QUICK_GELU);
+    if (c.ffn_act == TSSP_FFN_QUICK_GELU && c.score_point != 1)
+        return fail("config: QuickGELU is scored before the activation only (score_point=1, got %d)", c.score_point);
+    const int prefix = 1 + c.dist_token + c.register_tokens;
     if (c.n_blocks < 1 || c.n_blocks > TSSP_MAX_BLOCKS) return fail("config: n_blocks=%d out of range", c.n_blocks);
     if ((c.hidden % 128 && c.hidden != 192) || c.hidden > 1024 || c.hidden < 128)
         return fail("config: hidden=%d must be 192 or a multiple of 128 in [128,1024]", c.hidden);
@@ -803,10 +800,9 @@ static int validate(const tssp_config_t& c, const tssp_layout_t& l, const tssp_m
     return 0;
 }
 
-static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, const tssp_model_opts_t& opts, int device,
-                         tssp_engine** out) {
-    TSSP_TRY(validate(*cfg, layout, opts));
-    const int prefix = 1 + layout.dist_token + layout.register_tokens;
+static int engine_create(const tssp_config_t* cfg, int device, tssp_engine** out) {
+    TSSP_TRY(validate(*cfg));
+    const int prefix = 1 + cfg->dist_token + cfg->register_tokens;
     int n_dev = 0;
     TSSP_CUDA(cudaGetDeviceCount(&n_dev));
     if (device < 0 || device >= n_dev) return fail("device %d out of range (%d visible)", device, n_dev);
@@ -821,10 +817,8 @@ static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, 
     e->weights_loaded = false;
     const int D = cfg->hidden, B = cfg->n_blocks;
     e->G = cfg->image_size / cfg->patch_size;
-    e->layout = layout;
-    e->opts = opts;
     e->prefix = prefix;
-    e->head_rows = 1 + layout.dist_token;
+    e->head_rows = 1 + cfg->dist_token;
     e->dist_head = false;
     e->T = e->G * e->G + prefix;
     e->M_cap = cfg->max_images * e->T;
@@ -845,11 +839,11 @@ static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, 
     e->head_dist_b = nullptr;
     e->norm_pre_w = nullptr;
     e->norm_pre_b = nullptr;
-    if (opts.pre_norm) {
+    if (cfg->pre_norm) {
         A(&e->norm_pre_w, D);
         A(&e->norm_pre_b, D);
     }
-    if (layout.dist_token && cfg->n_classes > 0) {
+    if (cfg->dist_token && cfg->n_classes > 0) {
         A(&e->head_dist_w, static_cast<size_t>(e->Cp) * D);
         A(&e->head_dist_b, e->Cp);
     }
@@ -868,7 +862,7 @@ static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, 
         A(&w.fc1_w, static_cast<size_t>(w.F_cap) * D); A(&w.fc1_b, w.F_cap);
         A(&w.fc2_w, static_cast<size_t>(D) * w.F_cap); A(&w.fc2_b, D);
         w.ls1 = w.ls2 = nullptr;
-        if (layout.layer_scale) { A(&w.ls1, D); A(&w.ls2, D); }
+        if (cfg->layer_scale) { A(&w.ls1, D); A(&w.ls2, D); }
     }
     e->ldn = off;
     e->sumF = 0;
@@ -930,7 +924,7 @@ static int engine_create(const tssp_config_t* cfg, const tssp_layout_t& layout, 
 // posmod[0] = cls + pos[0]; posmod[t < prefix] = tokens[t - 1] + pos[t] (the distillation token or the register tokens);
 // posmod[t >= prefix] = pos[t] + conv_bias (so the patch GEMM needs no bias and the prefix rows, whose im2col rows are
 // zero, receive exactly token + pos: HF ViTEmbeddings.forward / DeiTEmbeddings.forward, timm _pos_embed). With a
-// class-free position table (pos_covers_prefix = 0, timm no_embed_class) pos has G^2 rows: the prefix rows are the
+// class-free position table (pos_patches_only = 1, timm no_embed_class) pos has G^2 rows: the prefix rows are the
 // bare tokens and patch row t takes pos[t - prefix].
 __global__ void build_posmod_kernel(const float* __restrict__ pos, const float* __restrict__ cls, const float* __restrict__ tokens,
                                     const float* __restrict__ conv_b, float* __restrict__ out, int T, int D, int prefix,
@@ -973,52 +967,61 @@ static int pack_ffn(tssp_engine* e, int b, int F, const float* fc1_w, const floa
 static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cudaStream_t s) {
     const tssp_config_t& c = e->cfg;
     const int D = c.hidden, B = c.n_blocks;
-    const tssp_layout_t& l = e->layout;
-    const int n_ext = l.dist_token ? TSSP_WX_COUNT : 0;
-    const int n_layout = (l.register_tokens > 0 ? 1 : 0) + (l.layer_scale ? 2 * B : 0);
-    const int n_expected = TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT + n_ext + n_layout + (e->opts.pre_norm ? 2 : 0);
+    const int n_expected = TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT;
     if (n_entries != n_expected)
-        return fail("load_weights: expected %d pointers for %d prefix token(s)%s%s, got %d", n_expected, e->prefix,
-                    l.layer_scale ? " and LayerScale" : "", e->opts.pre_norm ? " and a pre-norm" : "", n_entries);
+        return fail("load_weights: expected %d pointers (TSSP_W_GLOBAL_COUNT + %d blocks * TSSP_BW_COUNT), got %d", n_expected, B, n_entries);
     auto need = [&](int idx, const char* name) -> int { return t[idx] == nullptr ? fail("load_weights: %s is NULL", name) : 0; };
     TSSP_TRY(need(TSSP_W_PATCH_W, "patch_w")); TSSP_TRY(need(TSSP_W_CLS, "cls_token")); TSSP_TRY(need(TSSP_W_POS, "pos_embed"));
     TSSP_TRY(need(TSSP_W_FINAL_LN_W, "final_ln_w")); TSSP_TRY(need(TSSP_W_FINAL_LN_B, "final_ln_b"));
-    const float* const* x = t + TSSP_W_GLOBAL_COUNT + B * TSSP_BW_COUNT;  // extension entries (distillation token only)
-    const float* const* lx = x + n_ext;                                  // layout entries (tssp_create_layout)
-    const float* reg_tokens = l.register_tokens > 0 ? lx[0] : nullptr;
-    const float* const* ls = lx + (l.register_tokens > 0 ? 1 : 0);       // per block LS1, LS2
-    const float* const* pn = lx + n_layout;                              // option entries (tssp_create_model): norm_pre
-    if (l.register_tokens > 0 && reg_tokens == nullptr) return fail("load_weights: register tokens are NULL");
-    if (e->opts.pre_norm && (pn[0] == nullptr || pn[1] == nullptr)) return fail("load_weights: norm_pre weight or bias is NULL");
-    if (l.layer_scale)
-        for (int b = 0; b < B; ++b) {
-            if (ls[2 * b + 1] == nullptr) return fail("load_weights: block %d LS2 gamma is NULL", b);
-            if (c.attn_present[b] && ls[2 * b] == nullptr) return fail("load_weights: block %d LS1 gamma is NULL", b);
-        }
-    const bool dist_head = l.dist_token && x[TSSP_WX_HEAD_DIST_W] != nullptr;
-    if (l.dist_token) {
-        if (x[TSSP_WX_DIST_TOKEN] == nullptr) return fail("load_weights: distillation token is NULL");
+    // the slots of an option the config leaves off must be NULL: a table built for another config is refused
+    auto unused = [&](int idx, const char* slot, const char* field) -> int {
+        return t[idx] != nullptr ? fail("load_weights: %s is set, but the config has %s=0", slot, field) : 0;
+    };
+    if (!c.dist_token) {
+        TSSP_TRY(unused(TSSP_W_DIST_TOKEN, "TSSP_W_DIST_TOKEN", "dist_token"));
+        TSSP_TRY(unused(TSSP_W_HEAD_DIST_W, "TSSP_W_HEAD_DIST_W", "dist_token"));
+        TSSP_TRY(unused(TSSP_W_HEAD_DIST_B, "TSSP_W_HEAD_DIST_B", "dist_token"));
+    }
+    if (c.register_tokens == 0) TSSP_TRY(unused(TSSP_W_REG_TOKENS, "TSSP_W_REG_TOKENS", "register_tokens"));
+    if (!c.pre_norm) {
+        TSSP_TRY(unused(TSSP_W_NORM_PRE_W, "TSSP_W_NORM_PRE_W", "pre_norm"));
+        TSSP_TRY(unused(TSSP_W_NORM_PRE_B, "TSSP_W_NORM_PRE_B", "pre_norm"));
+    }
+    for (int b = 0; b < B; ++b) {
+        const float* const* w = t + TSSP_W_GLOBAL_COUNT + b * TSSP_BW_COUNT;
+        if (!c.layer_scale && (w[TSSP_BW_LS1] != nullptr || w[TSSP_BW_LS2] != nullptr))
+            return fail("load_weights: block %d TSSP_BW_LS%d is set, but the config has layer_scale=0", b, w[TSSP_BW_LS1] != nullptr ? 1 : 2);
+        if (c.layer_scale && w[TSSP_BW_LS2] == nullptr) return fail("load_weights: block %d LS2 gamma is NULL", b);
+        if (c.layer_scale && c.attn_present[b] && w[TSSP_BW_LS1] == nullptr) return fail("load_weights: block %d LS1 gamma is NULL", b);
+    }
+    if (c.register_tokens > 0 && t[TSSP_W_REG_TOKENS] == nullptr) return fail("load_weights: register tokens are NULL");
+    if (c.pre_norm && (t[TSSP_W_NORM_PRE_W] == nullptr || t[TSSP_W_NORM_PRE_B] == nullptr))
+        return fail("load_weights: norm_pre weight or bias is NULL");
+    const bool dist_head = c.dist_token && t[TSSP_W_HEAD_DIST_W] != nullptr;
+    if (c.dist_token) {
+        if (t[TSSP_W_DIST_TOKEN] == nullptr) return fail("load_weights: distillation token is NULL");
         if (dist_head && c.n_classes <= 0) return fail("load_weights: a distillation head needs n_classes > 0");
         if (dist_head && c.head_hidden > 0) return fail("load_weights: a distillation head cannot be combined with a Sequential head");
     }
     const int K = c.channels * c.patch_size * c.patch_size;  // Kp = K rounded up to 8: zero columns past K
     TSSP_TRY(op_cast(t[TSSP_W_PATCH_W], D, K, K, e->patch_w, D, e->Kp, e->Kp, s));
-    build_posmod_kernel<<<ceil_div(e->T * D, 256), 256, 0, s>>>(t[TSSP_W_POS], t[TSSP_W_CLS], l.dist_token ? x[TSSP_WX_DIST_TOKEN] : reg_tokens,
-                                                               t[TSSP_W_PATCH_B], e->posmod, e->T, D, e->prefix, l.pos_covers_prefix);
+    build_posmod_kernel<<<ceil_div(e->T * D, 256), 256, 0, s>>>(t[TSSP_W_POS], t[TSSP_W_CLS],
+                                                               t[c.dist_token ? TSSP_W_DIST_TOKEN : TSSP_W_REG_TOKENS], t[TSSP_W_PATCH_B],
+                                                               e->posmod, e->T, D, e->prefix, !c.pos_patches_only);
     TSSP_LAUNCH_CHECK("build_posmod_kernel");
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_W], D, e->final_ln_w, D, s));
     TSSP_TRY(copy_vec(t[TSSP_W_FINAL_LN_B], D, e->final_ln_b, D, s));
-    if (e->opts.pre_norm) {
-        TSSP_TRY(copy_vec(pn[0], D, e->norm_pre_w, D, s));
-        TSSP_TRY(copy_vec(pn[1], D, e->norm_pre_b, D, s));
+    if (c.pre_norm) {
+        TSSP_TRY(copy_vec(t[TSSP_W_NORM_PRE_W], D, e->norm_pre_w, D, s));
+        TSSP_TRY(copy_vec(t[TSSP_W_NORM_PRE_B], D, e->norm_pre_b, D, s));
     }
     if (c.n_classes > 0 && dist_head) {
         // (cls_head(x0) + dist_head(x1)) / 2 as two GEMMs into the same logits (run_head): both heads at half scale
         TSSP_TRY(need(TSSP_W_HEAD_W, "head_w"));
         TSSP_TRY(op_cast(t[TSSP_W_HEAD_W], c.n_classes, D, D, e->head_w, e->Cp, D, D, s, 0.5f));
         TSSP_TRY(copy_vec(t[TSSP_W_HEAD_B], c.n_classes, e->head_b, e->Cp, s, 0.5f));
-        TSSP_TRY(op_cast(x[TSSP_WX_HEAD_DIST_W], c.n_classes, D, D, e->head_dist_w, e->Cp, D, D, s, 0.5f));
-        TSSP_TRY(copy_vec(x[TSSP_WX_HEAD_DIST_B], c.n_classes, e->head_dist_b, e->Cp, s, 0.5f));
+        TSSP_TRY(op_cast(t[TSSP_W_HEAD_DIST_W], c.n_classes, D, D, e->head_dist_w, e->Cp, D, D, s, 0.5f));
+        TSSP_TRY(copy_vec(t[TSSP_W_HEAD_DIST_B], c.n_classes, e->head_dist_b, e->Cp, s, 0.5f));
     } else if (c.n_classes > 0) {
         TSSP_TRY(need(TSSP_W_HEAD_W, "head_w"));
         if (c.head_hidden > 0) {
@@ -1053,9 +1056,9 @@ static int engine_load(tssp_engine* e, const float* const* t, int n_entries, cud
         }
         TSSP_TRY(pack_ffn(e, b, bw.F, w[TSSP_BW_FC1_W], w[TSSP_BW_FC1_B], w[TSSP_BW_FC2_W], s));
         TSSP_TRY(copy_vec(w[TSSP_BW_FC2_B], D, bw.fc2_b, D, s));
-        if (l.layer_scale) {
-            TSSP_TRY(copy_vec(ls[2 * b], D, bw.ls1, D, s));  // NULL (no attention) -> zeros, never read
-            TSSP_TRY(copy_vec(ls[2 * b + 1], D, bw.ls2, D, s));
+        if (c.layer_scale) {
+            TSSP_TRY(copy_vec(w[TSSP_BW_LS1], D, bw.ls1, D, s));  // NULL (no attention) -> zeros, never read
+            TSSP_TRY(copy_vec(w[TSSP_BW_LS2], D, bw.ls2, D, s));
         }
     }
     e->dist_head = dist_head;
@@ -1212,12 +1215,7 @@ static unsigned long long block_mask(const int32_t* flags, int B) {
 // caller's / the staged pixels, kept outside the captured chains so that those do not depend on where a batch lives
 static int run_im2col(tssp_engine* e, const void* dev_pixels, int n, cudaStream_t s) {
     const tssp_config_t& c = e->cfg;
-    if (e->pix.format == TSSP_PIXELS_U8)
-        TSSP_PROF(KC_MISC, s, op_im2col_u8(static_cast<const uint8_t*>(dev_pixels), e->patchA, n, c.channels, c.image_size, c.image_size,
-                                           c.patch_size, e->pix, s, e->prefix));
-    else
-        TSSP_PROF(KC_MISC, s, op_im2col(static_cast<const float*>(dev_pixels), e->patchA, n, c.channels, c.image_size, c.image_size,
-                                        c.patch_size, s, e->prefix));
+    TSSP_PROF(KC_MISC, s, op_im2col(dev_pixels, e->patchA, n, c.channels, c.image_size, c.image_size, c.patch_size, e->prefix, &e->pix, s));
     if (e->staged_slot >= 0) {  // the host-staged pixel buffer may be refilled once im2col has read it
         TSSP_CUDA(cudaEventRecord(e->ev_consumed[e->staged_slot], s));
         e->staged_slot = -1;
@@ -1237,7 +1235,7 @@ static int run_embed(tssp_engine* e, int n, cudaStream_t s) {
         TSSP_LAUNCH_CHECK("broadcast_rows_kernel");
     }
     TSSP_PROF(KC_PATCH, s, gemm(EPI_F32, e->patchA, e->Kp, e->patch_w, e->Kp, e->x, D, M, D, e->Kp, nullptr, nullptr, 0, e->T, 1, s));
-    if (e->opts.pre_norm) TSSP_PROF(KC_LN, s, op_layernorm_f32(e->x, D, e->norm_pre_w, e->norm_pre_b, e->x, D, M, D, c.ln_eps, s));
+    if (c.pre_norm) TSSP_PROF(KC_LN, s, op_layernorm_f32(e->x, D, e->norm_pre_w, e->norm_pre_b, e->x, D, M, D, c.ln_eps, s));
     return 0;
 }
 
@@ -1260,7 +1258,7 @@ static int run_block(tssp_engine* e, int b, int n, bool skip_attn, Fc1Mode fc1_m
     const int rows = cls_only ? n : M;              // rows the row-wise part of the block works on
     const int pitch = cls_only ? e->T * D : D;      // their distance in x / ctx
     const bool attn = e->attn_present[b] && !skip_attn;
-    const bool qgelu = e->opts.ffn_act == TSSP_FFN_QUICK_GELU;
+    const bool qgelu = e->cfg.ffn_act == TSSP_FFN_QUICK_GELU;
     const int fc1_plain = qgelu ? EPI_BF16_QGELU : EPI_BF16_GELU;
     // proj / fc2 add their branch into the residual stream, scaled by the block's LayerScale gamma when the model has one
     auto residual_gemm = [&](const void* A, int lda, const __nv_bfloat16* W, int ldw, float* xr, int rows_, int K, const float* bias,
@@ -1438,28 +1436,11 @@ int tssp_profile_end(double* ms_per_class, unsigned long long* launches_per_clas
     return 0;
 }
 
-int tssp_create_model(const tssp_config_t* cfg, const tssp_layout_t* layout, const tssp_model_opts_t* opts, int device,
-                      tssp_handle_t* out) {
+int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out) {
     TSSP_ENTRY();
-    if (cfg == nullptr || layout == nullptr || opts == nullptr || out == nullptr) return fail("tssp_create: NULL argument");
-    return engine_create(cfg, *layout, *opts, device, out);
+    if (cfg == nullptr || out == nullptr) return fail("tssp_create: NULL argument");
+    return engine_create(cfg, device, out);
 }
-
-int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, int device, tssp_handle_t* out) {
-    const tssp_model_opts_t opts = {0, TSSP_FFN_GELU};
-    return tssp_create_model(cfg, layout, &opts, device, out);
-}
-
-int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out) {
-    if (prefix_tokens < 1 || prefix_tokens > 2) {
-        TSSP_ENTRY();
-        return fail("config: prefix_tokens=%d must be 1 (CLS) or 2 (CLS and distillation token)", prefix_tokens);
-    }
-    const tssp_layout_t layout = {prefix_tokens == 2 ? 1 : 0, 0, 1, 0};
-    return tssp_create_layout(cfg, &layout, device, out);
-}
-
-int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out) { return tssp_create_ex(cfg, 1, device, out); }
 
 int tssp_destroy(tssp_handle_t h) {
     TSSP_ENTRY();
@@ -1518,9 +1499,7 @@ int tssp_set_attention(tssp_handle_t h, const int32_t* present) {
 int tssp_set_pixel_input(tssp_handle_t h, const tssp_pixel_input_t* input) {
     TSSP_ENGINE_ENTRY(h, "tssp_set_pixel_input");
     if (input == nullptr) return fail("tssp_set_pixel_input: NULL argument");
-    if (input->format != TSSP_PIXELS_F32 && input->format != TSSP_PIXELS_U8)
-        return fail("tssp_set_pixel_input: format=%d must be %d (fp32) or %d (uint8)", input->format, TSSP_PIXELS_F32, TSSP_PIXELS_U8);
-    if (input->format == TSSP_PIXELS_U8) TSSP_TRY(check_pixel_norm(*input, h->cfg.channels, "tssp_set_pixel_input"));
+    TSSP_TRY(check_pixel_input(*input, h->cfg.channels, "tssp_set_pixel_input"));
     h->pix = *input;
     return 0;
 }
@@ -1844,19 +1823,11 @@ int tssp_debug_attention_trace(long long* device_buf) {
     ++g_launch_epoch;
     return 0;
 }
-int tssp_op_im2col_ex(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens, void* stream) {
+int tssp_op_im2col(const void* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens,
+                   const tssp_pixel_input_t* input, void* stream) {
     TSSP_ENTRY();
     if (pixels == nullptr || out_bf16 == nullptr) return fail("tssp_op_im2col: NULL argument");
-    return op_im2col(pixels, out_bf16, n_img, C, H, W, P, static_cast<cudaStream_t>(stream), prefix_tokens);
-}
-int tssp_op_im2col_u8(const uint8_t* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens,
-                      const tssp_pixel_input_t* norm, void* stream) {
-    TSSP_ENTRY();
-    if (pixels == nullptr || out_bf16 == nullptr || norm == nullptr) return fail("tssp_op_im2col_u8: NULL argument");
-    return op_im2col_u8(pixels, out_bf16, n_img, C, H, W, P, *norm, static_cast<cudaStream_t>(stream), prefix_tokens);
-}
-int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream) {
-    return tssp_op_im2col_ex(pixels, out_bf16, n_img, C, H, W, P, 1, stream);
+    return op_im2col(pixels, out_bf16, n_img, C, H, W, P, prefix_tokens, input, static_cast<cudaStream_t>(stream));
 }
 int tssp_op_cast_bf16(const float* in, int rows, int cols, int ld_in, void* out_bf16, int rows_pad, int cols_pad, int ld_out, void* stream) {
     TSSP_ENTRY();

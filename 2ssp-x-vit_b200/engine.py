@@ -13,10 +13,11 @@ import torch
 from . import _lib as L
 from .anatomy import Anatomy, describe
 
-_GLOBAL_ORDER = ["patch_w", "patch_b", "cls", "pos", "final_ln_w", "final_ln_b", "head0_w", "head_w", "head_b"]
-_EXT_ORDER = ["dist", "head_dist_w", "head_dist_b"]  # engines with a distillation token (include/tssp.h: tssp_weight_ext_index)
+# the weight table (include/tssp.h: tssp_weight_index / tssp_block_weight_index); a key the anatomy lacks is NULL
+_GLOBAL_ORDER = ["patch_w", "patch_b", "cls", "pos", "final_ln_w", "final_ln_b", "head0_w", "head_w", "head_b",
+                 "dist", "head_dist_w", "head_dist_b", "reg", "norm_pre_w", "norm_pre_b"]
 _BLOCK_ORDER = ["ln1_w", "ln1_b", "q_w", "q_b", "k_w", "k_b", "v_w", "v_b", "proj_w", "proj_b",
-                "ln2_w", "ln2_b", "fc1_w", "fc1_b", "fc2_w", "fc2_b"]
+                "ln2_w", "ln2_b", "fc1_w", "fc1_b", "fc2_w", "fc2_b", "ls1", "ls2"]
 
 
 def _cuda_device(device) -> torch.device:
@@ -42,6 +43,8 @@ class Engine:
         cfg.n_classes, cfg.head_hidden = a.n_classes, a.head_hidden
         cfg.max_images, cfg.score_point, cfg.cache_blocks = self.max_images, a.score_point, int(self.cache_blocks)
         cfg.ln_eps = a.ln_eps
+        cfg.dist_token, cfg.register_tokens, cfg.pos_patches_only = int(a.dist_token), a.register_tokens, int(not a.pos_covers_prefix)
+        cfg.layer_scale, cfg.pre_norm, cfg.ffn_act = int(a.layer_scale), int(a.pre_norm), L.FFN_ACTS[a.ffn_act]
         if a.n_blocks > L.TSSP_MAX_BLOCKS:
             raise L.TsspError(f"{a.n_blocks} blocks exceed TSSP_MAX_BLOCKS={L.TSSP_MAX_BLOCKS}")
         for i in range(a.n_blocks):
@@ -49,13 +52,7 @@ class Engine:
             cfg.attn_present[i] = 1 if a.attn_present[i] else 0
         self._handle = C.c_void_p()
         with torch.cuda.device(self.device):
-            layout = L.TsspLayout(int(a.dist_token), a.register_tokens, int(a.pos_covers_prefix), int(a.layer_scale))
-            if a.pre_norm or a.ffn_act != "gelu":
-                opts = L.TsspModelOpts(int(a.pre_norm), L.FFN_ACTS[a.ffn_act])
-                L.check(self.lib.tssp_create_model(C.byref(cfg), C.byref(layout), C.byref(opts), self.device.index,
-                                                   C.byref(self._handle)))
-            else:
-                L.check(self.lib.tssp_create_layout(C.byref(cfg), C.byref(layout), self.device.index, C.byref(self._handle)))
+            L.check(self.lib.tssp_create(C.byref(cfg), self.device.index, C.byref(self._handle)))
         self.ffn_dims = list(a.ffn_dims)
         self.pixel_norm = None                # (mean, std, rescale): see set_pixel_normalization
         self._pixel_format = (L.PIXELS_F32, None)  # what the library engine reads its `pixels` pointers as
@@ -76,15 +73,6 @@ class Engine:
         entries = [self._dev32(a.globals_.get(k), keep) for k in _GLOBAL_ORDER]
         for blk in a.blocks:
             entries += [self._dev32(blk.get(k), keep) for k in _BLOCK_ORDER]
-        if a.dist_token:
-            entries += [self._dev32(a.globals_.get(k), keep) for k in _EXT_ORDER]
-        if a.register_tokens > 0:  # then the layout entries of tssp_create_layout
-            entries.append(self._dev32(a.globals_["reg"], keep))
-        if a.layer_scale:
-            for blk in a.blocks:
-                entries += [self._dev32(blk.get("ls1"), keep), self._dev32(blk.get("ls2"), keep)]
-        if a.pre_norm:  # then the option entries of tssp_create_model
-            entries += [self._dev32(a.globals_["norm_pre_w"], keep), self._dev32(a.globals_["norm_pre_b"], keep)]
         table = (C.c_void_p * len(entries))(*entries)
         with torch.cuda.device(self.device):
             L.check(self.lib.tssp_load_weights(self._handle, table, len(entries), L.current_stream()))

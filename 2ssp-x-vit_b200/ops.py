@@ -148,12 +148,8 @@ def im2col(pixels: torch.Tensor, patch: int, prefix: int = 1, *, mean=None, std=
     n, c, h, w = pixels.shape
     T = (h // patch) * (w // patch) + prefix
     out = torch.empty(n * T, (c * patch * patch + 7) // 8 * 8, device=pixels.device, dtype=torch.bfloat16)
-    lib = L.load()
-    if u8:
-        norm = L.pixel_input(L.PIXELS_U8, [float(v) for v in mean], [float(v) for v in std], float(rescale))
-        L.check(lib.tssp_op_im2col_u8(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, norm, L.current_stream()))
-    else:
-        L.check(lib.tssp_op_im2col_ex(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, L.current_stream()))
+    norm = L.pixel_input(L.PIXELS_U8, [float(v) for v in mean], [float(v) for v in std], float(rescale)) if u8 else None
+    L.check(L.load().tssp_op_im2col(L.ptr(pixels), L.ptr(out), n, c, h, w, patch, prefix, norm, L.current_stream()))
     return out
 
 

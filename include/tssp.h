@@ -31,16 +31,21 @@ extern "C" {
 #endif
 
 #define TSSP_MAX_BLOCKS 64
-#define TSSP_ABI_VERSION 1
+#define TSSP_ABI_VERSION 2
 
 typedef struct tssp_engine* tssp_handle_t;
 
 /* Model anatomy, as discovered by the reference's _get_encoder/_gather_mlp_pairs walkers
- * (src/vit_pruning.py:28-75) on an HF ViTForImageClassification or a timm VisionTransformer.
- * Tokens per image T = (image_size / patch_size)^2 + prefix tokens (1 for ViT, 2 for DeiT: see tssp_create_ex; 1 + R with
- * R register tokens: see tssp_create_layout) must lie in [32, 1025]: ViT-x/16 up to 512x512 (T = 1025), ViT-x/8 up to
- * 256x256, ViT-x/14 up to 448x448; tssp_create rejects other shapes (DINOv2 at its native 518x518: T = 1370) before it
- * touches a device. */
+ * (src/vit_pruning.py:28-75) on an HF ViTForImageClassification or a timm VisionTransformer, and the options of the timm
+ * VisionTransformer models beyond plain ViT (timm vision_transformer.py: VisionTransformer._pos_embed, LayerScale,
+ * Block.forward, pre_norm, act_layer). Zero is the plain-ViT behaviour of every option, so a zeroed struct with the model's
+ * shape filled in describes a ViT with one CLS token.
+ * Tokens per image T = (image_size / patch_size)^2 + 1 + dist_token + register_tokens must lie in [32, 1025]: ViT-x/16 up
+ * to 512x512 (T = 1025), ViT-x/8 up to 256x256, ViT-x/14 up to 448x448; tssp_create rejects other shapes (DINOv2 at its
+ * native 518x518: T = 1370) and invalid options before it touches a device. */
+#define TSSP_MAX_REGISTER_TOKENS 7
+#define TSSP_FFN_GELU 0        /* erf GELU (nn.GELU(), HF "gelu") */
+#define TSSP_FFN_QUICK_GELU 1  /* QuickGELU, x * sigmoid(1.702 x) (timm QuickGELU); needs score_point = 1 */
 typedef struct tssp_config {
     int32_t n_blocks;                      /* B: encoder blocks */
     int32_t hidden;                        /* D: 192 (DeiT-Ti, ViT-Ti) or a multiple of 128, <= 1024 */
@@ -57,23 +62,48 @@ typedef struct tssp_config {
                                               1: hook before GELU (timm mlp.fc1, src/vit_pruning.py:135) */
     int32_t cache_blocks;                  /* 1: allocate the Stage-2 pre-block activation cache */
     float ln_eps;                          /* LayerNorm eps of the module (1e-12 HF, 1e-6 timm norms) */
+    int32_t dist_token;                    /* 1: DeiT distillation token after CLS (transformers DeiTEmbeddings.forward:
+                                              [CLS, distillation token, patches] + positions; timm
+                                              VisionTransformerDistilled). With a distillation head the logits are
+                                              (cls_head(row 0) + dist_head(row 1)) / 2, the eval-mode output of
+                                              DeiTForImageClassificationWithTeacher and of timm's distilled models; a
+                                              Sequential head cannot be combined with one. Without it
+                                              (DeiTForImageClassification) the head reads the CLS row only. */
+    int32_t register_tokens;               /* R timm register tokens after CLS (reg_token [1, R, D]), 0..7; not with
+                                              dist_token. The classifier reads the CLS row. */
+    int32_t pos_patches_only;              /* 0: pos table [T, D] covers the prefix rows (ViT, DeiT, DINOv2);
+                                              1: pos table [G^2, D] for the patches only, the prefix rows get no
+                                              position (timm no_embed_class: DeiT-III, DINOv2 with registers) */
+    int32_t layer_scale;                   /* 1: every block scales its attention and MLP outputs by ls1.gamma /
+                                              ls2.gamma before the residual add: x += gamma * (proj(a) + b), in fp32 */
+    int32_t pre_norm;                      /* 1: a LayerNorm (timm norm_pre, eps = ln_eps) over every token after the
+                                              position embedding and before block 0 (timm CLIP image towers) */
+    int32_t ffn_act;                       /* TSSP_FFN_GELU or TSSP_FFN_QUICK_GELU: the activation between fc1 and fc2 of
+                                              every block (a Sequential classification head keeps erf GELU) */
     int32_t ffn_dims[TSSP_MAX_BLOCKS];     /* F per block (intermediate width; may differ after Stage-1) */
     int32_t attn_present[TSSP_MAX_BLOCKS]; /* 0: this block's attention is already a bypass module */
 } tssp_config_t;
 
-/* Order of the fp32 device pointers handed to tssp_load_weights(). Per-block entries repeat n_blocks times
- * after the TSSP_W_GLOBAL_COUNT global ones. Q/K/V may alias one fused timm qkv weight (rows [0:D],[D:2D],[2D:3D],
+/* The table of fp32 device pointers handed to tssp_load_weights(): the TSSP_W_GLOBAL_COUNT global entries, then
+ * TSSP_BW_COUNT entries per block, always TSSP_W_GLOBAL_COUNT + n_blocks * TSSP_BW_COUNT pointers. The entries of an
+ * option the config does not enable must be NULL. Q/K/V may alias one fused timm qkv weight (rows [0:D],[D:2D],[2D:3D],
  * experiments/vit_pruning/auto_2ssp.py:436-440). */
 enum tssp_weight_index {
     TSSP_W_PATCH_W = 0, /* [D, C_in*P*P]  Conv2d weight flattened */
     TSSP_W_PATCH_B,     /* [D] */
     TSSP_W_CLS,         /* [D] */
-    TSSP_W_POS,         /* [T, D] */
+    TSSP_W_POS,         /* [T, D], or [G^2, D] with pos_patches_only */
     TSSP_W_FINAL_LN_W,  /* [D] */
     TSSP_W_FINAL_LN_B,  /* [D] */
     TSSP_W_HEAD0_W,     /* [head_hidden, D] or NULL */
     TSSP_W_HEAD_W,      /* [C, D] or [C, head_hidden] */
     TSSP_W_HEAD_B,      /* [C] or NULL */
+    TSSP_W_DIST_TOKEN,  /* dist_token: [D] distillation token (required) */
+    TSSP_W_HEAD_DIST_W, /* dist_token: [C, D] distillation head, or NULL: the classifier reads the CLS row only */
+    TSSP_W_HEAD_DIST_B, /* dist_token: [C] or NULL */
+    TSSP_W_REG_TOKENS,  /* register_tokens > 0: [R, D] (row-major reg_token[0]) */
+    TSSP_W_NORM_PRE_W,  /* pre_norm: [D] */
+    TSSP_W_NORM_PRE_B,  /* pre_norm: [D] */
     TSSP_W_GLOBAL_COUNT
 };
 enum tssp_block_weight_index {
@@ -83,64 +113,15 @@ enum tssp_block_weight_index {
     TSSP_BW_LN2_W, TSSP_BW_LN2_B,
     TSSP_BW_FC1_W, TSSP_BW_FC1_B, /* [F, D] / [F] */
     TSSP_BW_FC2_W, TSSP_BW_FC2_B, /* [D, F] / [D] */
+    TSSP_BW_LS1, TSSP_BW_LS2,     /* layer_scale: [D] gammas of the attention branch (NULL for a block without
+                                     attention) and of the MLP branch */
     TSSP_BW_COUNT
 };
-/* Engines with two prefix tokens (tssp_create_ex) take TSSP_WX_COUNT more entries after the per-block ones. */
-enum tssp_weight_ext_index {
-    TSSP_WX_DIST_TOKEN = 0, /* [D] distillation token (required) */
-    TSSP_WX_HEAD_DIST_W,    /* [C, D] distillation head, or NULL: the classifier reads the CLS row only */
-    TSSP_WX_HEAD_DIST_B,    /* [C] or NULL */
-    TSSP_WX_COUNT
-};
-
-/* Prefix-token and residual-branch layout of timm VisionTransformer models beyond ViT / DeiT (timm
- * vision_transformer.py: VisionTransformer._pos_embed, LayerScale, Block.forward). */
-#define TSSP_MAX_REGISTER_TOKENS 7
-typedef struct tssp_layout {
-    int32_t dist_token;        /* 1: DeiT distillation token after CLS (what tssp_create_ex(..., 2, ...) means) */
-    int32_t register_tokens;   /* R timm register tokens after CLS (reg_token [1, R, D]), 0..7; not with dist_token */
-    int32_t pos_covers_prefix; /* 1: pos table [T, D] covers the prefix rows (ViT, DeiT, DINOv2);
-                                  0: pos table [G^2, D] for the patches only, the prefix rows get no position
-                                  (timm no_embed_class: DeiT-III, DINOv2 with registers) */
-    int32_t layer_scale;       /* 1: every block scales its attention and MLP outputs by ls1.gamma / ls2.gamma before the
-                                  residual add: x += gamma * (proj(a) + b), in fp32 */
-} tssp_layout_t;
-/* Entries appended to the weight table of an engine made by tssp_create_layout, after the TSSP_WX_* ones (present only
- * with dist_token), in this order:
- *   register_tokens > 0: one entry, the register tokens [R, D] (row-major, reg_token[0]);
- *   layer_scale = 1:     2 * n_blocks entries, per block LS1 [D] (attention branch; NULL for a block without attention)
- *                        then LS2 [D] (MLP branch). */
-
-/* Model options beyond the token layout, for the timm CLIP image towers (timm vision_transformer.py: VisionTransformer with
- * pre_norm=True, act_layer='quick_gelu'; OpenAI and LAION ViT-B/32, B/16, L/14, L/14@336 and their fine-tunes). */
-#define TSSP_FFN_GELU 0        /* erf GELU (nn.GELU(), HF "gelu") */
-#define TSSP_FFN_QUICK_GELU 1  /* QuickGELU, x * sigmoid(1.702 x) (timm QuickGELU); needs score_point = 1 */
-typedef struct tssp_model_opts {
-    int32_t pre_norm; /* 1: a LayerNorm (timm norm_pre, eps = ln_eps) over every token after the position embedding and
-                         before block 0; its weight and bias [D] are the last two entries of the weight table */
-    int32_t ffn_act;  /* TSSP_FFN_GELU or TSSP_FFN_QUICK_GELU: the activation between fc1 and fc2 of every block (a
-                         Sequential classification head keeps erf GELU) */
-} tssp_model_opts_t;
 
 int tssp_abi_version(void);
 const char* tssp_last_error(void);
 
 int tssp_create(const tssp_config_t* cfg, int device, tssp_handle_t* out);
-/* Same, for models with `prefix_tokens` (1 or 2) tokens ahead of the patches; tssp_create is this with 1. Two is DeiT
- * (transformers models/deit/modeling_deit.py DeiTEmbeddings.forward: [CLS, distillation token, patches] + positions;
- * timm VisionTransformerDistilled): T = G^2 + 2, and the weight table carries the TSSP_WX_* entries. With a distillation
- * head the logits are (cls_head(row 0) + dist_head(row 1)) / 2, the eval-mode output of
- * DeiTForImageClassificationWithTeacher.forward and of timm's distilled models; a Sequential head (head_hidden > 0) cannot
- * be combined with one. Without it (DeiTForImageClassification.forward) the head reads the CLS row only. */
-int tssp_create_ex(const tssp_config_t* cfg, int32_t prefix_tokens, int device, tssp_handle_t* out);
-/* The general form: tssp_create is this with the layout {0, 0, 1, 0}, tssp_create_ex with {prefix_tokens == 2, 0, 1, 0}.
- * T = G^2 + 1 + dist_token + register_tokens. Models with register tokens feed the classifier from the CLS row. */
-int tssp_create_layout(const tssp_config_t* cfg, const tssp_layout_t* layout, int device, tssp_handle_t* out);
-/* The most general form: tssp_create_layout is this with the options {0, TSSP_FFN_GELU}. With pre_norm = 1 the weight table
- * ends with norm_pre weight [D], norm_pre bias [D], after every entry tssp_create_layout's table has. Invalid options are
- * refused before any device is touched. */
-int tssp_create_model(const tssp_config_t* cfg, const tssp_layout_t* layout, const tssp_model_opts_t* opts, int device,
-                      tssp_handle_t* out);
 
 /* Pixel input format of an engine's batch entry points (tssp_s1_batch, tssp_forward_logits, tssp_eval_batch,
  * tssp_s2_batch). TSSP_PIXELS_F32 (the default): `pixels` is fp32 [n, C, H, W], fed to the patch embedding as it is.
@@ -249,15 +230,14 @@ int tssp_op_layernorm_f32(const float* x, int64_t in_stride, const float* gamma,
 /* ctx[n*T, D] = softmax(Q K^T / 8) V per (image, head) from the fused qkv[n*T, 3D]; head_dim 64, 16 <= T <= 1025
  * (up to 208 padded keys one kernel holds a whole key row, beyond that a second one streams keys in tiles of 128). */
 int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream);
-int tssp_op_im2col(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, void* stream);
 /* out[n * T, Kp] with T = (H/P)^2 + prefix_tokens and Kp = round_up(C*P*P, 8): prefix_tokens (1..8) zero rows ahead of
- * every image's patches, columns past C*P*P zero (the padded patch vector of patch sizes that are not a multiple of 8) */
-int tssp_op_im2col_ex(const float* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens, void* stream);
-/* the same from uint8 pixels [n_img, C, H, W], C in [1, 4], normalised as under TSSP_PIXELS_U8 with norm's rescale, mean
- * and std (its format is ignored): bit for bit tssp_op_im2col_ex of the fp32 image (float(u) * rescale - mean) / std.
- * pixels must be 8-byte aligned when P is a multiple of 8, 2-byte aligned when P is even. */
-int tssp_op_im2col_u8(const uint8_t* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens,
-                      const tssp_pixel_input_t* norm, void* stream);
+ * every image's patches, columns past C*P*P zero (the padded patch vector of patch sizes that are not a multiple of 8).
+ * input NULL or of format TSSP_PIXELS_F32: pixels are fp32 [n_img, C, H, W]. TSSP_PIXELS_U8: pixels are uint8
+ * [n_img, C, H, W], C in [1, 4], normalised with input's rescale, mean and std as under tssp_set_pixel_input: bit for bit
+ * the fp32 form of the image (float(u) * rescale - mean) / std; they must be 8-byte aligned when P is a multiple of 8,
+ * 2-byte aligned when P is even. */
+int tssp_op_im2col(const void* pixels, void* out_bf16, int n_img, int C, int H, int W, int P, int prefix_tokens,
+                   const tssp_pixel_input_t* input, void* stream);
 int tssp_op_cast_bf16(const float* in, int rows, int cols, int ld_in, void* out_bf16, int rows_pad, int cols_pad,
                       int ld_out, void* stream);
 int tssp_op_argmax_count(const float* logits, int ld, int n, int C, const int64_t* labels, int32_t* preds,

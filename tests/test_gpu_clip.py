@@ -147,28 +147,29 @@ def test_create_model_validates_before_touching_a_device():
     from twossp_b200 import _lib as L
     lib = L.load()
     h = C.c_void_p()
-    layout = L.TsspLayout(0, 0, 1, 0)
 
-    def err(cfg, opts, lay=layout):
-        assert lib.tssp_create_model(C.byref(cfg), C.byref(lay), C.byref(opts), 4096, C.byref(h)) != 0   # no device 4096
+    def err(cfg, pre_norm, ffn_act, layout=(0, 0, 0, 0)):   # layout: (dist_token, register_tokens, pos_patches_only, layer_scale)
+        cfg.pre_norm, cfg.ffn_act = pre_norm, ffn_act
+        cfg.dist_token, cfg.register_tokens, cfg.pos_patches_only, cfg.layer_scale = layout
+        assert lib.tssp_create(C.byref(cfg), 4096, C.byref(h)) != 0   # no device 4096
         return lib.tssp_last_error().decode()
 
-    msg = err(_config(L), L.TsspModelOpts(2, 1))
+    msg = err(_config(L), 2, 1)
     assert "pre_norm=2" in msg, msg
-    msg = err(_config(L), L.TsspModelOpts(1, 2))
+    msg = err(_config(L), 1, 2)
     assert "ffn_act=2" in msg, msg
-    msg = err(_config(L, score_point=0), L.TsspModelOpts(1, 1))   # QuickGELU is scored before the activation only
+    msg = err(_config(L, score_point=0), 1, 1)   # QuickGELU is scored before the activation only
     assert "score_point=1" in msg, msg
-    msg = err(_config(L, hidden=1280, image=224, patch=14, heads=16), L.TsspModelOpts(1, 1))   # ViT-H/14 CLIP: head dim 80
+    msg = err(_config(L, hidden=1280, image=224, patch=14, heads=16), 1, 1)   # ViT-H/14 CLIP: head dim 80
     assert "config: hidden=1280" in msg, msg
-    assert lib.tssp_create_model(C.byref(_config(L)), C.byref(layout), None, 4096, C.byref(h)) != 0
+    assert lib.tssp_create(None, 4096, C.byref(h)) != 0
     assert "NULL" in lib.tssp_last_error().decode()
     # every CLIP shape passes validation and fails on the device: B/32 (T = 50), B/16, L/14, L/14@336 (T = 577), with and
     # without the pre-norm, and the combined layout of registers and LayerScale
-    for hidden, image, patch, opts, lay in ((768, 224, 32, L.TsspModelOpts(1, 1), layout), (768, 224, 16, L.TsspModelOpts(1, 1), layout),
-                                            (1024, 224, 14, L.TsspModelOpts(1, 1), layout), (1024, 336, 14, L.TsspModelOpts(1, 1), layout),
-                                            (768, 224, 16, L.TsspModelOpts(0, 1), layout), (128, 84, 14, L.TsspModelOpts(1, 1), L.TsspLayout(0, 4, 0, 1))):
-        msg = err(_config(L, hidden=hidden, image=image, patch=patch), opts, lay)
+    for hidden, image, patch, opts, layout in ((768, 224, 32, (1, 1), (0, 0, 0, 0)), (768, 224, 16, (1, 1), (0, 0, 0, 0)),
+                                               (1024, 224, 14, (1, 1), (0, 0, 0, 0)), (1024, 336, 14, (1, 1), (0, 0, 0, 0)),
+                                               (768, 224, 16, (0, 1), (0, 0, 0, 0)), (128, 84, 14, (1, 1), (0, 4, 1, 1))):
+        msg = err(_config(L, hidden=hidden, image=image, patch=patch), *opts, layout)
         assert "device" in msg.lower() and "config" not in msg and "options" not in msg, msg
 
 
@@ -331,22 +332,49 @@ def test_layernorm_f32(ops, D):
 
 
 @pytest.mark.gpu
-def test_load_weights_counts_the_pre_norm_entries(lib):
+def test_load_weights_refuses_a_table_that_disagrees_with_its_config(lib):
     L = lib
     lb = L.load()
-    cfg = _config(L, hidden=128, image=48, patch=8)
-    h = C.c_void_p()
-    L.check(lb.tssp_create_model(C.byref(cfg), C.byref(L.TsspLayout(0, 0, 1, 0)), C.byref(L.TsspModelOpts(1, 1)), 0, C.byref(h)))
-    try:
-        n = L.W_GLOBAL_COUNT + 2 * L.BW_COUNT
-        table = (C.c_void_p * (n + 2))()
-        assert lb.tssp_load_weights(h, table, n, None) != 0
-        msg = lb.tssp_last_error().decode()
-        assert f"expected {n + 2} pointers" in msg and "pre-norm" in msg, msg
-        assert lb.tssp_load_weights(h, table, n + 2, None) != 0      # all NULL: refused by name, nothing read
-        assert "NULL" in lb.tssp_last_error().decode()
-    finally:
-        lb.tssp_destroy(h)
+    n = L.W_GLOBAL_COUNT + 2 * L.BW_COUNT
+    buf = torch.zeros(1 << 20, device="cuda")   # what every set slot points at: large enough for any entry, never read
+    required = [L.W_PATCH_W, L.W_CLS, L.W_POS, L.W_FINAL_LN_W, L.W_FINAL_LN_B, L.W_HEAD_W] + \
+               [L.W_GLOBAL_COUNT + b * L.BW_COUNT + i for b in range(2) for i in range(L.BW_LS1)]
+
+    def refused(fields, set_slots=(), null_slots=(), entries=n):
+        """the message of tssp_load_weights for an engine of _config + fields and a table with every plain-ViT entry set"""
+        cfg = _config(L, hidden=128, image=48, patch=8)
+        for k, v in fields.items():
+            setattr(cfg, k, v)
+        table = (C.c_void_p * max(n, entries))()
+        for i in [i for i in required if i not in null_slots] + list(set_slots):
+            table[i] = buf.data_ptr()
+        h = C.c_void_p()
+        L.check(lb.tssp_create(C.byref(cfg), 0, C.byref(h)))
+        try:
+            assert lb.tssp_load_weights(h, table, entries, None) != 0
+            return lb.tssp_last_error().decode()
+        finally:
+            lb.tssp_destroy(h)
+
+    clip = {"pre_norm": 1, "ffn_act": 1}
+    for entries in (n - 2, n + 2):   # a table of another length: the count is named
+        msg = refused(clip, entries=entries)
+        assert f"expected {n} pointers" in msg and f"got {entries}" in msg, msg
+    msg = refused(clip, null_slots=required)   # all NULL: refused by name, nothing read
+    assert "NULL" in msg, msg
+    msg = refused(clip)
+    assert "norm_pre weight or bias is NULL" in msg, msg
+    msg = refused({"ffn_act": 1}, set_slots=[L.W_NORM_PRE_W, L.W_NORM_PRE_B])
+    assert "TSSP_W_NORM_PRE_W" in msg and "pre_norm=0" in msg, msg
+    # the same for the LayerScale gammas and the distillation token
+    msg = refused({"layer_scale": 1}, set_slots=[L.W_GLOBAL_COUNT + L.BW_LS1, L.W_GLOBAL_COUNT + L.BW_COUNT + L.BW_LS1])
+    assert "block 0 LS2 gamma is NULL" in msg, msg
+    msg = refused({}, set_slots=[L.W_GLOBAL_COUNT + L.BW_COUNT + L.BW_LS1])
+    assert "block 1 TSSP_BW_LS1" in msg and "layer_scale=0" in msg, msg
+    msg = refused({"dist_token": 1})
+    assert "distillation token is NULL" in msg, msg
+    msg = refused({}, set_slots=[L.W_DIST_TOKEN])
+    assert "TSSP_W_DIST_TOKEN" in msg and "dist_token=0" in msg, msg
 
 
 # ----------------------------------------------------------------------------------------------- exactness
@@ -364,25 +392,6 @@ def _bits(api, model, px, labels):
 def _same(x, y):
     assert all(torch.equal(a, b) for a, b in zip(x[0], y[0]))
     assert torch.equal(x[1], y[1]) and x[2] == y[2]
-
-
-@pytest.mark.gpu
-def test_default_options_through_create_model_give_create_layout_bits(api, lib, monkeypatch):
-    real = lib.load()
-
-    class ViaModel:  # the engine wrapper made to create its handle through tssp_create_model with {0, erf GELU}
-        def __getattr__(self, name):
-            return getattr(real, name)
-
-        def tssp_create_layout(self, cfg, layout, device, out):
-            return real.tssp_create_model(cfg, layout, C.byref(lib.TsspModelOpts(0, 0)), device, out)
-
-    model = CS.make_clip("tiny", act="gelu", pre_norm=False)
-    px = synth.make_pixels(24, 48, seed=9)
-    labels = _fp32_logits(model, px).argmax(-1)
-    ours = _bits(api, model, px, labels)
-    monkeypatch.setattr(lib, "load", lambda: ViaModel())
-    _same(ours, _bits(api, model, px, labels))
 
 
 @pytest.mark.gpu

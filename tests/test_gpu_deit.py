@@ -121,25 +121,26 @@ def test_create_ex_validates_before_touching_a_device():
     lib = L.load()
     h = C.c_void_p()
 
-    def err(cfg, prefix):
-        assert lib.tssp_create_ex(C.byref(cfg), prefix, 4096, C.byref(h)) != 0   # device 4096 exists nowhere
+    def err(cfg, dist_token):
+        cfg.dist_token = dist_token
+        assert lib.tssp_create(C.byref(cfg), 4096, C.byref(h)) != 0   # device 4096 exists nowhere
         return lib.tssp_last_error().decode()
 
-    for prefix in (0, 3):
-        msg = err(_config(L), prefix)
-        assert f"prefix_tokens={prefix}" in msg, msg
-    msg = err(_config(L, hidden=100), 2)
+    for dist_token in (-1, 2):
+        msg = err(_config(L), dist_token)
+        assert f"dist_token={dist_token}" in msg, msg
+    msg = err(_config(L, hidden=100), 1)
     assert "hidden=100" in msg and "192" in msg, msg
-    msg = err(_config(L, image=40, patch=8), 2)            # T = 25 + 2 = 27
+    msg = err(_config(L, image=40, patch=8), 1)            # T = 25 + 2 = 27
     assert "T=27" in msg and "[32,1025]" in msg, msg
-    msg = err(_config(L, image=256, patch=8), 2)           # T = 1024 + 2
+    msg = err(_config(L, image=256, patch=8), 1)           # T = 1024 + 2
     assert "T=1026" in msg and "[32,1025]" in msg, msg
     # valid shapes pass validation and fail on the device: D = 192, T = 38 / 198 / 578
     for image, patch in ((48, 8), (224, 16), (384, 16)):
-        msg = err(_config(L, image=image, patch=patch), 2)
+        msg = err(_config(L, image=image, patch=patch), 1)
         assert "device" in msg.lower() and "config" not in msg, msg
-    # one prefix token through tssp_create_ex is tssp_create: T = 1025 is the last accepted
-    assert "device" in err(_config(L, image=512, patch=16), 1).lower()
+    # without a distillation token (one prefix token) T = 1025 is the last accepted
+    assert "device" in err(_config(L, image=512, patch=16), 0).lower()
 
 
 @pytest.fixture(scope="module")
@@ -205,19 +206,15 @@ def tiny_teacher():
 
 # ----------------------------------------------------------------------------------------------- kernels
 @pytest.mark.gpu
-def test_im2col_ex_with_two_prefix_rows_is_bit_exact(ops, lib):
-    L = lib.load()
+def test_im2col_with_one_and_two_prefix_rows_is_bit_exact(ops):
     for (n, Cc, H, P) in ((2, 3, 48, 8), (3, 3, 224, 16), (2, 3, 384, 16)):
         px = torch.randn(n, Cc, H, H, device="cuda")
         G = H // P
-        out = ops.im2col(px, P, prefix=2)
-        ref = px.view(n, Cc, G, P, G, P).permute(0, 2, 4, 1, 3, 5).reshape(n, G * G, Cc * P * P)
-        ref = torch.cat([torch.zeros(n, 2, Cc * P * P, device="cuda"), ref], dim=1).bfloat16().reshape(n * (G * G + 2), -1)
-        assert torch.equal(out.view(torch.int16), ref.view(torch.int16))
-        one = ops.im2col(px, P, prefix=1)
-        old = torch.empty_like(one)
-        lib.check(L.tssp_op_im2col(lib.ptr(px), lib.ptr(old), n, Cc, H, H, P, lib.current_stream()))
-        assert torch.equal(one.view(torch.int16), old.view(torch.int16))
+        patches = px.view(n, Cc, G, P, G, P).permute(0, 2, 4, 1, 3, 5).reshape(n, G * G, Cc * P * P)
+        for prefix in (1, 2):
+            out = ops.im2col(px, P, prefix=prefix)
+            ref = torch.cat([torch.zeros(n, prefix, Cc * P * P, device="cuda"), patches], dim=1).bfloat16()
+            assert torch.equal(out.view(torch.int16), ref.reshape(n * (G * G + prefix), -1).view(torch.int16))
 
 
 @pytest.mark.gpu

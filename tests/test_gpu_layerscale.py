@@ -118,22 +118,22 @@ def test_create_layout_validates_before_touching_a_device():
     lib = L.load()
     h = C.c_void_p()
 
-    def err(cfg, layout):
-        assert lib.tssp_create_layout(C.byref(cfg), C.byref(layout), 4096, C.byref(h)) != 0   # device 4096 exists nowhere
+    def err(cfg, *layout):   # (dist_token, register_tokens, pos_patches_only, layer_scale)
+        cfg.dist_token, cfg.register_tokens, cfg.pos_patches_only, cfg.layer_scale = layout
+        assert lib.tssp_create(C.byref(cfg), 4096, C.byref(h)) != 0   # device 4096 exists nowhere
         return lib.tssp_last_error().decode()
 
-    msg = err(_config(L), L.TsspLayout(0, 8, 0, 1))
+    msg = err(_config(L), 0, 8, 1, 1)
     assert "register_tokens=8" in msg and "[0,7]" in msg, msg
-    msg = err(_config(L), L.TsspLayout(1, 4, 0, 1))
+    msg = err(_config(L), 1, 4, 1, 1)
     assert "distillation token and register tokens" in msg, msg
-    msg = err(_config(L, hidden=768, image=518, patch=14), L.TsspLayout(0, 0, 1, 1))   # DINOv2 at its native size
+    msg = err(_config(L, hidden=768, image=518, patch=14), 0, 0, 0, 1)   # DINOv2 at its native size
     assert "T=1370" in msg and "[32,1025]" in msg, msg
-    msg = err(_config(L, hidden=768, image=518, patch=14), L.TsspLayout(0, 4, 0, 1))   # ... with four registers
+    msg = err(_config(L, hidden=768, image=518, patch=14), 0, 4, 1, 1)   # ... with four registers
     assert "T=1374" in msg and "[32,1025]" in msg, msg
     # valid layouts pass validation and fail on the device: patch 14 (K = 588), T = 41 / 257 / 261, patch 8 with LayerScale
-    for layout, image, patch in ((L.TsspLayout(0, 4, 0, 1), 84, 14), (L.TsspLayout(0, 0, 1, 1), 224, 14),
-                                 (L.TsspLayout(0, 4, 0, 1), 224, 14), (L.TsspLayout(0, 0, 0, 1), 48, 8)):
-        msg = err(_config(L, image=image, patch=patch), layout)
+    for layout, image, patch in (((0, 4, 1, 1), 84, 14), ((0, 0, 0, 1), 224, 14), ((0, 4, 1, 1), 224, 14), ((0, 0, 1, 1), 48, 8)):
+        msg = err(_config(L, image=image, patch=patch), *layout)
         assert "device" in msg.lower() and "config" not in msg and "layout" not in msg, msg
 
 
@@ -319,26 +319,6 @@ def test_class_free_position_table_gives_the_bits_of_the_embedded_one(api):
     px = synth.make_pixels(24, 84, seed=8)
     labels = _fp32_logits(full, px).argmax(-1)
     _same(_bits(api, free, px, labels), _bits(api, full, px, labels))
-
-
-@pytest.mark.gpu
-def test_create_layout_with_the_default_layout_gives_create_bits(api, lib, monkeypatch):
-    real = lib.load()
-
-    class ViaCreate:  # the engine wrapper made to create its handle through tssp_create
-        def __getattr__(self, name):
-            return getattr(real, name)
-
-        def tssp_create_layout(self, cfg, layout, device, out):
-            return real.tssp_create(cfg, device, out)
-
-    model = synth.TimmLikeViT()
-    px = synth.make_pixels(24, 48, seed=9)
-    labels = _fp32_logits(model, px).argmax(-1)
-    ours = _bits(api, model, px, labels)
-    api.release_engine(model)
-    monkeypatch.setattr(lib, "load", lambda: ViaCreate())
-    _same(ours, _bits(api, model, px, labels))
 
 
 # ----------------------------------------------------------------------------------------------- tiny stand-ins

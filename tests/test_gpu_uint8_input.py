@@ -345,16 +345,16 @@ def test_c_abi_refusals_name_the_fault(api, lib):
 
     def msg():
         return raw.tssp_last_error().decode()
-    assert raw.tssp_op_im2col_u8(L.ptr(u), L.ptr(out), 4, 3, 64, 64, 16, 1, good, s) == 0
+    assert raw.tssp_op_im2col(L.ptr(u), L.ptr(out), 4, 3, 64, 64, 16, 1, good, s) == 0
     five = torch.zeros(5 * 64 * 64, device="cuda", dtype=torch.uint8)
-    assert raw.tssp_op_im2col_u8(L.ptr(five), L.ptr(out), 1, 5, 64, 64, 16, 1, L.pixel_input(L.PIXELS_U8, [0.0] * 4, [1.0] * 4), s) != 0
+    assert raw.tssp_op_im2col(L.ptr(five), L.ptr(out), 1, 5, 64, 64, 16, 1, L.pixel_input(L.PIXELS_U8, [0.0] * 4, [1.0] * 4), s) != 0
     assert "channels" in msg() and "C=5" in msg()
     bad = L.pixel_input(L.PIXELS_U8, IMAGENET[0], (0.2, 0.0, 0.2), 1 / 255)
-    assert raw.tssp_op_im2col_u8(L.ptr(u), L.ptr(out), 4, 3, 64, 64, 16, 1, bad, s) != 0
+    assert raw.tssp_op_im2col(L.ptr(u), L.ptr(out), 4, 3, 64, 64, 16, 1, bad, s) != 0
     assert "std[1]" in msg()
-    assert raw.tssp_op_im2col_u8(C.c_void_p(u.data_ptr() + 1), L.ptr(out), 4, 3, 64, 64, 16, 1, good, s) != 0
+    assert raw.tssp_op_im2col(C.c_void_p(u.data_ptr() + 1), L.ptr(out), 4, 3, 64, 64, 16, 1, good, s) != 0
     assert "aligned" in msg()
-    assert raw.tssp_op_im2col_u8(C.c_void_p(u.data_ptr() + 1), L.ptr(out), 1, 3, 28, 28, 14, 1, good, s) != 0
+    assert raw.tssp_op_im2col(C.c_void_p(u.data_ptr() + 1), L.ptr(out), 1, 3, 28, 28, 14, 1, good, s) != 0
     assert "2-byte aligned" in msg()
     # the engine setter: bad values are refused and the engine keeps its format
     model = synth.TimmLikeViT().cuda()

@@ -67,9 +67,9 @@ def im2col_times(api, ops, dev, rounds: int) -> dict:
         def fn():
             i = it["i"] = (it["i"] + 1) % 4
             if fp32:
-                rc = lib.tssp_op_im2col_ex(*args_f[i], n, 3, H, H, P, 1, stream)
+                rc = lib.tssp_op_im2col(*args_f[i], n, 3, H, H, P, 1, None, stream)
             else:
-                rc = lib.tssp_op_im2col_u8(*args_u[i], n, 3, H, H, P, 1, norm, stream)
+                rc = lib.tssp_op_im2col(*args_u[i], n, 3, H, H, P, 1, norm, stream)
             if rc:
                 L.check(rc)
         return fn

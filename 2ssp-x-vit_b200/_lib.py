@@ -10,7 +10,7 @@ import os
 from pathlib import Path
 
 TSSP_MAX_BLOCKS = 64
-TSSP_ABI_VERSION = 2
+TSSP_ABI_VERSION = 3
 
 _PKG_DIR = Path(__file__).resolve().parent
 LIB_PATH = _PKG_DIR / "lib" / "libtssp_b200.so"
@@ -117,7 +117,7 @@ SIGNATURES = {
     "tssp_op_score_finish": (_I, [_P, _I, _P, _I, _I, _I, _I, _P, _P]),
     "tssp_op_layernorm": (_I, [_P, _I64, _P, _P, _P, _I, _I, C.c_float, _P]),
     "tssp_op_layernorm_f32": (_I, [_P, _I64, _P, _P, _P, _I64, _I, _I, C.c_float, _P]),
-    "tssp_op_attention": (_I, [_P, _P, _I, _I, _I, _I, _P]),
+    "tssp_op_attention": (_I, [_P, _P, _I, _I, _I, _I, _P, _I, _I, _P]),
     "tssp_op_im2col": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, C.POINTER(TsspPixelInput), _P]),
     "tssp_op_cast_bf16": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P]),
     "tssp_op_argmax_count": (_I, [_P, _I, _I, _I, _P, _P, _P, _P]),

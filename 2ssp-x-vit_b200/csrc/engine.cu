@@ -1806,10 +1806,14 @@ int tssp_op_layernorm_f32(const float* x, int64_t in_stride, const float* gamma,
     if (x == nullptr || gamma == nullptr || beta == nullptr || out_f32 == nullptr) return fail("tssp_op_layernorm_f32: NULL argument");
     return op_layernorm_f32(x, in_stride, gamma, beta, out_f32, out_stride, rows, D, eps, static_cast<cudaStream_t>(stream));
 }
-int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream) {
+int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, const float* qk_norms,
+                      int ld_norms, int first_tile_only, void* stream) {
     TSSP_ENTRY();
     if (qkv_bf16 == nullptr || ctx_bf16 == nullptr) return fail("tssp_op_attention: NULL argument");
-    return op_attention(qkv_bf16, ctx_bf16, n_img, T, heads, D, static_cast<cudaStream_t>(stream));
+    if (qk_norms != nullptr && ld_norms < 2 * heads)
+        return fail("tssp_op_attention: ld_norms=%d is less than 2*heads=%d (|q|^2 and |k|^2 columns of every head)", ld_norms, 2 * heads);
+    return op_attention(qkv_bf16, ctx_bf16, n_img, T, heads, D, static_cast<cudaStream_t>(stream), qk_norms, ld_norms,
+                        first_tile_only != 0);
 }
 int tssp_debug_gemm_trace(long long* device_buf) {
     TSSP_ENTRY();

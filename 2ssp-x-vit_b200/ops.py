@@ -123,15 +123,30 @@ def layernorm_f32(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps:
     return out
 
 
-def attention(qkv: torch.Tensor, n_img: int, T: int, heads: int) -> torch.Tensor:
-    _need_cuda(qkv)
+def attention(qkv: torch.Tensor, n_img: int, T: int, heads: int, *, norms: torch.Tensor | None = None,
+              cls_only: bool = False, out: torch.Tensor | None = None) -> torch.Tensor:
+    """ctx [n*T, D] bf16 = softmax(Q K^T / 8) V per (image, head) of the fused qkv [n*T, 3*D].
+
+    norms: fp32 [n*T, ld >= 2*heads] with |q|^2 of head h in column h and |k|^2 in column heads + h (the rownorm output
+    of gemm_rownorm): the softmax shifts come from them, as in the engine's forward. cls_only: only rows [0, 128) of
+    every image are written, as in the engine's last block. out: the ctx tensor to write into (rows the kernel does not
+    write keep their contents)."""
+    _need_cuda(qkv, norms, out)
     if qkv.dtype != torch.bfloat16 or not qkv.is_contiguous():
         raise ValueError("attention: qkv must be a contiguous bfloat16 tensor [n*T, 3*D]")
     D = qkv.shape[1] // 3
-    ctx = torch.empty(n_img * T, D, device=qkv.device, dtype=torch.bfloat16)
+    if norms is not None and (norms.dtype != torch.float32 or norms.dim() != 2 or norms.stride(1) != 1
+                              or norms.shape[0] != n_img * T):
+        raise ValueError(f"attention: norms must be float32 [n*T, ld] with unit column stride, got {norms.dtype} "
+                         f"{tuple(norms.shape)}")
+    if out is None:
+        out = torch.empty(n_img * T, D, device=qkv.device, dtype=torch.bfloat16)
+    elif out.dtype != torch.bfloat16 or not out.is_contiguous() or tuple(out.shape) != (n_img * T, D):
+        raise ValueError(f"attention: out must be a contiguous bfloat16 tensor [{n_img * T}, {D}]")
     lib = L.load()
-    L.check(lib.tssp_op_attention(L.ptr(qkv), L.ptr(ctx), n_img, T, heads, D, L.current_stream()))
-    return ctx
+    L.check(lib.tssp_op_attention(L.ptr(qkv), L.ptr(out), n_img, T, heads, D, L.ptr(norms),
+                                  norms.stride(0) if norms is not None else 0, 1 if cls_only else 0, L.current_stream()))
+    return out
 
 
 def im2col(pixels: torch.Tensor, patch: int, prefix: int = 1, *, mean=None, std=None, rescale: float = 1 / 255) -> torch.Tensor:

@@ -31,7 +31,7 @@ extern "C" {
 #endif
 
 #define TSSP_MAX_BLOCKS 64
-#define TSSP_ABI_VERSION 2
+#define TSSP_ABI_VERSION 3
 
 typedef struct tssp_engine* tssp_handle_t;
 
@@ -229,7 +229,12 @@ int tssp_op_layernorm_f32(const float* x, int64_t in_stride, const float* gamma,
                           int64_t out_stride, int rows, int D, float eps, void* stream);
 /* ctx[n*T, D] = softmax(Q K^T / 8) V per (image, head) from the fused qkv[n*T, 3D]; head_dim 64, 16 <= T <= 1025
  * (up to 208 padded keys one kernel holds a whole key row, beyond that a second one streams keys in tiles of 128). */
-int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, void* stream);
+/* qk_norms: NULL, or fp32 [n*T][ld_norms] with |q|^2 of head h in column h and |k|^2 in column heads + h (the
+ * rownorm output of tssp_op_gemm_rownorm with ld_norms >= 2*heads): the softmax shifts are taken from them instead of
+ * from q and k, as the engine does. first_tile_only != 0: only rows [0, 128) of every image are written; the rest of
+ * ctx is left as it was. */
+int tssp_op_attention(const void* qkv_bf16, void* ctx_bf16, int n_img, int T, int heads, int D, const float* qk_norms,
+                      int ld_norms, int first_tile_only, void* stream);
 /* out[n * T, Kp] with T = (H/P)^2 + prefix_tokens and Kp = round_up(C*P*P, 8): prefix_tokens (1..8) zero rows ahead of
  * every image's patches, columns past C*P*P zero (the padded patch vector of patch sizes that are not a multiple of 8).
  * input NULL or of format TSSP_PIXELS_F32: pixels are fp32 [n_img, C, H, W]. TSSP_PIXELS_U8: pixels are uint8

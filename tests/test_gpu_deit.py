@@ -21,6 +21,7 @@ from oracle import twossp_oracle as O
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import deit_synth as DS  # noqa: E402
+import attention_ref as R  # noqa: E402
 
 SCORE_RTOL = 1e-2
 LOGIT_MAX_ABS = 3e-2
@@ -320,14 +321,8 @@ def test_gemm_score_epilogue_at_192(ops, lib, gemm_form, pre, n_img, T, N, K):
 @pytest.mark.gpu
 @pytest.mark.parametrize("n,T,heads", [(4, 198, 3), (3, 198, 12), (2, 578, 12), (5, 38, 3)])
 def test_attention_at_deit_shapes(ops, n, T, heads):
-    D = heads * 64
-    g = torch.Generator(device="cuda").manual_seed(T * 7 + heads)
-    qkv = torch.randn(n * T, 3 * D, device="cuda", generator=g).bfloat16()
-    ctx = ops.attention(qkv, n, T, heads)
-    q, k, v = qkv.float().view(n, T, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).permute(0, 2, 1, 3).reshape(n * T, D)
-    assert torch.isfinite(ctx.float()).all()
-    assert ((ctx.float() - ref).abs() <= ref.abs() * 2 ** -7 + 6e-3).all()
+    qkv = R.iid_qkv(n, T, heads, 1.0, seed=T * 7 + heads, device="cuda")
+    R.run_and_check(ops, qkv, n, T, heads, scale=1.0)
 
 
 # ----------------------------------------------------------------------------------------------- tiny distilled DeiT

@@ -19,6 +19,7 @@ from oracle import twossp_oracle as O
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import layerscale_synth as LS  # noqa: E402
+import attention_ref as R  # noqa: E402
 
 SCORE_RTOL = 1e-2
 LOGIT_MAX_ABS = 3e-2
@@ -262,14 +263,8 @@ def test_gemm_scaled_epilogue_matches_torch(ops, lib, gemm_form, M, N, K, reduce
 @pytest.mark.gpu
 @pytest.mark.parametrize("n,T,heads", [(4, 257, 6), (3, 261, 12), (2, 261, 6), (5, 41, 2), (5, 37, 3)])
 def test_attention_at_layerscale_shapes(ops, n, T, heads):
-    D = heads * 64
-    g = torch.Generator(device="cuda").manual_seed(T * 7 + heads)
-    qkv = torch.randn(n * T, 3 * D, device="cuda", generator=g).bfloat16()
-    ctx = ops.attention(qkv, n, T, heads)
-    q, k, v = qkv.float().view(n, T, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).permute(0, 2, 1, 3).reshape(n * T, D)
-    assert torch.isfinite(ctx.float()).all()
-    assert ((ctx.float() - ref).abs() <= ref.abs() * 2 ** -7 + 6e-3).all()
+    qkv = R.iid_qkv(n, T, heads, 1.0, seed=T * 7 + heads, device="cuda")
+    R.run_and_check(ops, qkv, n, T, heads, scale=1.0)
 
 
 # ----------------------------------------------------------------------------------------------- exactness

@@ -20,6 +20,9 @@ import torch
 from oracle import synth
 from oracle import twossp_oracle as O
 
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import attention_ref as R  # noqa: E402
+
 SCORE_RTOL = 1e-2
 LOGIT_MAX_ABS = 3e-2
 LOGIT_MEAN_ABS = 5e-3
@@ -70,21 +73,30 @@ def tiny_long():
 
 
 # ----------------------------------------------------------------------------------------------- kernel
+# key-tile and query-group edges: 255 / 256 (two key tiles, the second full), 384 / 385, 512 / 513 (one vs two
+# query-tile groups), 640 / 641 and 1024; n makes >= 1e5 outputs for the bias check
+_LONG_T = [(R.images_for(T, h), T, h) for T, h in ((255, 2), (256, 3), (384, 2), (385, 4), (512, 2), (513, 3), (640, 2),
+                                                   (641, 2), (1024, 2))]
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("scale", [1.0, 0.05, 3.0])   # 3.0 makes the Cauchy-Schwarz shift too loose: exact two-sweep route
 @pytest.mark.parametrize("n,T,heads", [(2, 209, 2), (2, 224, 4), (3, 257, 2), (3, 290, 2), (2, 577, 12), (1, 785, 12),
-                                       (1, 1025, 16), (130, 577, 12)])
+                                       (1, 1025, 16), (130, 577, 12)] + _LONG_T)
 def test_long_attention(ops, n, T, heads, scale):
-    D = heads * 64
-    g = torch.Generator(device="cuda").manual_seed(T * 31 + n)
-    qkv = (torch.randn(n * T, 3 * D, device="cuda", generator=g) * scale).bfloat16()
-    ctx = ops.attention(qkv, n, T, heads)
-    q, k, v = qkv.float().view(n, T, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).permute(0, 2, 1, 3).reshape(n * T, D)
-    assert torch.isfinite(ctx.float()).all()
-    # bf16 P and one bf16 rounding of outputs of magnitude O(scale)
-    assert ((ctx.float() - ref).abs() <= ref.abs() * 2 ** -7 + 6e-3 * max(1.0, scale)).all()
-    assert torch.equal(ops.attention(qkv, n, T, heads), ctx)
+    qkv = R.iid_qkv(n, T, heads, scale, seed=T * 31 + n, device="cuda")
+    R.run_and_check(ops, qkv, n, T, heads, scale=scale)
+
+
+# units just past one and two per SM (a persistent CTA walks one or two more units than its neighbours)
+@pytest.mark.gpu
+@pytest.mark.parametrize("scale", [1.0, 3.0])
+@pytest.mark.parametrize("extra", ["sms+1", "2sms-1", "2sms+1"])
+def test_long_attention_at_unit_counts_around_the_sm_count(ops, extra, scale):
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    n = {"sms+1": sms + 1, "2sms-1": 2 * sms - 1, "2sms+1": 2 * sms + 1}[extra]
+    qkv = R.iid_qkv(n, 577, 1, scale, seed=n, device="cuda")
+    R.run_and_check(ops, qkv, n, 577, 1, scale=scale)
 
 
 @pytest.mark.gpu

@@ -13,6 +13,7 @@ Tolerances (stated once, used below):
 """
 import copy
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -20,6 +21,9 @@ import torch
 
 from oracle import synth
 from oracle import twossp_oracle as O
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import attention_ref as R  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -148,17 +152,28 @@ def test_layernorm(ops):
     assert ((out.float() - ref).abs() <= ref.abs() * 2 ** -8 + 1e-4).all()
 
 
+# the short-sequence kernel at the edges of its structure: 16-31 keys (one 16- or 32-column chunk), 127 / 128 / 129 (one
+# vs two query tiles), 144 (a 16-wide last chunk), 192 / 193 and 208 (its limit); n makes >= 1e5 outputs for the bias check
+_SHORT_T = [(R.images_for(T, h), T, h) for T, h in ((16, 2), (17, 3), (31, 1), (33, 4), (127, 2), (128, 3), (129, 2),
+                                                    (144, 6), (192, 2), (193, 3), (208, 2))]
+
+
 @pytest.mark.parametrize("scale", [1.0, 0.05, 3.0])   # 3.0 makes the Cauchy-Schwarz shift too loose: exact two-pass route
-@pytest.mark.parametrize("n,T,heads", [(3, 37, 2), (2, 65, 4), (4, 197, 12), (2, 208, 6), (1, 32, 1), (130, 197, 12)])
+@pytest.mark.parametrize("n,T,heads", [(3, 37, 2), (2, 65, 4), (4, 197, 12), (2, 208, 6), (1, 32, 1), (130, 197, 12)] + _SHORT_T)
 def test_attention(ops, n, T, heads, scale):
-    D = heads * 64
-    qkv = (torch.randn(n * T, 3 * D, device="cuda") * scale).bfloat16()
-    ctx = ops.attention(qkv, n, T, heads)
-    q, k, v = qkv.float().view(n, T, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).permute(0, 2, 1, 3).reshape(n * T, D)
-    assert torch.isfinite(ctx.float()).all()
-    # bf16 P and one bf16 rounding of outputs of magnitude O(scale)
-    assert ((ctx.float() - ref).abs() <= ref.abs() * 2 ** -7 + 6e-3 * max(1.0, scale)).all()
+    qkv = R.iid_qkv(n, T, heads, scale, seed=T * 13 + n, device="cuda")
+    R.run_and_check(ops, qkv, n, T, heads, scale=scale)
+
+
+# units (image, head) just past one and two per SM: a CTA's two chains get unequal tile counts (the `other_tiles`
+# alternation of the two chains' softmax phases)
+@pytest.mark.parametrize("scale", [1.0, 3.0])
+@pytest.mark.parametrize("extra", ["sms+1", "2sms-1", "2sms+1"])
+def test_attention_at_unit_counts_around_the_sm_count(ops, extra, scale):
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    n = {"sms+1": sms + 1, "2sms-1": 2 * sms - 1, "2sms+1": 2 * sms + 1}[extra]
+    qkv = R.iid_qkv(n, 197, 1, scale, seed=n, device="cuda")
+    R.run_and_check(ops, qkv, n, 197, 1, scale=scale)
 
 
 def test_im2col_is_bit_exact(ops):

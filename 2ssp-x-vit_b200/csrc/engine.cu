@@ -333,6 +333,8 @@ static int gemm(int mode, const void* A, int lda, const void* W, int ldw, void* 
     if (mode == EPI_F32_SCALED && col_scale == nullptr) return fail("gemm: scaled fp32 epilogue needs a column scale");
     const bool score = gemm_mode_scores(mode);
     if (score && (partials == nullptr || T < 32 || ldp < N)) return fail("gemm: score epilogue needs partials, ldp >= N and T >= 32 (T=%d)", T);
+    // the epilogue stores each lane's two partials as one float2 and the finisher reads them as float4
+    if (score && (ldp & 3)) return fail("gemm: score partial row pitch %d must be a multiple of 4", ldp);
     const CUtensorMap *ta, *tb, *tc;
     TSSP_TRY(get_tmap(&ta, A, false, K, M, static_cast<uint64_t>(lda) * 2, 64, 128));
     // fp32-output GEMMs with a short reduction whose last 256-column tile would be at most half full (N = 384, K = 384: the
